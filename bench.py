@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # our arm (one rank per GPU; N>1 under torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU path (oracle port) on host cores
     python bench.py --sweep                                   # BASELINE config 5 table (chunk count 8..8192, low/high entropy)
+    python bench.py --steps K --warmup W --dump-outputs DIR   # also writes the last timed step's payload / segment offsets as DIR/*.npy
 
 Workload (BASELINE.json configs[1]): SmolLM-135M, 512 reprime-chunks batched on one B200, over enwik8.  Offline only the first
 3 MiB of enwik8 exist (tests/golden/data/enwik8_3mib.xz = final_bench/enwik8_samples/enwik8_128kb_{0..23}); a "step" is one
@@ -65,6 +66,20 @@ def enwik_slice_ids(k):
     d = corpus.load("enwik8_3mib")
     k %= len(d) // SLICE
     return corpus.byte_ids(d[k * SLICE:(k + 1) * SLICE], V_SMOLLM, spread=True)
+
+
+def dump_outputs(d, arrays, budget=64 << 20):
+    """writes each array as d/<name>.npy: 64-bit integers as float64 (exact below 2^53), everything else as float32.  Each array gets
+    an equal share of `budget` bytes; one larger than its share is replaced by a fixed sample of its elements (seed 0, ascending
+    positions), so that two builds given the same arguments write files that compare element for element."""
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a).ravel()
+        a = a.astype(np.float64 if a.dtype.itemsize == 8 else np.float32)
+        keep = budget // len(arrays) // a.itemsize
+        if a.size > keep:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(d, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -345,6 +360,11 @@ def run_ours(args):
     launches = ctx.launch_count() - l0
     clocks = sampler.stop()
     payload_bytes = int(seg_off[S])
+    if args.dump_outputs:
+        # what a caller of cz_encode_dev receives from the last timed step: the concatenated segment bitstreams and their offsets
+        sfx = f"_rank{rank}" if world > 1 else ""
+        dump_outputs(args.dump_outputs, {"payload" + sfx: out_dev[:payload_bytes].cpu().numpy(), "seg_off" + sfx: seg_off},
+                     budget=(64 << 20) // world)
     ms_max = D.max(ms)
     value = world * n * args.steps / (ms_max / 1e3) / 1e6
 
@@ -602,7 +622,11 @@ def main():
     ap.add_argument("--cpu-tokens", type=int, default=4096, help="prefix of alice29.txt the CPU reference codes (>= 7 reprimes)")
     ap.add_argument("--rwkv-bytes", type=int, default=1048576, help="RWKV-7 figures on this prefix of the enwik8 stand-in (0 = skip)")
     ap.add_argument("--rwkv-segments", type=int, default=1024)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the payload bytes and segment offsets of the last timed step as DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.sweep or args.steps < 1):
+        ap.error("--dump-outputs needs the default GPU arm and --steps >= 1")
     if args.impl == "reference":
         # torchrun exports OMP_NUM_THREADS=1; the reference arm is meant to use every host core it can
         os.environ["OMP_NUM_THREADS"] = str(os.cpu_count() or 1)

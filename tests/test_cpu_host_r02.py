@@ -175,3 +175,19 @@ def test_built_library_is_made_of_tcgen05_tma_and_fp64_kernels():
     prefix = kernels("cdf_bounds_warp_kernel<")
     assert prefix and all(c["DADD"] >= 32 for c in prefix)
     assert kernels("attn_mma_kernel<") and all(c["HMMA"] > 0 for c in kernels("attn_mma_kernel<"))  # the bisecting fallback, and only it
+
+
+def test_bench_dump_outputs_is_exact_bounded_and_repeatable(tmp_path):
+    """bench.py --dump-outputs: bytes as float32 and 64-bit offsets as float64 without loss, and an output over the size budget
+    replaced by the same sample of its elements on every run"""
+    import bench
+
+    pay = np.random.default_rng(3).integers(0, 256, 5000).astype(np.uint8)
+    off = np.array([0, 17, 2 ** 40 + 1], np.uint64)
+    bench.dump_outputs(str(tmp_path / "a"), {"payload": pay, "seg_off": off})
+    a, o = np.load(tmp_path / "a" / "payload.npy"), np.load(tmp_path / "a" / "seg_off.npy")
+    assert a.dtype == np.float32 and np.array_equal(a, pay) and o.dtype == np.float64 and np.array_equal(o.astype(np.uint64), off)
+    for d in ("b", "c"):
+        bench.dump_outputs(str(tmp_path / d), {"payload": pay, "seg_off": off}, budget=8000)
+    b, c = np.load(tmp_path / "b" / "payload.npy"), np.load(tmp_path / "c" / "payload.npy")
+    assert b.nbytes == 4000 and np.array_equal(b, c) and set(b.tolist()) <= set(pay.tolist())
