@@ -5,6 +5,7 @@ batched B200 path.  Out of scope here, as in DESIGN.md: hf-hub download, agents,
 Weights: --weights *.safetensors (HF LLaMA / candle_rwkv7 tensor names) or --random-init SEED (no checkpoints exist offline).
 Tokenizer: --tokenizer tokenizer.json (HF `tokenizers`, SmolLM) or a RWKV vocab json; default = byte-level ids (lossless for
 every input).  --segments N > 1 writes the SEG1 container extension (parallel decode); N = 1 is the reference's v2 layout.
+--on-zero-width {stored,floor}: what compress does when the SmolLM coder meets a token of mass < 2^-30 (codec.compress).
 """
 import argparse
 import sys
@@ -108,6 +109,9 @@ def main(argv=None):
     ap.add_argument("--random-init", type=int, default=0)
     ap.add_argument("--tokenizer")
     ap.add_argument("--device", type=int, default=0)
+    ap.add_argument("--on-zero-width", choices=["stored", "floor"],
+                    help="compress / self-test: a token the SmolLM coder cannot code stores the input uncoded (stored) or codes it "
+                         "again with the floored pdf (floor); default stored")
     # the agentic gate, replay only (src/main.rs:74-118: --scan, --scan-lookahead, --reuse-scan-dir, gate thresholds); SmolLM backend
     ap.add_argument("--reuse-scan-dir", help="directory with agent_cache.jsonl (+ proof.csv) of a finished run: replay the gate scan")
     ap.add_argument("--scan-lookahead", type=int, default=512)
@@ -119,11 +123,14 @@ def main(argv=None):
     scan = bool(args.reuse_scan_dir)
     if scan and (args.backend != "smollm" or args.segments != 1):
         ap.error("--reuse-scan-dir works on the SmolLM backend with one AC stream (--segments 1), like the reference's container")
+    if scan and args.on_zero_width:
+        ap.error("--on-zero-width is not available with --reuse-scan-dir (the gated stream has no fallback of either kind)")
     model, tok = _model(args)
     data = open(args.input, "rb").read()
     if args.command == "compress":
         blob = _scan_compress(model, tok, data, args) if scan else \
-            codec.compress(model, data, tok, args.segments, context=args.context, reprime_interval=args.reprime_interval)
+            codec.compress(model, data, tok, args.segments, context=args.context, reprime_interval=args.reprime_interval,
+                           on_zero_width=args.on_zero_width or "stored")
         open(args.output or args.input + ".canz", "wb").write(blob)
         print(f"{len(data)} -> {len(blob)} bytes ({8 * len(blob) / max(1, len(data)):.4f} bits/byte)")
     elif args.command == "decompress":
@@ -133,7 +140,8 @@ def main(argv=None):
     else:  # self-test: encode + decode round trip with timings (src/main.rs:156-221)
         t0 = time.perf_counter()
         blob = _scan_compress(model, tok, data, args) if scan else \
-            codec.compress(model, data, tok, args.segments, context=args.context, reprime_interval=args.reprime_interval)
+            codec.compress(model, data, tok, args.segments, context=args.context, reprime_interval=args.reprime_interval,
+                           on_zero_width=args.on_zero_width or "stored")
         t1 = time.perf_counter()
         out = _scan_decompress(model, tok, blob, args) if scan else codec.decompress(model, blob, tok)
         t2 = time.perf_counter()

@@ -22,12 +22,13 @@ CZ_ERR_NO_DEVICE = -2
 CZ_ERR_ZERO_WIDTH = -4
 CZ_ERR_UNSUPPORTED = -7
 CZ_ERR_SYMBOL_RANGE = -8
-CZ_CDF_SMOLLM, CZ_CDF_RWKV_LITERALS = 0, 1
+CZ_CDF_SMOLLM, CZ_CDF_RWKV_LITERALS, CZ_CDF_SMOLLM_FLOOR = 0, 1, 2
 CZ_ARCH_SMOLLM, CZ_ARCH_RWKV7 = 0, 1
 CZ_DTYPE_F32, CZ_DTYPE_BF16, CZ_DTYPE_F16 = 0, 1, 2
 CZ_ENGINE_TCGEN05, CZ_ENGINE_SIMT = 0, 1
 CZ_FLAG_SEGMENTS = 1 << 8
 CZ_FLAG_STORED = 1 << 9
+CZ_FLAG_PDF_FLOOR = 1 << 10
 K_FAMILIES = ("gemm_qkv", "attn", "elemwise", "cdf", "coder", "other", "gemm_o", "gemm_gu", "gemm_down", "gemm_head", "cdf_prefix")
 
 
@@ -125,6 +126,7 @@ SIGNATURES = {
     "cz_decode": (C.c_int, [_vp, u8p, u64p, C.c_size_t, C.POINTER(Schedule), u32p]),
     "cz_encode_dev": (C.c_int, [_vp, _vp, C.c_size_t, C.POINTER(Schedule), _vp, C.c_size_t, u64p]),
     "cz_model_set_digest_out": (C.c_int, [_vp, u8p, C.c_size_t]),
+    "cz_model_set_pdf_floor": (C.c_int, [_vp, C.c_int]),
     "cz_xe_bits": (C.c_int, [_vp, C.POINTER(XeJob), C.c_size_t, f64p]),
     "cz_chunk_logits": (C.c_int, [_vp, u32p, C.c_size_t, u32p, C.c_size_t, f32p]),
     "cz_container_header_size": (C.c_size_t, [C.POINTER(HeaderV2)]),

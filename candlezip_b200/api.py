@@ -252,8 +252,15 @@ class Model:
             keep.append(arr)
         return s, keep
 
-    def encode(self, ids, n_segments=1, bos=0, context=512, reprime_interval=512, events=None, seg_start=None, max_batch_tokens=0):
-        """ids: coded tokens (no BOS). Returns (list of per-segment payload bytes, seg_start)."""
+    def set_pdf_floor(self, enabled):
+        """code SmolLM streams with the floored pdf (CZ_CDF_SMOLLM_FLOOR) in the following encode / decode calls; RWKV-7 refuses"""
+        check(lib.cz_model_set_pdf_floor(self._h, 1 if enabled else 0))
+
+    def encode(self, ids, n_segments=1, bos=0, context=512, reprime_interval=512, events=None, seg_start=None, max_batch_tokens=0,
+               pdf_floor=False):
+        """ids: coded tokens (no BOS). Returns (list of per-segment payload bytes, seg_start).
+        pdf_floor: code with softmax_pdf_floor (no token is zero-width); the stream must be decoded with pdf_floor=True too."""
+        self.set_pdf_floor(pdf_floor)
         a, p = _u32(ids)
         n = a.shape[0]
         seg_start = split_segments(n, n_segments) if seg_start is None else np.asarray(seg_start, np.uint64)
@@ -266,8 +273,10 @@ class Model:
         pay = [data[int(seg_off[g]) : int(seg_off[g + 1])].tobytes() for g in range(int(s.n_segments))]
         return pay, seg_start
 
-    def decode(self, payloads, seg_start, bos=0, context=512, reprime_interval=512, max_batch_tokens=0, events=None):
-        """events: the same gated hint primes the encoder was given (src/main.rs:2586-2614), single segment only"""
+    def decode(self, payloads, seg_start, bos=0, context=512, reprime_interval=512, max_batch_tokens=0, events=None, pdf_floor=False):
+        """events: the same gated hint primes the encoder was given (src/main.rs:2586-2614), single segment only;
+        pdf_floor: the setting the stream was encoded with"""
+        self.set_pdf_floor(pdf_floor)
         seg_start = np.asarray(seg_start, np.uint64)
         n = int(seg_start[-1])
         s, keep = self._schedule(n, seg_start, bos, context, reprime_interval, events, max_batch_tokens)

@@ -91,8 +91,13 @@ def rwkv_detok_with_literals(tok: RwkvTokenizer, symbols, vocab_size: int) -> by
 
 
 def compress(model, data: bytes, tokenizer=None, n_segments=1, bos=0, context=512, reprime_interval=512, model_repr=b"model.safetensors",
-             model_hash16=b"\0" * 16, tokenizer_hash16=b"\0" * 16):
-    """bytes -> .canz container bytes.  n_segments == 1 gives the reference's v2 layout (header | payload)."""
+             model_hash16=b"\0" * 16, tokenizer_hash16=b"\0" * 16, on_zero_width="stored"):
+    """bytes -> .canz container bytes.  n_segments == 1 gives the reference's v2 layout (header | payload).
+    on_zero_width: what to do when the SmolLM coder meets a token it cannot code (CZ_ERR_ZERO_WIDTH): "stored" writes the bytes
+    uncoded (CZ_FLAG_STORED), "floor" codes the whole input again with the floored pdf (CZ_FLAG_PDF_FLOOR).  An input that codes
+    without such a token gives the same container either way."""
+    if on_zero_width not in ("stored", "floor"):
+        raise ValueError(f"on_zero_width must be 'stored' or 'floor', not {on_zero_width!r}")
     tokenizer = tokenizer or ByteTokenizer()
     vocab = int(model.cfg["vocab"])
     if model.cfg.get("arch", 0) == 1:
@@ -108,13 +113,16 @@ def compress(model, data: bytes, tokenizer=None, n_segments=1, bos=0, context=51
         if e.code != _lib.CZ_ERR_ZERO_WIDTH:
             raise
         # SmolLM coding has no probability floor (src/main.rs:2295): a token whose mass quantises to a zero-width interval cannot be
-        # coded -- the reference writes a corrupt stream there (SURVEY 7.3a).  Every input must still round-trip: store the bytes
-        # uncoded under the STORED flag (the message names the offending token index for whoever wants to know why).
-        sys.stderr.write(f"candlezip_b200: {e}; writing a STORED container\n")
-        return container.write_container(dict(fields, reserved_flags=_lib.CZ_FLAG_STORED), model_repr, [bytes(data)])
-    fields = dict(bos_token_id=bos, token_count=len(ids), orig_len_bytes=len(data), model_hash16=model_hash16,
-                  tokenizer_hash16=tokenizer_hash16, orig_hash16=container.blake3_16(data), context_window=context, vocab_size=vocab,
-                  reprime_interval=reprime_interval, reserved_flags=0)
+        # coded -- the reference writes a corrupt stream there (SURVEY 7.3a).  Every input must still round-trip: either code it with
+        # the floored pdf (softmax_pdf_floor, src/main.rs:758-767, under which no token is zero-width) or store the bytes uncoded
+        # (the message names the offending token index for whoever wants to know why).
+        if on_zero_width == "floor":
+            sys.stderr.write(f"candlezip_b200: {e}; coding with the floored pdf\n")
+            pays, seg = model.encode(ids, n_segments=n_segments, bos=bos, context=context, reprime_interval=reprime_interval, pdf_floor=True)
+            fields["reserved_flags"] = _lib.CZ_FLAG_PDF_FLOOR
+        else:
+            sys.stderr.write(f"candlezip_b200: {e}; writing a STORED container\n")
+            return container.write_container(dict(fields, reserved_flags=_lib.CZ_FLAG_STORED), model_repr, [bytes(data)])
     seg_tokens = np.diff(seg) if len(pays) > 1 else None
     return container.write_container(fields, model_repr, pays, seg_tokens=seg_tokens, engine=model.engine)
 
@@ -123,6 +131,9 @@ def decompress(model, blob: bytes, tokenizer=None, verify=True) -> bytes:
     tokenizer = tokenizer or ByteTokenizer()
     f, _, gates, _, seg_tokens, pays = container.read_container(blob)
     n = int(f["token_count"])
+    pdf_floor = bool(f["reserved_flags"] & _lib.CZ_FLAG_PDF_FLOOR)
+    if pdf_floor and (f["reserved_flags"] & _lib.CZ_FLAG_STORED or model.cfg.get("arch", 0) == 1):
+        raise ValueError("PDF_FLOOR marks a SmolLM payload coded with the floored pdf: invalid with STORED or on an RWKV-7 model")
     if f["reserved_flags"] & _lib.CZ_FLAG_STORED:
         data = b"".join(pays)
         if len(data) != int(f["orig_len_bytes"]) or (verify and container.blake3_16(data) != f["orig_hash16"]):
@@ -133,7 +144,8 @@ def decompress(model, blob: bytes, tokenizer=None, verify=True) -> bytes:
     seg = np.concatenate([[0], np.cumsum(seg_tokens)]).astype(np.uint64) if seg_tokens is not None else np.array([0, n], np.uint64)
     if int(seg[-1]) != n:
         raise ValueError("segment table does not add up to token_count")
-    ids = model.decode(pays, seg, bos=int(f["bos_token_id"]), context=int(f["context_window"]), reprime_interval=int(f["reprime_interval"]))
+    ids = model.decode(pays, seg, bos=int(f["bos_token_id"]), context=int(f["context_window"]), reprime_interval=int(f["reprime_interval"]),
+                       pdf_floor=pdf_floor)
     vocab = int(model.cfg["vocab"])
     if model.cfg.get("arch", 0) == 1 and isinstance(tokenizer, RwkvTokenizer):
         data = rwkv_detok_with_literals(tokenizer, ids, vocab)

@@ -212,7 +212,9 @@ __device__ __forceinline__ void cdf_col(const float *__restrict__ p_in, size_t l
   const bool uniform = (MODE == CZ_CDF_SMOLLM && OP != OP_XE) && (S <= 0.0);  // src/main.rs:794-798
   const double uni = 1.0 / (double)V;
 
-  if (MODE == CZ_CDF_RWKV_LITERALS || OP == OP_XE) {
+  // the floored SmolLM pdf: what OP_XE evaluates for every SmolLM mode, and what CZ_CDF_SMOLLM_FLOOR codes with
+  constexpr bool kFloorPdf = OP == OP_XE || MODE == CZ_CDF_SMOLLM_FLOOR;
+  if (MODE == CZ_CDF_RWKV_LITERALS || kFloorPdf) {
     // softmax_pdf_floor: norm = sum_i max(e_i / S, floor)   (src/main.rs:763-764)
     double acc = 0.0;
     cdf_walk<!kCache>(p, ld, V, [&](int, float x) {
@@ -241,7 +243,7 @@ __device__ __forceinline__ void cdf_col(const float *__restrict__ p_in, size_t l
       double q = __ddiv_rn((double)ex(x), S);
       q = __dmul_rn(__ddiv_rn(fmax(q, CZ_P_FLOOR), norm), scale);
       return sum2 > 0.0 ? __ddiv_rn(q, sum2) : q;
-    } else if (OP == OP_XE) {
+    } else if (kFloorPdf) {
       const double q = __ddiv_rn((double)ex(x), S);
       return __ddiv_rn(fmax(q, CZ_P_FLOOR), norm);
     } else {

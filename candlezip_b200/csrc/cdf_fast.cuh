@@ -148,7 +148,7 @@ __device__ __forceinline__ void cdf_walk_groups(const float *p, size_t ld, int n
 // per-column results of the full passes, consumed by the prefix / XE kernels
 struct __align__(16) CdfStats {
   double S;      // sum_i (f64)expf(l_i - max)                                        (src/main.rs:789-793)
-  double norm;   // sum_i max(e_i / S, 2^-29)          (softmax_pdf_floor, :763-764)  -- RWKV alphabet and XE only, else 1
+  double norm;   // sum_i max(e_i / S, 2^-29)          (softmax_pdf_floor, :763-764)  -- floored alphabets and XE only, else 1
   double sum2;   // combined_pdf_with_literals' second normaliser (:773-779)           -- RWKV alphabet only, else 1
   float mx;      // max_i l_i
   int pad;
@@ -310,7 +310,7 @@ __device__ __forceinline__ void cdf_search_warp_n(const float *const (&p)[NC], s
     sum2[c] = 1.0;
     any_uniform = any_uniform || (MODE == CZ_CDF_SMOLLM && S[c] <= 0.0);  // src/main.rs:794-798
   }
-  if (MODE == CZ_CDF_RWKV_LITERALS) {
+  if (MODE != CZ_CDF_SMOLLM) {  // softmax_pdf_floor's normaliser (src/main.rs:763-764): the RWKV and the floored SmolLM alphabet
     if (okS) {
       auto g = [&](int c, double e) { return fmax(cz_div_rcp(e, S[c], yS[c]), CZ_P_FLOOR); };
       seq_sum([&](int c, float x, bool &ok) { return g(c, ex_fast(c, x, ok)); }, [&](int c, float x) { return g(c, ex_slow(c, x)); }, norm);
@@ -318,6 +318,8 @@ __device__ __forceinline__ void cdf_search_warp_n(const float *const (&p)[NC], s
       auto g = [&](int c, double e) { return fmax(__ddiv_rn(e, S[c]), CZ_P_FLOOR); };
       seq_sum([&](int c, float x, bool &ok) { return g(c, ex_fast(c, x, ok)); }, [&](int c, float x) { return g(c, ex_slow(c, x)); }, norm);
     }
+  }
+  if (MODE == CZ_CDF_RWKV_LITERALS) {
     bool okN = okS;
 #pragma unroll
     for (int c = 0; c < NC; c++) {
@@ -443,6 +445,7 @@ __device__ __forceinline__ void cdf_search_warp_n(const float *const (&p)[NC], s
         const double q = __dmul_rn(__ddiv_rn(fmax(__ddiv_rn(e, S[c]), CZ_P_FLOOR), norm[c]), scale);
         return sum2[c] > 0.0 ? __ddiv_rn(q, sum2[c]) : q;
       }
+      if (MODE == CZ_CDF_SMOLLM_FLOOR) return __ddiv_rn(fmax(__ddiv_rn(e, S[c]), CZ_P_FLOOR), norm[c]);
       return S[c] <= 0.0 ? uni : __ddiv_rn(e, S[c]);
     };
     search([&](int, float, bool &ok) { ok = false; return 0.0; }, [&](int c, float x) { return g(c, ex_slow(c, x)); });
@@ -451,6 +454,9 @@ __device__ __forceinline__ void cdf_search_warp_n(const float *const (&p)[NC], s
     auto g = [&](int c, double e) {
       return cz_div_rcp(__dmul_rn(cz_div_rcp(fmax(cz_div_rcp(e, S[c], yS[c]), CZ_P_FLOOR), norm[c], yN[c]), scale), sum2[c], y2[c]);
     };
+    search([&](int c, float x, bool &ok) { return g(c, ex_fast(c, x, ok)); }, [&](int c, float x) { return g(c, ex_slow(c, x)); });
+  } else if (MODE == CZ_CDF_SMOLLM_FLOOR) {
+    auto g = [&](int c, double e) { return cz_div_rcp(fmax(cz_div_rcp(e, S[c], yS[c]), CZ_P_FLOOR), norm[c], yN[c]); };
     search([&](int c, float x, bool &ok) { return g(c, ex_fast(c, x, ok)); }, [&](int c, float x) { return g(c, ex_slow(c, x)); });
   } else {
     search([&](int c, float x, bool &ok) { return cz_div_rcp(ex_fast(c, x, ok), S[c], yS[c]); },

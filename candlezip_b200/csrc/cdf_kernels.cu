@@ -61,13 +61,13 @@ __global__ void __launch_bounds__(128) cdf_cols_kernel(const float *__restrict__
 // Full passes.  One thread owns NCOL adjacent columns (vector loads: one LDG + one address per NCOL logits); every column is still
 // summed by one thread in ascending vocab order.  MODE / OP decide which passes run:
 //   pass 1  S = sum (f64)expf(l - max)                      always            (RWKV alphabet: leaves e_v in the logit's slot)
-//   pass 2  norm = sum max(e / S, 2^-29)                    RWKV alphabet, XE
+//   pass 2  norm = sum max(e / S, 2^-29)                    RWKV alphabet, floored SmolLM alphabet, XE
 //   pass 3  sum2 = sum RN(RN(max(e / S, 2^-29) / norm) (1 - 2^-21)) + 256 x 2^-29   RWKV alphabet
 template <int MODE, int OP, int NCOL>
 __global__ void __launch_bounds__(128) cdf_stats_kernel(float *__restrict__ logits, int V, size_t M, size_t ld, const int *__restrict__ colmax,
                                                         CdfStats *__restrict__ stats, int *__restrict__ err) {
   constexpr bool kLit = MODE == CZ_CDF_RWKV_LITERALS;
-  constexpr bool kNorm = kLit || OP == OP_XE;
+  constexpr bool kNorm = kLit || OP == OP_XE || MODE == CZ_CDF_SMOLLM_FLOOR;
   constexpr int GRP = NCOL == 4 ? 4 : 8;
   constexpr int NE = GRP * NCOL;
   __shared__ uint64_t s_tab[32 * 32];
@@ -141,7 +141,7 @@ __global__ void __launch_bounds__(128) cdf_stats_kernel(float *__restrict__ logi
       fast = fast && cz_div_rcp_ok(S[c]);
       yS[c] = __drcp_rn(S[c]);
     }
-    // e_v (as a double) of the rows of a group: the cached f32 (RWKV alphabet) or recomputed from the logit (SmolLM XE)
+    // e_v (as a double) of the rows of a group: the cached f32 (RWKV alphabet) or recomputed from the logit (SmolLM: floored / XE)
     auto e_of = [&](const typename CdfVec<NCOL>::T(&rows)[GRP], double(&d)[NE]) {
       float a[NE], ef[NE];
 #pragma unroll
@@ -308,7 +308,7 @@ __global__ void __launch_bounds__(ST_COLS + 32, 2) cdf_stats_tma_kernel(const __
                                                                        const uint32_t *__restrict__ syms, const uint32_t *__restrict__ eoff,
                                                                        double *__restrict__ ecache, const int *__restrict__ eflag) {
   constexpr bool kLit = MODE == CZ_CDF_RWKV_LITERALS;
-  constexpr bool kNorm = kLit || OP == OP_XE;
+  constexpr bool kNorm = kLit || OP == OP_XE || MODE == CZ_CDF_SMOLLM_FLOOR;
   constexpr bool kSpill = OP == OP_BOUNDS;  // (ecache may still be null: no e-cache for this batch)
   constexpr int ST_ROWS = StCfg<MODE>::ROWS, ST_STAGES = StCfg<MODE>::STAGES, ST_TILE_BYTES = StCfg<MODE>::TILE_BYTES;
   extern __shared__ __align__(1024) uint8_t st_smem[];
@@ -445,7 +445,7 @@ __global__ void __launch_bounds__(ST_COLS + 32, 2) cdf_stats_tma_kernel(const __
     const bool fast = __all_sync(0xffffffffu, cz_div_rcp_ok(S));
     const double yS = __drcp_rn(S);
     // e_v of the 8 rows: the cached f32 (RWKV alphabet; WIDEN: exact integer widening, values below 2^-126 are floored either way)
-    // or expf again (SmolLM's XE pass)
+    // or expf again (SmolLM's floored alphabet and XE pass)
     auto e_of = [&](const float(&x)[8], double(&d)[8], auto widen) {
       if (kLit) {
 #pragma unroll
@@ -605,7 +605,7 @@ __global__ void __launch_bounds__(256) cdf_bounds_warp_kernel(const float *__res
       continue;
     }
     const CdfStats st = stats[col];
-    PdfOf<MODE, false> pdf;
+    PdfOf<MODE, MODE == CZ_CDF_SMOLLM_FLOOR> pdf;
     pdf.init(st, V);
     const float mx = st.mx;
     const float *p = logits + col;
@@ -860,12 +860,14 @@ __global__ void cdf_full_kernel(const float *__restrict__ logits, int V, uint32_
   for (int v = 0; v < V; v++) S = __dadd_rn(S, (double)cz_expf(__fsub_rn(logits[v], mx), tab));
   double norm = 1.0, sum2 = 1.0;
   const double scale = 1.0 - 256.0 * CZ_P_FLOOR;
-  if (MODE == CZ_CDF_RWKV_LITERALS) {
+  if (MODE != CZ_CDF_SMOLLM) {
     double acc = 0.0;
     for (int v = 0; v < V; v++)
       acc = __dadd_rn(acc, fmax(__ddiv_rn((double)cz_expf(__fsub_rn(logits[v], mx), tab), S), CZ_P_FLOOR));
     norm = acc;
-    acc = 0.0;
+  }
+  if (MODE == CZ_CDF_RWKV_LITERALS) {
+    double acc = 0.0;
     for (int v = 0; v < V; v++) {
       double q = fmax(__ddiv_rn((double)cz_expf(__fsub_rn(logits[v], mx), tab), S), CZ_P_FLOOR);
       acc = __dadd_rn(acc, __dmul_rn(__ddiv_rn(q, norm), scale));
@@ -887,6 +889,8 @@ __global__ void cdf_full_kernel(const float *__restrict__ logits, int V, uint32_
         q = CZ_P_FLOOR;
       }
       if (sum2 > 0.0) q = __ddiv_rn(q, sum2);
+    } else if (MODE == CZ_CDF_SMOLLM_FLOOR) {
+      q = __ddiv_rn(fmax(__ddiv_rn((double)cz_expf(__fsub_rn(logits[v], mx), tab), S), CZ_P_FLOOR), norm);
     } else {
       q = uniform ? 1.0 / (double)V : __ddiv_rn((double)cz_expf(__fsub_rn(logits[v], mx), tab), S);
     }
@@ -948,11 +952,17 @@ static int make_logits_map(CUtensorMap *map, const float *logits, size_t V, size
 int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size_t V, size_t M, size_t ld,
                     const uint32_t *arg_dev, uint32_t *sym_out_dev, uint32_t *c_lo_dev, uint32_t *c_hi_dev,
                     double *xe_dev, cudaStream_t stream, const int *colmax_dev) {
+  if (mode != CZ_CDF_SMOLLM && mode != CZ_CDF_RWKV_LITERALS && mode != CZ_CDF_SMOLLM_FLOOR) {
+    set_error("cdf: unknown mode");
+    return CZ_ERR_INVALID;
+  }
   if (M == 0) return CZ_OK;
   if (V == 0 || V > (1u << 24) || ld < M) {
     set_error("cdf: bad shape");
     return CZ_ERR_INVALID;
   }
+  // OP_XE evaluates the floored pdf for SmolLM whatever the coding alphabet (src/main.rs:1745): mode 2 IS mode 0 there
+  if (op == czk::OP_XE && mode == CZ_CDF_SMOLLM_FLOOR) mode = CZ_CDF_SMOLLM;
   if (op == czk::OP_SEARCH && M <= 8192) {  // decode-sized: warp per column
     const unsigned g = (unsigned)ceil_div(M, 8);  // 4 warps x 2 columns
     if (mode == CZ_CDF_SMOLLM)
@@ -963,10 +973,10 @@ int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size
       CZ_LAUNCH(ctx, CZ_K_CDF,
                 (czk::cdf_search_warp_kernel<CZ_CDF_RWKV_LITERALS><<<g, 128, 0, stream>>>(logits_dev, (int)V, M, ld, arg_dev, sym_out_dev,
                                                                                           c_lo_dev, c_hi_dev, ctx->err_flag_dev, colmax_dev)));
-    else {
-      set_error("cdf: unknown mode");
-      return CZ_ERR_INVALID;
-    }
+    else
+      CZ_LAUNCH(ctx, CZ_K_CDF,
+                (czk::cdf_search_warp_kernel<CZ_CDF_SMOLLM_FLOOR><<<g, 128, 0, stream>>>(logits_dev, (int)V, M, ld, arg_dev, sym_out_dev,
+                                                                                         c_lo_dev, c_hi_dev, ctx->err_flag_dev, colmax_dev)));
     CZ_CHECK_LAUNCH();
     return CZ_OK;
   }
@@ -1060,6 +1070,7 @@ int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size
         CZ_TMA_ATTR(CZ_CDF_SMOLLM, czk::OP_XE);
         CZ_TMA_ATTR(CZ_CDF_RWKV_LITERALS, czk::OP_BOUNDS);
         CZ_TMA_ATTR(CZ_CDF_RWKV_LITERALS, czk::OP_XE);
+        CZ_TMA_ATTR(CZ_CDF_SMOLLM_FLOOR, czk::OP_BOUNDS);
 #undef CZ_TMA_ATTR
         attr = true;
       }
@@ -1075,8 +1086,7 @@ int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size
         if (op == czk::OP_BOUNDS) CZ_TMA_STATS(CZ_CDF_RWKV_LITERALS, czk::OP_BOUNDS);
         else CZ_TMA_STATS(CZ_CDF_RWKV_LITERALS, czk::OP_XE);
       } else {
-        set_error("cdf: unknown mode");
-        return CZ_ERR_INVALID;
+        CZ_TMA_STATS(CZ_CDF_SMOLLM_FLOOR, czk::OP_BOUNDS);  // (OP_XE runs as mode 0)
       }
 #undef CZ_TMA_STATS
       CZ_CHECK_LAUNCH();
@@ -1099,8 +1109,7 @@ int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size
       if (op == czk::OP_BOUNDS) CZ_STATS_N(CZ_CDF_RWKV_LITERALS, czk::OP_BOUNDS);
       else CZ_STATS_N(CZ_CDF_RWKV_LITERALS, czk::OP_XE);
     } else {
-      set_error("cdf: unknown mode");
-      return CZ_ERR_INVALID;
+      CZ_STATS_N(CZ_CDF_SMOLLM_FLOOR, czk::OP_BOUNDS);  // (OP_XE runs as mode 0)
     }
 #undef CZ_STATS_N
 #undef CZ_STATS
@@ -1120,9 +1129,12 @@ int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size
       if (mode == CZ_CDF_SMOLLM) {
         if (ecache) CZ_PREFIX(CZ_CDF_SMOLLM, true);
         CZ_PREFIX(CZ_CDF_SMOLLM, false);
-      } else {
+      } else if (mode == CZ_CDF_RWKV_LITERALS) {
         if (ecache) CZ_PREFIX(CZ_CDF_RWKV_LITERALS, true);
         CZ_PREFIX(CZ_CDF_RWKV_LITERALS, false);
+      } else {
+        if (ecache) CZ_PREFIX(CZ_CDF_SMOLLM_FLOOR, true);
+        CZ_PREFIX(CZ_CDF_SMOLLM_FLOOR, false);
       }
 #undef CZ_PREFIX
     } else {
@@ -1153,8 +1165,8 @@ int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size
     else if (op == czk::OP_SEARCH) CZ_CDF_CASE(CZ_CDF_RWKV_LITERALS, czk::OP_SEARCH);
     else CZ_CDF_CASE(CZ_CDF_RWKV_LITERALS, czk::OP_XE);
   } else {
-    set_error("cdf: unknown mode");
-    return CZ_ERR_INVALID;
+    if (op == czk::OP_BOUNDS) CZ_CDF_CASE(CZ_CDF_SMOLLM_FLOOR, czk::OP_BOUNDS);
+    else CZ_CDF_CASE(CZ_CDF_SMOLLM_FLOOR, czk::OP_SEARCH);  // (OP_XE runs as mode 0)
   }
 #undef CZ_CDF_CASE
   CZ_CHECK_LAUNCH();
@@ -1164,9 +1176,15 @@ int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size
 int launch_cdf_full(cz_ctx *ctx, int mode, const float *logits_dev, size_t V, uint32_t *cdf_dev, cudaStream_t stream) {
   if (mode == CZ_CDF_SMOLLM)
     CZ_LAUNCH(ctx, CZ_K_CDF, (czk::cdf_full_kernel<CZ_CDF_SMOLLM><<<1, 32, 0, stream>>>(logits_dev, (int)V, cdf_dev)));
-  else
+  else if (mode == CZ_CDF_RWKV_LITERALS)
     CZ_LAUNCH(ctx, CZ_K_CDF,
               (czk::cdf_full_kernel<CZ_CDF_RWKV_LITERALS><<<1, 32, 0, stream>>>(logits_dev, (int)V, cdf_dev)));
+  else if (mode == CZ_CDF_SMOLLM_FLOOR)
+    CZ_LAUNCH(ctx, CZ_K_CDF, (czk::cdf_full_kernel<CZ_CDF_SMOLLM_FLOOR><<<1, 32, 0, stream>>>(logits_dev, (int)V, cdf_dev)));
+  else {
+    set_error("cdf: unknown mode");
+    return CZ_ERR_INVALID;
+  }
   CZ_CHECK_LAUNCH();
   return CZ_OK;
 }

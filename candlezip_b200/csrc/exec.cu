@@ -172,6 +172,7 @@ static void decode_set_carveout() {
   const auto mx = cudaSharedmemCarveoutMaxShared;
   cudaFuncSetAttribute(czk::decode_step_kernel<CZ_CDF_SMOLLM>, cudaFuncAttributePreferredSharedMemoryCarveout, mx);
   cudaFuncSetAttribute(czk::decode_step_kernel<CZ_CDF_RWKV_LITERALS>, cudaFuncAttributePreferredSharedMemoryCarveout, mx);
+  cudaFuncSetAttribute(czk::decode_step_kernel<CZ_CDF_SMOLLM_FLOOR>, cudaFuncAttributePreferredSharedMemoryCarveout, mx);
   cudaFuncSetAttribute(czk::fill_pos_from_ctr_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, mx);
   cudaFuncSetAttribute(czk::advance_ctr_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, mx);
 }
@@ -202,10 +203,14 @@ int launch_decode_step(cz_ctx *ctx, int mode, const float *logits, int V, size_t
     CZ_LAUNCH(ctx, CZ_K_CDF,
               (czk::decode_step_kernel<CZ_CDF_SMOLLM><<<grid, czk::DS_WARPS * 32, 0, st>>>(logits, V, ld, n_lanes, payload, seg_off, seg_start, coded_index, ds,
                                                                             ids_out, next_tok, ctx->err_flag_dev, colmax, ctr)));
-  else
+  else if (mode == CZ_CDF_RWKV_LITERALS)
     CZ_LAUNCH(ctx, CZ_K_CDF,
               (czk::decode_step_kernel<CZ_CDF_RWKV_LITERALS><<<grid, czk::DS_WARPS * 32, 0, st>>>(logits, V, ld, n_lanes, payload, seg_off, seg_start, coded_index,
                                                                                    ds, ids_out, next_tok, ctx->err_flag_dev, colmax, ctr)));
+  else
+    CZ_LAUNCH(ctx, CZ_K_CDF,
+              (czk::decode_step_kernel<CZ_CDF_SMOLLM_FLOOR><<<grid, czk::DS_WARPS * 32, 0, st>>>(logits, V, ld, n_lanes, payload, seg_off, seg_start, coded_index,
+                                                                                  ds, ids_out, next_tok, ctx->err_flag_dev, colmax, ctr)));
   CZ_CHECK_LAUNCH();
   return CZ_OK;
 }
@@ -431,7 +436,9 @@ static int check_schedule_ids(const cz_model *m, const cz_schedule *s) {
   return CZ_OK;
 }
 
-static int coded_mode(const cz_model *m) { return m->cfg.arch == CZ_ARCH_RWKV7 ? CZ_CDF_RWKV_LITERALS : CZ_CDF_SMOLLM; }
+static int arch_mode(const cz_model *m) { return m->cfg.arch == CZ_ARCH_RWKV7 ? CZ_CDF_RWKV_LITERALS : CZ_CDF_SMOLLM; }
+// the alphabet cz_encode / cz_decode code with (cz_model_set_pdf_floor only ever sets pdf_floor on a SmolLM model)
+static int coded_mode(const cz_model *m) { return m->pdf_floor ? CZ_CDF_SMOLLM_FLOOR : arch_mode(m); }
 
 // Core of cz_encode / cz_encode_dev: ids already on the device.  Leaves the compacted payload in out_dev
 // (device) and the per-segment offsets in seg_off_host.
@@ -995,7 +1002,7 @@ int cz_xe_bits(cz_model *m, const cz_xe_job *jobs, size_t n_jobs, double *bits_o
     if (w.n_rows() == 0) return CZ_OK;
     CZ_TRY(d_src.reserve(w.n_rows() * 8, st));
     CZ_TRY(run_wave_trunk(m, w, nullptr, d_extra.as<uint32_t>(), 0, d_src.as<long long>(), st));
-    CZ_TRY(run_wave_head(m, w.n_logit(), czk::OP_XE, coded_mode(m), d_tgt.as<uint32_t>() + col_first, nullptr, nullptr,
+    CZ_TRY(run_wave_head(m, w.n_logit(), czk::OP_XE, arch_mode(m), d_tgt.as<uint32_t>() + col_first, nullptr, nullptr,
                          d_bits.as<double>() + col_first, st));
     col_first += w.n_logit();
     w.clear();

@@ -125,6 +125,8 @@ struct cz_model {
   // cz_encode / cz_encode_dev / cz_decode and the 16-byte digests are copied here (index = global coded index)
   uint8_t *digest_host = nullptr;
   size_t digest_cap = 0;
+  // cz_model_set_pdf_floor: SmolLM streams are coded with CZ_CDF_SMOLLM_FLOOR (exec.cu, coded_mode)
+  bool pdf_floor = false;
 };
 
 namespace cz {

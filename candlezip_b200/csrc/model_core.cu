@@ -525,6 +525,15 @@ int cz_model_config_get(const cz_model *m, cz_model_config *out) {
   *out = m->cfg;
   return CZ_OK;
 }
+int cz_model_set_pdf_floor(cz_model *m, int enabled) {
+  if (!m) return CZ_ERR_INVALID;
+  if (enabled && m->cfg.arch != CZ_ARCH_SMOLLM) {
+    set_error("pdf floor: only the SmolLM alphabet has an unfloored pdf (RWKV-7 codes with a floor already)");
+    return CZ_ERR_UNSUPPORTED;
+  }
+  m->pdf_floor = enabled != 0;
+  return CZ_OK;
+}
 int cz_model_tensor_count(const cz_model *m) { return m ? (int)m->tensors.size() : 0; }
 int cz_model_tensor_info(const cz_model *m, int idx, const char **name, size_t *n_elems) {
   if (!m || idx < 0 || idx >= (int)m->tensors.size()) return CZ_ERR_INVALID;

@@ -76,7 +76,13 @@ int cz_profile_read(cz_ctx *ctx, double ms_out[CZ_K_FAMILIES], uint64_t launches
 /* ---------------------------------------------------------------- K1: logits -> integer CDF */
 enum {
   CZ_CDF_SMOLLM = 0,        /* softmax_pdf, no floor: src/main.rs:2294-2296 */
-  CZ_CDF_RWKV_LITERALS = 1  /* floor 2^-29, 256 literal symbols appended: src/main.rs:2303-2321 */
+  CZ_CDF_RWKV_LITERALS = 1, /* floor 2^-29, 256 literal symbols appended: src/main.rs:2303-2321 */
+  CZ_CDF_SMOLLM_FLOOR = 2   /* quantize_pdf_to_cdf(softmax_pdf_floor(logits, 2^-29)) over the V vocabulary symbols (src/main.rs:758-767):
+                               the SmolLM alphabet with the floor the reference's RWKV coder and gate XE use.  No symbol is ever
+                               zero-width: with f = 2^-29, p_i = max(e_i / S, f) / norm and norm <= 1 + V f (+ rounding), p_i 2^30 >=
+                               2 / norm > 1 whenever V < 2^29, so consecutive partial sums differ by more than one quantum and every
+                               cdf[i+1] - cdf[i] >= 1 (no partial sum before the last reaches 1; the clamp at 2^30 only touches
+                               cdf[V]).  For cz_xe_bits_cols the mode is the same as CZ_CDF_SMOLLM (which already floors there). */
 };
 /* logits are VOCAB-MAJOR: logits[v * ld + m], m = 0..M-1 (one column per stream/token), ld >= M.
  * For each column m: (c_lo, c_hi) = (cdf[sym], cdf[sym+1]) of the reference's quantised CDF, bit-exact.
@@ -211,6 +217,12 @@ int cz_encode_dev(cz_model *m, const uint32_t *ids_dev, size_t n_tokens, const c
  * equal byte for byte (decode safety), whatever the wave size, batch size or GPU count.  NULL disables.  (RWKV-7: encode only.) */
 int cz_model_set_digest_out(cz_model *m, uint8_t *digests_out, size_t cap_tokens);
 
+/* enabled != 0: cz_encode / cz_encode_dev / cz_decode code SmolLM streams with CZ_CDF_SMOLLM_FLOOR instead of CZ_CDF_SMOLLM, so no
+ * token can be zero-width (CZ_ERR_ZERO_WIDTH cannot occur); the stream must be decoded with the same setting (the container's
+ * CZ_FLAG_PDF_FLOOR).  cz_xe_bits, the session shim and cz_chunk_logits are unaffected.  Off when the model is created.
+ * RWKV-7: enabled != 0 returns CZ_ERR_UNSUPPORTED (its alphabet is floored already). */
+int cz_model_set_pdf_floor(cz_model *m, int enabled);
+
 typedef struct {
   const uint32_t *prime;     /* tail(history, 511-|hint|) ++ hint, built by the caller or cz_xe_make_prime */
   uint32_t prime_len;
@@ -246,6 +258,9 @@ typedef struct {
 #define CZ_FLAG_STORED (1u << 9)   /* extension: the payload is the original bytes, uncoded.  Written by the file-level compress()
                                       when the SmolLM coder meets a symbol of mass < 2^-30 (CZ_ERR_ZERO_WIDTH: softmax_pdf has no
                                       floor, src/main.rs:2295; the reference would emit a corrupt stream there, SURVEY 7.3a) */
+#define CZ_FLAG_PDF_FLOOR (1u << 10) /* extension: the payload was coded with the floored SmolLM pdf (CZ_CDF_SMOLLM_FLOOR,
+                                        cz_model_set_pdf_floor).  Written by compress(on_zero_width="floor") when the unfloored pdf
+                                        meets a zero-width symbol; never together with CZ_FLAG_STORED, never on RWKV-7 */
 
 size_t cz_container_header_size(const cz_header_v2 *h);
 /* writes header (+repr); returns bytes written or 0 if cap is too small */
