@@ -6,6 +6,8 @@ Weights: --weights *.safetensors (HF LLaMA / candle_rwkv7 tensor names) or --ran
 Tokenizer: --tokenizer tokenizer.json (HF `tokenizers`, SmolLM) or a RWKV vocab json; default = byte-level ids (lossless for
 every input).  --segments N > 1 writes the SEG1 container extension (parallel decode); N = 1 is the reference's v2 layout.
 --on-zero-width {stored,floor}: what compress does when the SmolLM coder meets a token of mass < 2^-30 (codec.compress).
+compress-many / decompress-many IN... [--out-dir DIR]: many files through one encode call and lock-step decode waves of at most
+--max-streams streams (codec.compress_many / decompress_many); each .canz is the one `compress` writes for that file.
 """
 import argparse
 import sys
@@ -96,15 +98,40 @@ def _scan_decompress(model, tok, blob, args):
     return data
 
 
+def _main_many(args, ap):
+    """compress-many / decompress-many: every input in one codec.compress_many / decompress_many call"""
+    import os
+
+    ext = ".canz" if args.command == "compress-many" else ".out"
+    outs = [os.path.join(args.out_dir or os.path.dirname(p), os.path.basename(p) + ext) for p in args.input]
+    if len(set(map(os.path.abspath, outs))) != len(outs):
+        ap.error("two inputs would write the same output file")
+    model, tok = _model(args)
+    datas = [open(p, "rb").read() for p in args.input]
+    t0 = time.perf_counter()
+    if args.command == "compress-many":
+        res = codec.compress_many(model, datas, tok, args.segments, context=args.context, reprime_interval=args.reprime_interval,
+                                  on_zero_width=args.on_zero_width or "stored")
+    else:
+        res = codec.decompress_many(model, datas, tok, max_streams=args.max_streams)
+    dt = time.perf_counter() - t0
+    if args.out_dir:
+        os.makedirs(args.out_dir, exist_ok=True)
+    for path, blob in zip(outs, res):
+        open(path, "wb").write(blob)
+    n_in, n_out = sum(map(len, datas)), sum(map(len, res))
+    print(f"{len(datas)} files: {n_in} -> {n_out} bytes in {dt:.3f} s")
+    return 0
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(prog="candlezip_b200")
-    ap.add_argument("command", choices=["compress", "decompress", "self-test"])
-    ap.add_argument("input")
-    ap.add_argument("output", nargs="?")
+    ap.add_argument("command", choices=["compress", "decompress", "self-test", "compress-many", "decompress-many"])
+    ap.add_argument("input", nargs="+", help="INPUT [OUTPUT]; compress-many / decompress-many: one or more inputs")
     ap.add_argument("--backend", choices=["smollm", "rwkv7"], default="smollm")
     ap.add_argument("--context", type=int, default=512)
     ap.add_argument("--reprime-interval", type=int, default=512)
-    ap.add_argument("--segments", type=int, default=1)
+    ap.add_argument("--segments", type=int, help="independently coded segments per file (compress / self-test / compress-many); default 1")
     ap.add_argument("--weights", nargs="*")
     ap.add_argument("--random-init", type=int, default=0)
     ap.add_argument("--tokenizer")
@@ -119,7 +146,27 @@ def main(argv=None):
     ap.add_argument("--scan-gate-threshold-abs-bits", type=float, default=0.0)
     ap.add_argument("--scan-gate-threshold-pct", type=float, default=0.0)
     ap.add_argument("--scan-output-dir", help="where the proof.csv ledger of a scan goes")
+    ap.add_argument("--out-dir", help="compress-many / decompress-many: where NAME.canz / NAME.out go (default: beside each input)")
+    ap.add_argument("--max-streams", type=int, help="decompress-many: most segments decoded together in one lock-step wave; default 2048")
     args = ap.parse_args(argv)
+    # flags that only one side uses are refused on the other instead of being ignored
+    if args.command == "decompress-many" and (args.segments is not None or args.on_zero_width):
+        ap.error("--segments and --on-zero-width are compress settings: a container carries its own (decompress-many)")
+    if args.command != "decompress-many" and args.max_streams is not None:
+        ap.error("--max-streams applies to decompress-many only")
+    if args.segments is None:
+        args.segments = 1
+    if args.command.endswith("-many"):
+        if args.reuse_scan_dir:
+            ap.error("--reuse-scan-dir codes one file at a time: not available with compress-many / decompress-many")
+        if args.max_streams is None:
+            args.max_streams = 2048
+        if args.max_streams < 1:
+            ap.error("--max-streams must be >= 1")
+        return _main_many(args, ap)
+    if len(args.input) > 2:
+        ap.error(f"{args.command} takes INPUT [OUTPUT]")
+    args.input, args.output = args.input[0], (args.input[1] if len(args.input) > 1 else None)
     scan = bool(args.reuse_scan_dir)
     if scan and (args.backend != "smollm" or args.segments != 1):
         ap.error("--reuse-scan-dir works on the SmolLM backend with one AC stream (--segments 1), like the reference's container")

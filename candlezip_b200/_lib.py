@@ -29,6 +29,7 @@ CZ_ENGINE_TCGEN05, CZ_ENGINE_SIMT = 0, 1
 CZ_FLAG_SEGMENTS = 1 << 8
 CZ_FLAG_STORED = 1 << 9
 CZ_FLAG_PDF_FLOOR = 1 << 10
+NO_ZERO_WIDTH = 2 ** 64 - 1  # cz_model_set_zero_width_out: the segment has no zero-width token
 K_FAMILIES = ("gemm_qkv", "attn", "elemwise", "cdf", "coder", "other", "gemm_o", "gemm_gu", "gemm_down", "gemm_head", "cdf_prefix")
 
 
@@ -127,6 +128,7 @@ SIGNATURES = {
     "cz_encode_dev": (C.c_int, [_vp, _vp, C.c_size_t, C.POINTER(Schedule), _vp, C.c_size_t, u64p]),
     "cz_model_set_digest_out": (C.c_int, [_vp, u8p, C.c_size_t]),
     "cz_model_set_pdf_floor": (C.c_int, [_vp, C.c_int]),
+    "cz_model_set_zero_width_out": (C.c_int, [_vp, u64p, C.c_size_t]),
     "cz_xe_bits": (C.c_int, [_vp, C.POINTER(XeJob), C.c_size_t, f64p]),
     "cz_chunk_logits": (C.c_int, [_vp, u32p, C.c_size_t, u32p, C.c_size_t, f32p]),
     "cz_container_header_size": (C.c_size_t, [C.POINTER(HeaderV2)]),

@@ -257,9 +257,12 @@ class Model:
         check(lib.cz_model_set_pdf_floor(self._h, 1 if enabled else 0))
 
     def encode(self, ids, n_segments=1, bos=0, context=512, reprime_interval=512, events=None, seg_start=None, max_batch_tokens=0,
-               pdf_floor=False):
+               pdf_floor=False, zero_width_out=False):
         """ids: coded tokens (no BOS). Returns (list of per-segment payload bytes, seg_start).
-        pdf_floor: code with softmax_pdf_floor (no token is zero-width); the stream must be decoded with pdf_floor=True too."""
+        pdf_floor: code with softmax_pdf_floor (no token is zero-width); the stream must be decoded with pdf_floor=True too.
+        zero_width_out: a zero-width token does not raise CZ_ERR_ZERO_WIDTH; returns (payloads, seg_start, first_zw) instead, first_zw
+        a uint64 array with each segment's segment-relative index of its first zero-width token or _lib.NO_ZERO_WIDTH (a segment with
+        an index has an unspecified payload: cz_model_set_zero_width_out)."""
         self.set_pdf_floor(pdf_floor)
         a, p = _u32(ids)
         n = a.shape[0]
@@ -269,9 +272,17 @@ class Model:
         data = np.empty(cap, np.uint8)
         seg_off = np.zeros(int(s.n_segments) + 1, np.uint64)
         bs = _lib.Bitstreams(data.ctypes.data_as(_lib.u8p), cap, seg_off.ctypes.data_as(_lib.u64p))
-        check(lib.cz_encode(self._h, p, n, C.byref(s), C.byref(bs)))
+        if not zero_width_out:
+            check(lib.cz_encode(self._h, p, n, C.byref(s), C.byref(bs)))
+        else:
+            first_zw = np.zeros(max(1, int(s.n_segments)), np.uint64)
+            check(lib.cz_model_set_zero_width_out(self._h, first_zw.ctypes.data_as(_lib.u64p), first_zw.shape[0]))
+            try:
+                check(lib.cz_encode(self._h, p, n, C.byref(s), C.byref(bs)))
+            finally:
+                check(lib.cz_model_set_zero_width_out(self._h, None, 0))
         pay = [data[int(seg_off[g]) : int(seg_off[g + 1])].tobytes() for g in range(int(s.n_segments))]
-        return pay, seg_start
+        return (pay, seg_start, first_zw[: int(s.n_segments)]) if zero_width_out else (pay, seg_start)
 
     def decode(self, payloads, seg_start, bos=0, context=512, reprime_interval=512, max_batch_tokens=0, events=None, pdf_floor=False):
         """events: the same gated hint primes the encoder was given (src/main.rs:2586-2614), single segment only;

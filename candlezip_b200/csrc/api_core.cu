@@ -30,7 +30,7 @@ int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size
 int launch_cdf_full(cz_ctx *ctx, int mode, const float *logits_dev, size_t V, uint32_t *cdf_dev, cudaStream_t stream);
 int launch_ac_encode_lanes(cz_ctx *ctx, const uint32_t *c_lo_dev, const uint32_t *c_hi_dev, const uint64_t *lane_off_dev,
                            size_t n_lanes, uint8_t *out_dev, const uint64_t *out_off_dev, uint64_t *out_len_dev,
-                           unsigned long long *err_index_dev, cudaStream_t stream);
+                           unsigned long long *err_index_dev, cudaStream_t stream, unsigned long long *lane_zw_dev = nullptr);
 int launch_ac_decode_lanes_static(cz_ctx *ctx, const uint8_t *payload_dev, const uint64_t *pay_off_dev,
                                   const uint64_t *pay_len_dev, const uint64_t *lane_off_dev, size_t n_lanes,
                                   const uint32_t *cdf_dev, uint32_t n_sym, uint32_t *syms_dev, cudaStream_t stream);
@@ -47,8 +47,9 @@ int require_device(cz_ctx *ctx) {
   return CZ_OK;
 }
 
-// reads and clears the device status word; maps it to a cz_status
-int fetch_device_status(cz_ctx *ctx, unsigned long long *err_index_dev, unsigned long long *err_index_out) {
+// reads and clears the device status word; maps it to a cz_status.  ignore_bits: status bits the caller reports some other way
+// (the zero-width bit when a per-segment zero-width sink is set)
+int fetch_device_status_masked(cz_ctx *ctx, unsigned long long *err_index_dev, unsigned long long *err_index_out, int ignore_bits) {
   int flag = 0;
   CZ_CUDA_TRY(cudaMemcpyAsync(&flag, ctx->err_flag_dev, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
   unsigned long long idx = ~0ull;
@@ -57,6 +58,7 @@ int fetch_device_status(cz_ctx *ctx, unsigned long long *err_index_dev, unsigned
   CZ_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
   if (flag) CZ_CUDA_TRY(cudaMemsetAsync(ctx->err_flag_dev, 0, sizeof(int), ctx->stream));
   if (err_index_out) *err_index_out = idx;
+  flag &= ~ignore_bits;
   if (flag & 2) {  // (checked before the zero-width bit: an out-of-range symbol also yields an empty interval)
     set_error("symbol id out of range for the coded alphabet");
     return CZ_ERR_SYMBOL_RANGE;
@@ -71,6 +73,9 @@ int fetch_device_status(cz_ctx *ctx, unsigned long long *err_index_dev, unsigned
     return CZ_ERR_INVALID;
   }
   return CZ_OK;
+}
+int fetch_device_status(cz_ctx *ctx, unsigned long long *err_index_dev, unsigned long long *err_index_out) {
+  return fetch_device_status_masked(ctx, err_index_dev, err_index_out, 0);
 }
 
 }  // namespace cz

@@ -11,14 +11,18 @@ namespace czk {
 // One WARP per lane: the 32 threads prefetch the next AC_BATCH intervals into shared memory with coalesced loads and
 // flush the produced bytes with coalesced stores; thread 0 runs the (inherently sequential) coder out of shared memory.
 // A single thread reading (c_lo, c_hi) straight from global memory pays a full DRAM round trip per symbol.
-// err[0]: OR of status bits; err_index: smallest interval index that had zero width (atomicMin)
+// err[0]: OR of status bits; err_index: smallest interval index that had zero width (atomicMin).
+// LANE_ZW (cz_model_set_zero_width_out): every lane also writes lane_zw[lane], the lane-relative index of its own first zero-width
+// interval or ~0 when it has none, so that one segment's zero-width token does not make the caller re-code the other segments.
 constexpr int AC_BATCH = 512;
 constexpr int AC_STAGE = 4096;
+template <bool LANE_ZW>
 __global__ void __launch_bounds__(32) ac_encode_lanes_kernel(const uint32_t *__restrict__ c_lo, const uint32_t *__restrict__ c_hi,
                                                              const uint64_t *__restrict__ lane_off, size_t n_lanes,
                                                              uint8_t *__restrict__ out, const uint64_t *__restrict__ out_off,
                                                              uint64_t *__restrict__ out_len, int *__restrict__ err,
-                                                             unsigned long long *__restrict__ err_index) {
+                                                             unsigned long long *__restrict__ err_index,
+                                                             unsigned long long *__restrict__ lane_zw) {
   __shared__ uint32_t s_lo[AC_BATCH], s_hi[AC_BATCH];
   __shared__ __align__(16) uint8_t s_stage[AC_STAGE];
   const size_t lane = blockIdx.x;
@@ -44,6 +48,7 @@ __global__ void __launch_bounds__(32) ac_encode_lanes_kernel(const uint32_t *__r
         if (hi <= lo || hi > CZ_AC_CDF_TOTAL) {
           atomicOr(err, 4);
           atomicMin(err_index, (unsigned long long)(base + i));
+          if constexpr (LANE_ZW) lane_zw[lane] = (unsigned long long)(base + i - t0);
           bad = 1;
           break;
         }
@@ -67,6 +72,7 @@ __global__ void __launch_bounds__(32) ac_encode_lanes_kernel(const uint32_t *__r
     const uint64_t total = enc.finish();
     enc.flush_stage_serial();
     out_len[lane] = total;
+    if constexpr (LANE_ZW) lane_zw[lane] = ~0ull;
   }
 }
 
@@ -98,12 +104,18 @@ namespace cz {
 
 int launch_ac_encode_lanes(cz_ctx *ctx, const uint32_t *c_lo_dev, const uint32_t *c_hi_dev, const uint64_t *lane_off_dev,
                            size_t n_lanes, uint8_t *out_dev, const uint64_t *out_off_dev, uint64_t *out_len_dev,
-                           unsigned long long *err_index_dev, cudaStream_t stream) {
+                           unsigned long long *err_index_dev, cudaStream_t stream, unsigned long long *lane_zw_dev) {
   if (n_lanes == 0) return CZ_OK;
-  CZ_LAUNCH(ctx, CZ_K_CODER,
-            (czk::ac_encode_lanes_kernel<<<(unsigned)n_lanes, 32, 0, stream>>>(
-                c_lo_dev, c_hi_dev, lane_off_dev, n_lanes, out_dev, out_off_dev, out_len_dev, ctx->err_flag_dev,
-                err_index_dev)));
+  if (lane_zw_dev)
+    CZ_LAUNCH(ctx, CZ_K_CODER,
+              (czk::ac_encode_lanes_kernel<true><<<(unsigned)n_lanes, 32, 0, stream>>>(
+                  c_lo_dev, c_hi_dev, lane_off_dev, n_lanes, out_dev, out_off_dev, out_len_dev, ctx->err_flag_dev,
+                  err_index_dev, lane_zw_dev)));
+  else
+    CZ_LAUNCH(ctx, CZ_K_CODER,
+              (czk::ac_encode_lanes_kernel<false><<<(unsigned)n_lanes, 32, 0, stream>>>(
+                  c_lo_dev, c_hi_dev, lane_off_dev, n_lanes, out_dev, out_off_dev, out_len_dev, ctx->err_flag_dev,
+                  err_index_dev, nullptr)));
   CZ_CHECK_LAUNCH();
   return CZ_OK;
 }

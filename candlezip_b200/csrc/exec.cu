@@ -20,9 +20,10 @@ int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size
                     double *xe_dev, cudaStream_t stream, const int *colmax_dev = nullptr);
 int launch_ac_encode_lanes(cz_ctx *ctx, const uint32_t *c_lo_dev, const uint32_t *c_hi_dev, const uint64_t *lane_off_dev,
                            size_t n_lanes, uint8_t *out_dev, const uint64_t *out_off_dev, uint64_t *out_len_dev,
-                           unsigned long long *err_index_dev, cudaStream_t stream);
+                           unsigned long long *err_index_dev, cudaStream_t stream, unsigned long long *lane_zw_dev = nullptr);
 int require_device(cz_ctx *ctx);
 int fetch_device_status(cz_ctx *ctx, unsigned long long *err_index_dev, unsigned long long *err_index_out);
+int fetch_device_status_masked(cz_ctx *ctx, unsigned long long *err_index_dev, unsigned long long *err_index_out, int ignore_bits);
 // exec_rwkv.cu
 int rwkv_encode_bounds(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids_host, size_t n_tokens, const cz_schedule *sched,
                        const uint32_t *extra_dev, const std::vector<size_t> &ev_off, uint32_t *lo_dev, uint32_t *hi_dev, cudaStream_t st);
@@ -456,6 +457,10 @@ static int encode_core(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
   const double t_begin = host_ms();
   double t_build = 0, t_flush = 0;
   const uint32_t S = sched->n_segments;
+  if (m->zw_host && m->zw_cap < S) {
+    set_error("zero-width sink too small: " + std::to_string(m->zw_cap) + " < " + std::to_string(S) + " segments");
+    return CZ_ERR_INVALID;
+  }
   static const size_t env_rows = getenv("CZ_WAVE_ROWS") ? (size_t)atoll(getenv("CZ_WAVE_ROWS")) : 0;  // tuning aid
   const size_t max_rows = sched->max_batch_tokens ? sched->max_batch_tokens : (env_rows ? env_rows : (size_t)262144);
   GrowBuf &d_lo = m->sb[SB_LO], &d_hi = m->sb[SB_HI], &d_src = m->sb[SB_SRC], &d_extra = m->sb[SB_EXTRA], &d_lane = m->sb[SB_LANE],
@@ -537,20 +542,22 @@ static int encode_core(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
   // ---- arithmetic-coder lanes: one per segment ----
   std::vector<uint64_t> lane_off(sched->seg_start, sched->seg_start + S + 1), raw_off(S + 1);
   for (uint32_t g = 0; g <= S; g++) raw_off[g] = 4 * lane_off[g] + 8 * (uint64_t)g;
-  CZ_TRY(d_lane.reserve((S + 1) * 8 * 4 + 64, st));
+  CZ_TRY(d_lane.reserve((S + 1) * 8 * 5 + 64, st));
   uint64_t *d_lane_off = d_lane.as<uint64_t>(), *d_raw_off = d_lane_off + (S + 1), *d_len = d_raw_off + (S + 1),
            *d_dst_off = d_len + (S + 1);
-  unsigned long long *d_eidx = (unsigned long long *)(d_dst_off + (S + 1));
+  unsigned long long *d_eidx = (unsigned long long *)(d_dst_off + (S + 1)), *d_zw = m->zw_host ? d_eidx + 1 : nullptr;
   const unsigned long long none = ~0ull;
   CZ_CUDA_TRY(cudaMemcpyAsync(d_lane_off, lane_off.data(), (S + 1) * 8, cudaMemcpyHostToDevice, st));
   CZ_CUDA_TRY(cudaMemcpyAsync(d_raw_off, raw_off.data(), (S + 1) * 8, cudaMemcpyHostToDevice, st));
   CZ_CUDA_TRY(cudaMemcpyAsync(d_eidx, &none, 8, cudaMemcpyHostToDevice, st));
   CZ_TRY(d_raw.reserve(raw_off[S] + 16, st));
   CZ_TRY(launch_ac_encode_lanes(ctx, d_lo.as<uint32_t>(), d_hi.as<uint32_t>(), d_lane_off, S, d_raw.as<uint8_t>(), d_raw_off, d_len,
-                                d_eidx, st));
+                                d_eidx, st, d_zw));
   std::vector<uint64_t> len(S);
   CZ_CUDA_TRY(cudaMemcpyAsync(len.data(), d_len, S * 8, cudaMemcpyDeviceToHost, st));
-  CZ_TRY(fetch_device_status(ctx, d_eidx, nullptr));
+  // with a zero-width sink each lane reports its own first zero-width index there (its payload is left empty) instead of the call failing
+  if (d_zw) CZ_CUDA_TRY(cudaMemcpyAsync(m->zw_host, d_zw, S * 8, cudaMemcpyDeviceToHost, st));
+  CZ_TRY(fetch_device_status_masked(ctx, d_eidx, nullptr, d_zw ? 4 : 0));
   seg_off_host[0] = 0;
   for (uint32_t g = 0; g < S; g++) seg_off_host[g + 1] = seg_off_host[g] + len[g];
   if (seg_off_host[S] > out_cap) {

@@ -127,6 +127,9 @@ struct cz_model {
   size_t digest_cap = 0;
   // cz_model_set_pdf_floor: SmolLM streams are coded with CZ_CDF_SMOLLM_FLOOR (exec.cu, coded_mode)
   bool pdf_floor = false;
+  // cz_model_set_zero_width_out: per-segment first zero-width index of cz_encode / cz_encode_dev (exec.cu, encode_core)
+  uint64_t *zw_host = nullptr;
+  size_t zw_cap = 0;
 };
 
 namespace cz {

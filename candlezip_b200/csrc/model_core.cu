@@ -534,6 +534,12 @@ int cz_model_set_pdf_floor(cz_model *m, int enabled) {
   m->pdf_floor = enabled != 0;
   return CZ_OK;
 }
+int cz_model_set_zero_width_out(cz_model *m, uint64_t *first_zw_out, size_t cap_segments) {
+  if (!m || (first_zw_out && cap_segments == 0)) return CZ_ERR_INVALID;
+  m->zw_host = first_zw_out;
+  m->zw_cap = first_zw_out ? cap_segments : 0;
+  return CZ_OK;
+}
 int cz_model_tensor_count(const cz_model *m) { return m ? (int)m->tensors.size() : 0; }
 int cz_model_tensor_info(const cz_model *m, int idx, const char **name, size_t *n_elems) {
   if (!m || idx < 0 || idx >= (int)m->tensors.size()) return CZ_ERR_INVALID;

@@ -223,6 +223,17 @@ int cz_model_set_digest_out(cz_model *m, uint8_t *digests_out, size_t cap_tokens
  * RWKV-7: enabled != 0 returns CZ_ERR_UNSUPPORTED (its alphabet is floored already). */
 int cz_model_set_pdf_floor(cz_model *m, int enabled);
 
+/* Per-segment zero-width report.  With a sink set, cz_encode / cz_encode_dev do not fail on a zero-width interval (SmolLM's unfloored
+ * pdf, CZ_ERR_ZERO_WIDTH): they return CZ_OK and write first_zw_out[g] for every segment g of the call, the SEGMENT-RELATIVE coded
+ * index of segment g's first zero-width token (the arithmetic-coder lane stops there), or UINT64_MAX when the segment has none.
+ * The payload of a segment with an entry other than UINT64_MAX is UNSPECIFIED (the caller stores or re-codes that data); every other
+ * segment's payload is the one it gets when coded alone, byte for byte.  This lets a batch of many files coded in one call single out
+ * the files that need a fallback.  Out-of-range symbols (CZ_ERR_SYMBOL_RANGE) and NaN logits still fail the call.
+ * RWKV-7 (floored alphabet) never has a zero-width token: it writes UINT64_MAX for every segment.  cap_segments < the call's
+ * n_segments makes the call return CZ_ERR_INVALID.  NULL (the default when the model is created) restores failing with
+ * CZ_ERR_ZERO_WIDTH; first_zw_out != NULL with cap_segments == 0 is CZ_ERR_INVALID. */
+int cz_model_set_zero_width_out(cz_model *m, uint64_t *first_zw_out, size_t cap_segments);
+
 typedef struct {
   const uint32_t *prime;     /* tail(history, 511-|hint|) ++ hint, built by the caller or cz_xe_make_prime */
   uint32_t prime_len;
