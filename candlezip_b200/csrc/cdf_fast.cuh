@@ -1,7 +1,7 @@
-// Round-2 CDF arithmetic: the same values as cdf_device.cuh, bit for bit, in far fewer issue slots.
+// Round-2 CDF arithmetic: the same values as cdf_device.cuh's cz_expf and IEEE divisions, bit for bit, in far fewer issue slots.
 //
-// What bounded the round-1 kernel (profiles/ncu_summary_r01g.md: 33 instructions per logit, 58% issue, 0.32 of HBM) was not the
-// ten FP64 operations of the glibc expf but what surrounds them:
+// What bounded the round-1 thread-per-column kernel (profiles/ncu_summary_r01g.md: 33 instructions per logit, 58% issue, 0.32 of
+// HBM) was not the ten FP64 operations of the glibc expf but what surrounds them:
 //   * three F2F conversions per logit (f32 -> f64 of the argument, f64 -> f32 -> f64 of the result).  Conversions to / from 64-bit
 //     types run at a quarter of the FP64 rate, so they cost more pipe time than the arithmetic.  Here the argument is widened with
 //     one integer multiply-add ((u64)bits * 2^29 + bias: exact for a normal f32) and the result is rounded to the f32 grid
@@ -82,66 +82,43 @@ __device__ __forceinline__ double cz_widen_pos(float e) {
 
 // (cz_div_rcp / cz_div_rcp_ok: cdf_device.cuh -- the decode-side search uses them too)
 
-// ---- vectorised full-column walk: NCOL adjacent columns per thread ------------------------------------------------------------
-template <int NCOL>
-struct CdfVec;
-template <>
-struct CdfVec<1> {
-  using T = float;
-  static __device__ __forceinline__ void unpack(const T &t, float (&x)[1]) { x[0] = t; }
-};
-template <>
-struct CdfVec<2> {
-  using T = float2;
-  static __device__ __forceinline__ void unpack(const T &t, float (&x)[2]) {
-    x[0] = t.x;
-    x[1] = t.y;
-  }
-};
-template <>
-struct CdfVec<4> {
-  using T = float4;
-  static __device__ __forceinline__ void unpack(const T &t, float (&x)[4]) {
-    x[0] = t.x;
-    x[1] = t.y;
-    x[2] = t.z;
-    x[3] = t.w;
-  }
-};
-
-// Calls f(v0, rows, cnt) for consecutive groups of up to GRP rows (cnt valid) of the NCOL columns starting at p, in ascending
-// row order, with the next group's loads in flight and an L2 prefetch CDF_PF rows ahead (cdf_walk's pipelining).  NC: read-only path.
-template <int NCOL, int GRP, bool NC, class F>
+// Calls f(v0, rows, cnt) for consecutive groups of CDF_GRP rows (cnt of them valid) of the column at p, in ascending row order, with
+// the loads software-pipelined: the next group is already in flight (registers) while the current one is consumed, and an L2
+// prefetch runs CDF_PF rows ahead.  Consecutive rows of a column are ld * 4 bytes apart (a new DRAM page every row), so without
+// this the direct-load stats kernel is bound by memory latency x the few loads a warp has in flight, not by bandwidth.
+// NC: loads go through the read-only path (__ldg).  NC = false is for a column that this thread rewrites in place between passes
+// (the RWKV alphabet caches exp(l - max) in the logit's slot): ordinary loads, which see the thread's own earlier stores.
+constexpr int CDF_GRP = 8;
+constexpr int CDF_PF = 48;
+template <bool NC, class F>
 __device__ __forceinline__ void cdf_walk_groups(const float *p, size_t ld, int n, F f) {
-  using T = typename CdfVec<NCOL>::T;
-  auto ldv = [&](size_t row) -> T {
-    const T *q = reinterpret_cast<const T *>(p + row * ld);
+  auto ldv = [&](size_t row) -> float {
+    const float *q = p + row * ld;
     return NC ? __ldg(q) : *q;
   };
-  T cur[GRP], nxt[GRP];
-  const T zero = T();
+  float cur[CDF_GRP], nxt[CDF_GRP];
 #pragma unroll
-  for (int k = 0; k < GRP; k++) cur[k] = k < n ? ldv((size_t)k) : zero;
+  for (int k = 0; k < CDF_GRP; k++) cur[k] = k < n ? ldv((size_t)k) : 0.f;
   int v0 = 0;
-  for (; v0 + CDF_PF + GRP <= n; v0 += GRP) {
+  for (; v0 + CDF_PF + CDF_GRP <= n; v0 += CDF_GRP) {
 #pragma unroll
-    for (int k = 0; k < GRP; k++) {
-      nxt[k] = ldv((size_t)(v0 + GRP + k));
+    for (int k = 0; k < CDF_GRP; k++) {
+      nxt[k] = ldv((size_t)(v0 + CDF_GRP + k));
       asm volatile("prefetch.global.L2 [%0];" ::"l"(p + (size_t)(v0 + CDF_PF + k) * ld));
     }
-    f(v0, cur, GRP);
+    f(v0, cur, CDF_GRP);
 #pragma unroll
-    for (int k = 0; k < GRP; k++) cur[k] = nxt[k];
+    for (int k = 0; k < CDF_GRP; k++) cur[k] = nxt[k];
   }
-  for (; v0 < n; v0 += GRP) {
+  for (; v0 < n; v0 += CDF_GRP) {
 #pragma unroll
-    for (int k = 0; k < GRP; k++) {
-      const int v = v0 + GRP + k;
-      nxt[k] = v < n ? ldv((size_t)v) : zero;
+    for (int k = 0; k < CDF_GRP; k++) {
+      const int v = v0 + CDF_GRP + k;
+      nxt[k] = v < n ? ldv((size_t)v) : 0.f;
     }
-    f(v0, cur, n - v0 < GRP ? n - v0 : GRP);
+    f(v0, cur, n - v0 < CDF_GRP ? n - v0 : CDF_GRP);
 #pragma unroll
-    for (int k = 0; k < GRP; k++) cur[k] = nxt[k];
+    for (int k = 0; k < CDF_GRP; k++) cur[k] = nxt[k];
   }
 }
 
@@ -184,7 +161,7 @@ __device__ __forceinline__ void exp_group(const float (&a)[N], const ExpTab64 &t
 // step a thread-per-column walk is a ~10^5-deep dependent chain per thread with nothing to overlap.  Here the 32 lanes evaluate
 // expf / the pdf for 32 consecutive vocab entries in parallel and only the order-dependent f64 accumulation is serial (every lane
 // performs it redundantly on values exchanged through a shared-memory line, so all lanes hold the same S / acc and branches stay
-// warp-uniform).  Same operations in the same order per column as cdf_col => bit-identical results.
+// warp-uniform).  Same operations in the same order per column as cdf_full_kernel => bit-identical results.
 //
 // What a step costs is the latency of one warp's instruction stream (one or two warps per scheduler), so the loop is built for
 // the in-order issue of a single warp (ncu, profiles/ncu_summary_r02.md: the first version took 1,240 cycles per group of 32 rows
@@ -204,8 +181,8 @@ template <int MODE, int NC>
 __device__ __forceinline__ void cdf_search_warp_n(const float *const (&p)[NC], size_t ld, int V, const uint32_t (&value)[NC],
                                                   const float (&mx)[NC], const ExpTab64 &tab, uint32_t (&sym_out)[NC],
                                                   uint32_t (&lo_out)[NC], uint32_t (&hi_out)[NC], int &errbits, double *xch) {
-  // (No in-place caching of expf here, unlike cdf_col: the stepwise RWKV decoder keeps a stream's logits column across steps while
-  // it decodes literal bytes, so the column must stay intact.)
+  // (No in-place caching of expf here, unlike the RWKV alphabet's stats passes: the stepwise RWKV decoder keeps a stream's logits
+  // column across steps while it decodes literal bytes, so the column must stay intact.)
   const int lane = threadIdx.x & 31;
   const int n_sym = MODE == CZ_CDF_RWKV_LITERALS ? V + 256 : V;
   const int n_full = V / 32, n_grp = (V + 31) / 32;

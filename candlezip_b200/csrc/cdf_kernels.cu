@@ -12,8 +12,9 @@
 // f32::exp lowers to on Linux; every mul/add/fma is an explicit round-to-nearest intrinsic so nvcc cannot
 // re-contract.  Algorithmic bytes = 4*V per column (one read).  Encode (OP_BOUNDS / OP_XE): the max comes from the LM-head
 // GEMM's epilogue, cdf_stats_tma_kernel reads the column once per pass (one pass for SmolLM coding) and leaves the few e_v the
-// prefix walk needs in a compact cache, cdf_bounds_warp_kernel walks that cache; cdf_cols_kernel is the round-1 single kernel,
-// kept for unaligned / tiny batches and bisecting.  Decode (OP_SEARCH): cdf_search_warp_n (cdf_fast.cuh), a warp per stream.
+// prefix walk needs in a compact cache, cdf_bounds_warp_kernel walks that cache; cdf_stats_kernel does the same passes by direct
+// loads for batches the tensor map cannot describe (ld % 4 != 0, an unaligned base) or too small to fill the machine.
+// Decode (OP_SEARCH): cdf_search_warp_n (cdf_fast.cuh), a warp per stream.
 #include <stdlib.h>
 
 #include <algorithm>
@@ -24,198 +25,110 @@
 
 namespace czk {
 
-// One thread per column of the vocab-major logits.
-template <int MODE, int OP>
-__global__ void __launch_bounds__(128) cdf_cols_kernel(const float *__restrict__ logits, int V, size_t M, size_t ld,
-                                                       const uint32_t *__restrict__ syms_or_values,
-                                                       uint32_t *__restrict__ sym_out, uint32_t *__restrict__ c_lo_out,
-                                                       uint32_t *__restrict__ c_hi_out, double *__restrict__ xe_out,
-                                                       int *__restrict__ err, const int *__restrict__ colmax) {
-  __shared__ uint32_t s_lo[32 * 32], s_hi[32 * 32];
-  exp_tab_init(s_lo, s_hi);
-  ExpTab tab{s_lo, s_hi, (int)(threadIdx.x & 31)};
-  size_t col = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const bool active = col < M;
-  if (!active) col = M - 1;  // keep the warp converged; results of inactive lanes are discarded
-  uint32_t sym, lo, hi;
-  double xe;
-  int errbits = 0;
-  cdf_col<MODE, OP>(logits + col, ld, V, syms_or_values[col], active, tab, sym, lo, hi, xe, errbits, colmax != nullptr,
-                    colmax ? colmax_decode(colmax[col]) : 0.f);
-  if (!active) return;
-  if (errbits) atomicOr(err, errbits);
-  if (OP == OP_XE) {
-    xe_out[col] = xe;
-  } else {
-    if (OP == OP_SEARCH) sym_out[col] = sym;
-    c_lo_out[col] = lo;
-    c_hi_out[col] = hi;
-  }
-}
-
-
 // =================================================================================================================
 // Round-2 encode-side kernels (OP_BOUNDS / OP_XE): full passes and the prefix walk are separate kernels.
 // =================================================================================================================
 
-// Full passes.  One thread owns NCOL adjacent columns (vector loads: one LDG + one address per NCOL logits); every column is still
-// summed by one thread in ascending vocab order.  MODE / OP decide which passes run:
+// Full passes by direct loads, one thread per column, every column summed in ascending vocab order.  MODE / OP decide which passes run:
 //   pass 1  S = sum (f64)expf(l - max)                      always            (RWKV alphabet: leaves e_v in the logit's slot)
 //   pass 2  norm = sum max(e / S, 2^-29)                    RWKV alphabet, floored SmolLM alphabet, XE
 //   pass 3  sum2 = sum RN(RN(max(e / S, 2^-29) / norm) (1 - 2^-21)) + 256 x 2^-29   RWKV alphabet
-template <int MODE, int OP, int NCOL>
+template <int MODE, int OP>
 __global__ void __launch_bounds__(128) cdf_stats_kernel(float *__restrict__ logits, int V, size_t M, size_t ld, const int *__restrict__ colmax,
                                                         CdfStats *__restrict__ stats, int *__restrict__ err) {
   constexpr bool kLit = MODE == CZ_CDF_RWKV_LITERALS;
   constexpr bool kNorm = kLit || OP == OP_XE || MODE == CZ_CDF_SMOLLM_FLOOR;
-  constexpr int GRP = NCOL == 4 ? 4 : 8;
-  constexpr int NE = GRP * NCOL;
   __shared__ uint64_t s_tab[32 * 32];
   exp_tab64_init(s_tab);
   const ExpTab64 tab{s_tab + (threadIdx.x & 31)};
-  const size_t col0 = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) * NCOL;
-  if (col0 >= M) return;
-  float *p = logits + col0;
-  float mx[NCOL];
+  const size_t col = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (col >= M) return;
+  float *p = logits + col;
+  float mx;
   if (colmax) {
-#pragma unroll
-    for (int c = 0; c < NCOL; c++) mx[c] = col0 + c < M ? colmax_decode(colmax[col0 + c]) : 0.f;
+    mx = colmax_decode(colmax[col]);
   } else {
+    mx = __int_as_float(0xff800000);
+    cdf_walk_groups<true>(p, ld, V, [&](int, const float(&x)[CDF_GRP], int cnt) {
 #pragma unroll
-    for (int c = 0; c < NCOL; c++) mx[c] = __int_as_float(0xff800000);
-    cdf_walk_groups<NCOL, GRP, true>(p, ld, V, [&](int, const typename CdfVec<NCOL>::T(&rows)[GRP], int cnt) {
-#pragma unroll
-      for (int k = 0; k < GRP; k++) {
-        if (k < cnt) {
-          float x[NCOL];
-          CdfVec<NCOL>::unpack(rows[k], x);
-#pragma unroll
-          for (int c = 0; c < NCOL; c++)
-            if (x[c] > mx[c]) mx[c] = x[c];  // NaN-ignoring, like `if v > max` (src/main.rs:786-788)
-        }
-      }
+      for (int k = 0; k < CDF_GRP; k++)
+        if (k < cnt && x[k] > mx) mx = x[k];  // NaN-ignoring, like `if v > max` (src/main.rs:786-788)
     });
   }
   // ---- pass 1 ----
-  double S[NCOL];
+  double S = 0.0;
+  cdf_walk_groups<!kLit>(p, ld, V, [&](int v0, const float(&x)[CDF_GRP], int cnt) {
+    float a[CDF_GRP], ef[CDF_GRP];
+    double d[CDF_GRP];
 #pragma unroll
-  for (int c = 0; c < NCOL; c++) S[c] = 0.0;
-  cdf_walk_groups<NCOL, GRP, !kLit>(p, ld, V, [&](int v0, const typename CdfVec<NCOL>::T(&rows)[GRP], int cnt) {
-    float a[NE], ef[NE];
-    double d[NE];
+    for (int k = 0; k < CDF_GRP; k++) a[k] = __fsub_rn(mx, x[k]);  // = -(l - max), exactly
+    exp_group<CDF_GRP, kLit>(a, tab, d, ef);
 #pragma unroll
-    for (int k = 0; k < GRP; k++) {
-      float x[NCOL];
-      CdfVec<NCOL>::unpack(rows[k], x);
-#pragma unroll
-      for (int c = 0; c < NCOL; c++) a[k * NCOL + c] = __fsub_rn(mx[c], x[c]);  // = -(l - max), exactly
-    }
-    exp_group<NE, kLit>(a, tab, d, ef);
-#pragma unroll
-    for (int k = 0; k < GRP; k++) {
+    for (int k = 0; k < CDF_GRP; k++) {
       if (k < cnt) {
-#pragma unroll
-        for (int c = 0; c < NCOL; c++) S[c] = __dadd_rn(S[c], d[k * NCOL + c]);
-        if (kLit) {  // cache e_v for the later passes (columns beyond M are row padding: scratch)
-          typename CdfVec<NCOL>::T o;
-          float *of = reinterpret_cast<float *>(&o);
-#pragma unroll
-          for (int c = 0; c < NCOL; c++) of[c] = ef[k * NCOL + c];
-          *reinterpret_cast<typename CdfVec<NCOL>::T *>(p + (size_t)(v0 + k) * ld) = o;
-        }
+        S = __dadd_rn(S, d[k]);
+        if (kLit) p[(size_t)(v0 + k) * ld] = ef[k];  // cache e_v for the later passes
       }
     }
   });
   int errbits = 0;
-#pragma unroll
-  for (int c = 0; c < NCOL; c++)
-    if (col0 + c < M && !(S[c] == S[c])) errbits |= CZ_DEVERR_NAN;
-  double norm[NCOL], sum2[NCOL];
-#pragma unroll
-  for (int c = 0; c < NCOL; c++) norm[c] = sum2[c] = 1.0;
+  if (!(S == S)) errbits |= CZ_DEVERR_NAN;
+  double norm = 1.0, sum2 = 1.0;
   if (kNorm) {
+    // (spelled as a running AND on purpose: `const bool fast = cz_div_rcp_ok(S)` makes nvcc 12.9 build different code for the passes
+    // below, e.g. 72 registers and 16 B of spill stores instead of 90 and none for XE and the floored alphabet)
     bool fast = true;
-    double yS[NCOL];
-#pragma unroll
-    for (int c = 0; c < NCOL; c++) {
-      fast = fast && cz_div_rcp_ok(S[c]);
-      yS[c] = __drcp_rn(S[c]);
-    }
+    fast = fast && cz_div_rcp_ok(S);
+    const double yS = __drcp_rn(S);
     // e_v (as a double) of the rows of a group: the cached f32 (RWKV alphabet) or recomputed from the logit (SmolLM: floored / XE)
-    auto e_of = [&](const typename CdfVec<NCOL>::T(&rows)[GRP], double(&d)[NE]) {
-      float a[NE], ef[NE];
+    auto e_of = [&](const float(&x)[CDF_GRP], double(&d)[CDF_GRP]) {
+      float a[CDF_GRP], ef[CDF_GRP];
 #pragma unroll
-      for (int k = 0; k < GRP; k++) {
-        float x[NCOL];
-        CdfVec<NCOL>::unpack(rows[k], x);
-#pragma unroll
-        for (int c = 0; c < NCOL; c++) {
-          if (kLit) d[k * NCOL + c] = fast ? cz_widen_pos(x[c]) : (double)x[c];  // (values below 2^-126 are floored either way)
-          else a[k * NCOL + c] = __fsub_rn(mx[c], x[c]);
-        }
+      for (int k = 0; k < CDF_GRP; k++) {
+        if (kLit) d[k] = fast ? cz_widen_pos(x[k]) : (double)x[k];  // (values below 2^-126 are floored either way)
+        else a[k] = __fsub_rn(mx, x[k]);
       }
-      if (!kLit) exp_group<NE, false>(a, tab, d, ef);
+      if (!kLit) exp_group<CDF_GRP, false>(a, tab, d, ef);
     };
-    auto div_S = [&](double e, int c) { return fast ? cz_div_rcp(e, S[c], yS[c]) : __ddiv_rn(e, S[c]); };
+    auto div_S = [&](double e) { return fast ? cz_div_rcp(e, S, yS) : __ddiv_rn(e, S); };
     // ---- pass 2 ----
-    double acc[NCOL];
+    double acc = 0.0;
+    cdf_walk_groups<!kLit>(p, ld, V, [&](int, const float(&x)[CDF_GRP], int cnt) {
+      double d[CDF_GRP];
+      e_of(x, d);
 #pragma unroll
-    for (int c = 0; c < NCOL; c++) acc[c] = 0.0;
-    cdf_walk_groups<NCOL, GRP, !kLit>(p, ld, V, [&](int, const typename CdfVec<NCOL>::T(&rows)[GRP], int cnt) {
-      double d[NE];
-      e_of(rows, d);
-#pragma unroll
-      for (int k = 0; k < GRP; k++)
-        if (k < cnt) {
-#pragma unroll
-          for (int c = 0; c < NCOL; c++) acc[c] = __dadd_rn(acc[c], fmax(div_S(d[k * NCOL + c], c), CZ_P_FLOOR));
-        }
+      for (int k = 0; k < CDF_GRP; k++)
+        if (k < cnt) acc = __dadd_rn(acc, fmax(div_S(d[k]), CZ_P_FLOOR));
     });
-#pragma unroll
-    for (int c = 0; c < NCOL; c++) norm[c] = acc[c];
+    norm = acc;
     if (kLit) {
       // ---- pass 3 ----
       const double scale = 1.0 - 256.0 * CZ_P_FLOOR;
-      double yN[NCOL];
-      bool fastn = fast;
+      const bool fastn = fast && cz_div_rcp_ok(norm);
+      const double yN = __drcp_rn(norm);
+      acc = 0.0;
+      cdf_walk_groups<false>(p, ld, V, [&](int, const float(&x)[CDF_GRP], int cnt) {
+        double d[CDF_GRP];
+        e_of(x, d);
 #pragma unroll
-      for (int c = 0; c < NCOL; c++) {
-        fastn = fastn && cz_div_rcp_ok(norm[c]);
-        yN[c] = __drcp_rn(norm[c]);
-        acc[c] = 0.0;
-      }
-      cdf_walk_groups<NCOL, GRP, false>(p, ld, V, [&](int, const typename CdfVec<NCOL>::T(&rows)[GRP], int cnt) {
-        double d[NE];
-        e_of(rows, d);
-#pragma unroll
-        for (int k = 0; k < GRP; k++)
+        for (int k = 0; k < CDF_GRP; k++)
           if (k < cnt) {
-#pragma unroll
-            for (int c = 0; c < NCOL; c++) {
-              const double q = fmax(div_S(d[k * NCOL + c], c), CZ_P_FLOOR);
-              const double q2 = fastn ? cz_div_rcp(q, norm[c], yN[c]) : __ddiv_rn(q, norm[c]);
-              acc[c] = __dadd_rn(acc[c], __dmul_rn(q2, scale));
-            }
+            const double q = fmax(div_S(d[k]), CZ_P_FLOOR);
+            const double q2 = fastn ? cz_div_rcp(q, norm, yN) : __ddiv_rn(q, norm);
+            acc = __dadd_rn(acc, __dmul_rn(q2, scale));
           }
       });
-#pragma unroll
-      for (int c = 0; c < NCOL; c++) {
-        for (int j = 0; j < 256; j++) acc[c] = __dadd_rn(acc[c], CZ_P_FLOOR);
-        sum2[c] = acc[c];
-      }
+      for (int j = 0; j < 256; j++) acc = __dadd_rn(acc, CZ_P_FLOOR);
+      sum2 = acc;
     }
   }
-#pragma unroll
-  for (int c = 0; c < NCOL; c++)
-    if (col0 + c < M) {
-      CdfStats st;
-      st.S = S[c];
-      st.norm = norm[c];
-      st.sum2 = sum2[c];
-      st.mx = mx[c];
-      st.pad = 0;
-      stats[col0 + c] = st;
-    }
+  CdfStats st;
+  st.S = S;
+  st.norm = norm;
+  st.sum2 = sum2;
+  st.mx = mx;
+  st.pad = 0;
+  stats[col] = st;
   if (errbits) atomicOr(err, errbits);
 }
 
@@ -507,7 +420,7 @@ __global__ void __launch_bounds__(ST_COLS + 32, 2) cdf_stats_tma_kernel(const __
   }
 }
 
-// pdf entry of vocab element v from its logit (SmolLM) / cached e_v (RWKV alphabet): the same expressions as cdf_col's pdf_vocab
+// pdf entry of vocab element v from its logit (SmolLM) / cached e_v (RWKV alphabet): the same expressions as cdf_full_kernel's
 template <int MODE, bool FLOORED>
 struct PdfOf {
   double S, norm, sum2, yS, yN, y2, uni;
@@ -564,7 +477,7 @@ struct PdfOf {
 // shared-memory line the values were exchanged through (cdf_search_warp's scheme), so all lanes hold the same acc and every branch
 // is warp-uniform.  Columns are independent warps of very different lengths, thousands per SM over the kernel's life: the machine
 // stays full until the end, and the longest column costs V / 32 short iterations.
-// Same operations in the same order as cdf_col's OP_BOUNDS: bit-identical results.
+// Same operations in the same order as cdf_full_kernel's prefix sum: bit-identical results.
 // Columns are handed out one at a time from a global counter (persistent warps): a warp that finishes a short column takes the
 // next one instead of idling until the longest column of its CTA is done.  (Reading the vocab-major logits this way was meant to
 // share a row's 32-byte sector between the warps of adjacent columns through L1 / L2; ncu showed it does not -- the walks drift
@@ -792,8 +705,9 @@ __global__ void __launch_bounds__(256) div_random_kernel(unsigned long long seed
   if (bad) atomicAdd(out, bad);
 }
 
-// OP_SEARCH for a small number of columns (what the stepwise decoder does per step): cdf_search_warp_n with NC columns per warp
-// (2 here, so that the multi-column form stays covered by the kernel-level parity tests; the decoder itself uses 1, exec.cu)
+// OP_SEARCH for any number of columns (the stepwise decoder runs the same search inside decode_step_kernel, exec.cu):
+// cdf_search_warp_n with NC columns per warp (2 here, so that the multi-column form stays covered by the kernel-level parity tests;
+// the decoder itself uses 1)
 template <int MODE>
 __global__ void __launch_bounds__(128) cdf_search_warp_kernel(const float *__restrict__ logits, int V, size_t M, size_t ld,
                                                               const uint32_t *__restrict__ values, uint32_t *__restrict__ sym_out,
@@ -848,10 +762,10 @@ __global__ void __launch_bounds__(128) cdf_search_warp_kernel(const float *__res
 // full CDF of one column (debug / watchdog parity): single thread, sequential
 template <int MODE>
 __global__ void cdf_full_kernel(const float *__restrict__ logits, int V, uint32_t *__restrict__ cdf) {
-  __shared__ uint32_t s_lo[32 * 32], s_hi[32 * 32];
-  exp_tab_init(s_lo, s_hi);
+  __shared__ uint64_t s_tab[32 * 32];
+  exp_tab64_init(s_tab);
   if (threadIdx.x != 0) return;
-  ExpTab tab{s_lo, s_hi, 0};
+  const ExpTab64 tab{s_tab};
   const int n_sym = MODE == CZ_CDF_RWKV_LITERALS ? V + 256 : V;
   float mx = __int_as_float(0xff800000);
   for (int v = 0; v < V; v++)
@@ -948,245 +862,166 @@ static int make_logits_map(CUtensorMap *map, const float *logits, size_t V, size
   return CZ_OK;
 }
 
-// Device-pointer launchers (used by the executor and by the host-buffer C-ABI wrappers in api.cu)
-int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size_t V, size_t M, size_t ld,
-                    const uint32_t *arg_dev, uint32_t *sym_out_dev, uint32_t *c_lo_dev, uint32_t *c_hi_dev,
-                    double *xe_dev, cudaStream_t stream, const int *colmax_dev) {
-  if (mode != CZ_CDF_SMOLLM && mode != CZ_CDF_RWKV_LITERALS && mode != CZ_CDF_SMOLLM_FLOOR) {
-    set_error("cdf: unknown mode");
-    return CZ_ERR_INVALID;
+// Calls f(std::integral_constant<int, MODE>{}) for the coding alphabet `mode`, so that each launch is written once for all of them;
+// any other value is CZ_ERR_INVALID.
+template <class F>
+static int with_cdf_mode(int mode, F &&f) {
+  switch (mode) {
+    case CZ_CDF_SMOLLM:
+      return f(std::integral_constant<int, CZ_CDF_SMOLLM>{});
+    case CZ_CDF_RWKV_LITERALS:
+      return f(std::integral_constant<int, CZ_CDF_RWKV_LITERALS>{});
+    case CZ_CDF_SMOLLM_FLOOR:
+      return f(std::integral_constant<int, CZ_CDF_SMOLLM_FLOOR>{});
   }
-  if (M == 0) return CZ_OK;
-  if (V == 0 || V > (1u << 24) || ld < M) {
-    set_error("cdf: bad shape");
-    return CZ_ERR_INVALID;
-  }
-  // OP_XE evaluates the floored pdf for SmolLM whatever the coding alphabet (src/main.rs:1745): mode 2 IS mode 0 there
-  if (op == czk::OP_XE && mode == CZ_CDF_SMOLLM_FLOOR) mode = CZ_CDF_SMOLLM;
-  if (op == czk::OP_SEARCH && M <= 8192) {  // decode-sized: warp per column
-    const unsigned g = (unsigned)ceil_div(M, 8);  // 4 warps x 2 columns
-    if (mode == CZ_CDF_SMOLLM)
-      CZ_LAUNCH(ctx, CZ_K_CDF,
-                (czk::cdf_search_warp_kernel<CZ_CDF_SMOLLM><<<g, 128, 0, stream>>>(logits_dev, (int)V, M, ld, arg_dev, sym_out_dev, c_lo_dev,
-                                                                                   c_hi_dev, ctx->err_flag_dev, colmax_dev)));
-    else if (mode == CZ_CDF_RWKV_LITERALS)
-      CZ_LAUNCH(ctx, CZ_K_CDF,
-                (czk::cdf_search_warp_kernel<CZ_CDF_RWKV_LITERALS><<<g, 128, 0, stream>>>(logits_dev, (int)V, M, ld, arg_dev, sym_out_dev,
-                                                                                          c_lo_dev, c_hi_dev, ctx->err_flag_dev, colmax_dev)));
-    else
-      CZ_LAUNCH(ctx, CZ_K_CDF,
-                (czk::cdf_search_warp_kernel<CZ_CDF_SMOLLM_FLOOR><<<g, 128, 0, stream>>>(logits_dev, (int)V, M, ld, arg_dev, sym_out_dev,
-                                                                                         c_lo_dev, c_hi_dev, ctx->err_flag_dev, colmax_dev)));
-    CZ_CHECK_LAUNCH();
-    return CZ_OK;
-  }
-  static const bool legacy = getenv("CZ_CDF_LEGACY") != nullptr;  // bisecting aid: the round-1 single-kernel path
-  if (!legacy && (op == czk::OP_BOUNDS || op == czk::OP_XE)) {
-    // round-2 path: full passes (vectorised over adjacent columns) -> per-column stats -> sorted prefix walk / XE lookup
-    const size_t need = M * sizeof(czk::CdfStats);
-    if (need > ctx->cdf_stats_bytes) {
-      if (ctx->cdf_stats) {
-        CZ_CUDA_TRY(cudaStreamSynchronize(stream));
-        cudaFree(ctx->cdf_stats);
-        ctx->cdf_stats = nullptr;
-        ctx->cdf_stats_bytes = 0;
-      }
-      const size_t want = need + (need >> 2) + 4096;
-      CZ_CUDA_TRY(cudaMalloc(&ctx->cdf_stats, want));
-      ctx->cdf_stats_bytes = want;
+  set_error("cdf: unknown mode");
+  return CZ_ERR_INVALID;
+}
+
+// Encode side (OP_BOUNDS / OP_XE): full passes -> per-column stats -> prefix walk / XE lookup
+template <int MODE, int OP>
+static int launch_cdf_encode(cz_ctx *ctx, const float *logits_dev, size_t V, size_t M, size_t ld, const uint32_t *syms_dev,
+                             uint32_t *c_lo_dev, uint32_t *c_hi_dev, double *xe_dev, cudaStream_t stream, const int *colmax_dev) {
+  const size_t need = M * sizeof(czk::CdfStats);
+  if (need > ctx->cdf_stats_bytes) {
+    if (ctx->cdf_stats) {
+      CZ_CUDA_TRY(cudaStreamSynchronize(stream));
+      cudaFree(ctx->cdf_stats);
+      ctx->cdf_stats = nullptr;
+      ctx->cdf_stats_bytes = 0;
     }
-    czk::CdfStats *stats = (czk::CdfStats *)ctx->cdf_stats;
-    float *lg = const_cast<float *>(logits_dev);  // (the RWKV alphabet caches expf in place: the logits batch is scratch)
-    // adjacent columns per thread: vector loads need the alignment, and enough columns to fill the machine with fewer threads
-    const char *env_ncol = getenv("CZ_CDF_NCOL");  // (read per call: the tests switch it between calls)
-    const int force_ncol = env_ncol ? atoi(env_ncol) : 0;
-    // (measured on B200, scripts/cdf_bench.py: 1 column per thread is the fastest at every batch size -- 131,072 columns: 13.9 ms
-    // against 14.0 / 16.5 ms for 2 / 4; the RWKV alphabet 28 / 37 / 65 ms: the wider variants leave too few warps per scheduler)
-    int ncol = 1;
-    if (force_ncol == 1 || force_ncol == 2 || force_ncol == 4) ncol = force_ncol;
-    while (ncol > 1 && (ld % ncol != 0 || ((uintptr_t)logits_dev & (size_t)(4 * ncol - 1)) != 0)) ncol >>= 1;
-    // TMA-staged variant: needs tensor-map-compatible strides / alignment and enough columns to fill the machine with 256-column CTAs
-    static const bool no_tma = getenv("CZ_CDF_NO_TMA") != nullptr;  // bisecting aid
-    const bool tma_ok = !no_tma && force_ncol == 0 && ld % 4 == 0 && ((uintptr_t)logits_dev & 15) == 0 && M >= 256 && V >= 64;
-    // e-cache for the prefix walk (see ecache_offsets_kernel): only with the TMA-staged stats kernel, which fills it
-    uint32_t *eoff = nullptr;
-    double *ecache = nullptr;
-    int *eflag = nullptr;
-    if (op == czk::OP_BOUNDS) ctx->cdf_eflag_last = nullptr;
-    if (tma_ok && op == czk::OP_BOUNDS && !ctx->cdf_ecache_failed && getenv("CZ_CDF_NO_ECACHE") == nullptr) {
-      const char *env_frac = getenv("CZ_CDF_ECACHE_FRAC");  // (read per call: the tests switch it between calls)
-      double frac = env_frac ? atof(env_frac) : 0.25;       // capacity as a fraction of the batch's rows (real text needs 0.1)
-      frac = frac < 0.0 ? 0.0 : frac > 1.0 ? 1.0 : frac;
-      const size_t grp_per_col = ceil_div(V, (size_t)czk::EC_GRP);
-      size_t cap_groups = std::min<size_t>((size_t)((double)M * (double)grp_per_col * frac) + 1, 0xffffffffull);
-      const size_t need_e = cap_groups * czk::EC_GRP * sizeof(double), need_o = (M + 2) * sizeof(uint32_t);
-      bool ok = true;
-      if (need_o > ctx->cdf_eoff_bytes || need_e > ctx->cdf_ecache_bytes) {
-        if (ctx->capturing) {
-          ok = false;  // no allocation inside a graph capture
-        } else {
-          CZ_CUDA_TRY(cudaStreamSynchronize(stream));
-          if (need_o > ctx->cdf_eoff_bytes) {
-            if (ctx->cdf_eoff) cudaFree(ctx->cdf_eoff);
-            ctx->cdf_eoff = nullptr;
-            ctx->cdf_eoff_bytes = 0;
-            const size_t want = need_o + (need_o >> 2) + 4096;
-            CZ_CUDA_TRY(cudaMalloc(&ctx->cdf_eoff, want));
-            ctx->cdf_eoff_bytes = want;
-          }
-          if (need_e > ctx->cdf_ecache_bytes) {
-            if (ctx->cdf_ecache) cudaFree(ctx->cdf_ecache);
+    const size_t want = need + (need >> 2) + 4096;
+    CZ_CUDA_TRY(cudaMalloc(&ctx->cdf_stats, want));
+    ctx->cdf_stats_bytes = want;
+  }
+  czk::CdfStats *stats = (czk::CdfStats *)ctx->cdf_stats;
+  float *lg = const_cast<float *>(logits_dev);  // (the RWKV alphabet caches expf in place: the logits batch is scratch)
+  // TMA-staged variant: needs tensor-map-compatible strides / alignment and enough columns to fill the machine with 256-column CTAs
+  const bool tma_ok = ld % 4 == 0 && ((uintptr_t)logits_dev & 15) == 0 && M >= 256 && V >= 64;
+  // e-cache for the prefix walk (see ecache_offsets_kernel): only with the TMA-staged stats kernel, which fills it
+  uint32_t *eoff = nullptr;
+  double *ecache = nullptr;
+  int *eflag = nullptr;
+  if (OP == czk::OP_BOUNDS) ctx->cdf_eflag_last = nullptr;
+  if (tma_ok && OP == czk::OP_BOUNDS && !ctx->cdf_ecache_failed && getenv("CZ_CDF_NO_ECACHE") == nullptr) {
+    const char *env_frac = getenv("CZ_CDF_ECACHE_FRAC");  // (read per call: the tests switch it between calls)
+    double frac = env_frac ? atof(env_frac) : 0.25;       // capacity as a fraction of the batch's rows (real text needs 0.1)
+    frac = frac < 0.0 ? 0.0 : frac > 1.0 ? 1.0 : frac;
+    const size_t grp_per_col = ceil_div(V, (size_t)czk::EC_GRP);
+    size_t cap_groups = std::min<size_t>((size_t)((double)M * (double)grp_per_col * frac) + 1, 0xffffffffull);
+    const size_t need_e = cap_groups * czk::EC_GRP * sizeof(double), need_o = (M + 2) * sizeof(uint32_t);
+    bool ok = true;
+    if (need_o > ctx->cdf_eoff_bytes || need_e > ctx->cdf_ecache_bytes) {
+      if (ctx->capturing) {
+        ok = false;  // no allocation inside a graph capture
+      } else {
+        CZ_CUDA_TRY(cudaStreamSynchronize(stream));
+        if (need_o > ctx->cdf_eoff_bytes) {
+          if (ctx->cdf_eoff) cudaFree(ctx->cdf_eoff);
+          ctx->cdf_eoff = nullptr;
+          ctx->cdf_eoff_bytes = 0;
+          const size_t want = need_o + (need_o >> 2) + 4096;
+          CZ_CUDA_TRY(cudaMalloc(&ctx->cdf_eoff, want));
+          ctx->cdf_eoff_bytes = want;
+        }
+        if (need_e > ctx->cdf_ecache_bytes) {
+          if (ctx->cdf_ecache) cudaFree(ctx->cdf_ecache);
+          ctx->cdf_ecache = nullptr;
+          ctx->cdf_ecache_bytes = 0;
+          if (cudaMalloc(&ctx->cdf_ecache, need_e) != cudaSuccess) {
+            cudaGetLastError();  // out of memory: the prefix walk keeps reading the logits, for good
             ctx->cdf_ecache = nullptr;
-            ctx->cdf_ecache_bytes = 0;
-            if (cudaMalloc(&ctx->cdf_ecache, need_e) != cudaSuccess) {
-              cudaGetLastError();  // out of memory: the prefix walk keeps reading the logits, for good
-              ctx->cdf_ecache = nullptr;
-              ctx->cdf_ecache_failed = true;
-              ok = false;
-            } else {
-              ctx->cdf_ecache_bytes = need_e;
-            }
+            ctx->cdf_ecache_failed = true;
+            ok = false;
+          } else {
+            ctx->cdf_ecache_bytes = need_e;
           }
         }
       }
-      if (ok) {
-        eoff = (uint32_t *)ctx->cdf_eoff;
-        eflag = (int *)(eoff + M + 1);
-        ecache = (double *)ctx->cdf_ecache;
-        const int n_sym = mode == CZ_CDF_RWKV_LITERALS ? (int)V + 256 : (int)V;
-        CZ_LAUNCH(ctx, CZ_K_CDF, (czk::ecache_offsets_kernel<<<1, 1024, 0, stream>>>(arg_dev, M, (int)V, n_sym, eoff, (unsigned long long)cap_groups, eflag)));
-        CZ_CHECK_LAUNCH();
-        ctx->cdf_eflag_last = eflag;
-      }
     }
-    if (tma_ok) {
-      CUtensorMap tm;
-      CZ_TRY(make_logits_map(&tm, logits_dev, V, ld, mode == CZ_CDF_RWKV_LITERALS ? czk::StCfg<CZ_CDF_RWKV_LITERALS>::ROWS : czk::StCfg<CZ_CDF_SMOLLM>::ROWS));
-      static bool attr = false;
-      if (!attr) {
-#define CZ_TMA_ATTR(MODE, OP) \
-  CZ_CUDA_TRY(cudaFuncSetAttribute(czk::cdf_stats_tma_kernel<MODE, OP>, cudaFuncAttributeMaxDynamicSharedMemorySize, czk::StCfg<MODE>::SMEM))
-        CZ_TMA_ATTR(CZ_CDF_SMOLLM, czk::OP_BOUNDS);
-        CZ_TMA_ATTR(CZ_CDF_SMOLLM, czk::OP_XE);
-        CZ_TMA_ATTR(CZ_CDF_RWKV_LITERALS, czk::OP_BOUNDS);
-        CZ_TMA_ATTR(CZ_CDF_RWKV_LITERALS, czk::OP_XE);
-        CZ_TMA_ATTR(CZ_CDF_SMOLLM_FLOOR, czk::OP_BOUNDS);
-#undef CZ_TMA_ATTR
-        attr = true;
-      }
-      const unsigned g = (unsigned)ceil_div(M, (size_t)czk::ST_COLS);
-#define CZ_TMA_STATS(MODE, OP)                                                                                                        \
-  CZ_LAUNCH(ctx, CZ_K_CDF,                                                                                                            \
-            (czk::cdf_stats_tma_kernel<MODE, OP><<<g, czk::ST_COLS + 32, czk::StCfg<MODE>::SMEM, stream>>>(tm, lg, (int)V, M, ld, colmax_dev, stats, \
-                                                                                                 ctx->err_flag_dev, arg_dev, eoff, ecache, eflag)))
-      if (mode == CZ_CDF_SMOLLM) {
-        if (op == czk::OP_BOUNDS) CZ_TMA_STATS(CZ_CDF_SMOLLM, czk::OP_BOUNDS);
-        else CZ_TMA_STATS(CZ_CDF_SMOLLM, czk::OP_XE);
-      } else if (mode == CZ_CDF_RWKV_LITERALS) {
-        if (op == czk::OP_BOUNDS) CZ_TMA_STATS(CZ_CDF_RWKV_LITERALS, czk::OP_BOUNDS);
-        else CZ_TMA_STATS(CZ_CDF_RWKV_LITERALS, czk::OP_XE);
-      } else {
-        CZ_TMA_STATS(CZ_CDF_SMOLLM_FLOOR, czk::OP_BOUNDS);  // (OP_XE runs as mode 0)
-      }
-#undef CZ_TMA_STATS
+    if (ok) {
+      eoff = (uint32_t *)ctx->cdf_eoff;
+      eflag = (int *)(eoff + M + 1);
+      ecache = (double *)ctx->cdf_ecache;
+      const int n_sym = MODE == CZ_CDF_RWKV_LITERALS ? (int)V + 256 : (int)V;
+      CZ_LAUNCH(ctx, CZ_K_CDF, (czk::ecache_offsets_kernel<<<1, 1024, 0, stream>>>(syms_dev, M, (int)V, n_sym, eoff, (unsigned long long)cap_groups, eflag)));
       CZ_CHECK_LAUNCH();
+      ctx->cdf_eflag_last = eflag;
     }
-    const unsigned g_stats = (unsigned)ceil_div(ceil_div(M, (size_t)ncol), 128);
-    if (!tma_ok) {
-#define CZ_STATS(MODE, OP, NC)                                                                                                   \
-  CZ_LAUNCH(ctx, CZ_K_CDF,                                                                                                       \
-            (czk::cdf_stats_kernel<MODE, OP, NC><<<g_stats, 128, 0, stream>>>(lg, (int)V, M, ld, colmax_dev, stats, ctx->err_flag_dev)))
-#define CZ_STATS_N(MODE, OP)            \
-  do {                                  \
-    if (ncol == 4) CZ_STATS(MODE, OP, 4); \
-    else if (ncol == 2) CZ_STATS(MODE, OP, 2); \
-    else CZ_STATS(MODE, OP, 1);         \
-  } while (0)
-    if (mode == CZ_CDF_SMOLLM) {
-      if (op == czk::OP_BOUNDS) CZ_STATS_N(CZ_CDF_SMOLLM, czk::OP_BOUNDS);
-      else CZ_STATS_N(CZ_CDF_SMOLLM, czk::OP_XE);
-    } else if (mode == CZ_CDF_RWKV_LITERALS) {
-      if (op == czk::OP_BOUNDS) CZ_STATS_N(CZ_CDF_RWKV_LITERALS, czk::OP_BOUNDS);
-      else CZ_STATS_N(CZ_CDF_RWKV_LITERALS, czk::OP_XE);
-    } else {
-      CZ_STATS_N(CZ_CDF_SMOLLM_FLOOR, czk::OP_BOUNDS);  // (OP_XE runs as mode 0)
-    }
-#undef CZ_STATS_N
-#undef CZ_STATS
-    CZ_CHECK_LAUNCH();
-    }
-    if (op == czk::OP_BOUNDS) {
-      // persistent warps pulling columns from a counter in the ctx's status block (word 12; the attention kernel's is word 8)
-      unsigned int *counter = reinterpret_cast<unsigned int *>(ctx->err_flag_dev + 12);
-      CZ_CUDA_TRY(cudaMemsetAsync(counter, 0, sizeof(unsigned int), stream));
-      const size_t want_ctas = ceil_div(M, 8);
-      const unsigned g = (unsigned)std::min<size_t>(want_ctas, (size_t)ctx->sm_count * 8);
-#define CZ_PREFIX(MODE, CACHED)                                                                                                          \
-  CZ_LAUNCH(ctx, CZ_K_CDF_PREFIX,                                                                                                        \
-            (czk::cdf_bounds_warp_kernel<MODE, CACHED><<<g, 256, 0, stream>>>(logits_dev, (int)V, M, ld, arg_dev, stats, c_lo_dev, c_hi_dev, \
-                                                                              ctx->err_flag_dev, counter, eoff, ecache, eflag)))
-      // with an e-cache both variants are issued: the flag the offsets kernel wrote decides on the device which one works
-      if (mode == CZ_CDF_SMOLLM) {
-        if (ecache) CZ_PREFIX(CZ_CDF_SMOLLM, true);
-        CZ_PREFIX(CZ_CDF_SMOLLM, false);
-      } else if (mode == CZ_CDF_RWKV_LITERALS) {
-        if (ecache) CZ_PREFIX(CZ_CDF_RWKV_LITERALS, true);
-        CZ_PREFIX(CZ_CDF_RWKV_LITERALS, false);
-      } else {
-        if (ecache) CZ_PREFIX(CZ_CDF_SMOLLM_FLOOR, true);
-        CZ_PREFIX(CZ_CDF_SMOLLM_FLOOR, false);
-      }
-#undef CZ_PREFIX
-    } else {
-      const unsigned g = (unsigned)ceil_div(M, 128);
-      if (mode == CZ_CDF_SMOLLM)
-        CZ_LAUNCH(ctx, CZ_K_CDF,
-                  (czk::cdf_xe_final_kernel<CZ_CDF_SMOLLM><<<g, 128, 0, stream>>>(logits_dev, (int)V, M, ld, arg_dev, stats, xe_dev)));
-      else
-        CZ_LAUNCH(ctx, CZ_K_CDF,
-                  (czk::cdf_xe_final_kernel<CZ_CDF_RWKV_LITERALS><<<g, 128, 0, stream>>>(logits_dev, (int)V, M, ld, arg_dev, stats, xe_dev)));
-    }
-    CZ_CHECK_LAUNCH();
-    return CZ_OK;
   }
-  const int threads = 128;
-  dim3 grid((unsigned)ceil_div(M, threads));
-#define CZ_CDF_CASE(MODE, OP)                                                                                 \
-  CZ_LAUNCH(ctx, CZ_K_CDF,                                                                                    \
-            (czk::cdf_cols_kernel<MODE, OP><<<grid, threads, 0, stream>>>(logits_dev, (int)V, M, ld, arg_dev, \
-                                                                          sym_out_dev, c_lo_dev, c_hi_dev,    \
-                                                                          xe_dev, ctx->err_flag_dev, colmax_dev)))
-  if (mode == CZ_CDF_SMOLLM) {
-    if (op == czk::OP_BOUNDS) CZ_CDF_CASE(CZ_CDF_SMOLLM, czk::OP_BOUNDS);
-    else if (op == czk::OP_SEARCH) CZ_CDF_CASE(CZ_CDF_SMOLLM, czk::OP_SEARCH);
-    else CZ_CDF_CASE(CZ_CDF_SMOLLM, czk::OP_XE);
-  } else if (mode == CZ_CDF_RWKV_LITERALS) {
-    if (op == czk::OP_BOUNDS) CZ_CDF_CASE(CZ_CDF_RWKV_LITERALS, czk::OP_BOUNDS);
-    else if (op == czk::OP_SEARCH) CZ_CDF_CASE(CZ_CDF_RWKV_LITERALS, czk::OP_SEARCH);
-    else CZ_CDF_CASE(CZ_CDF_RWKV_LITERALS, czk::OP_XE);
+  if (tma_ok) {
+    CUtensorMap tm;
+    CZ_TRY(make_logits_map(&tm, logits_dev, V, ld, czk::StCfg<MODE>::ROWS));
+    static bool attr = false;
+    if (!attr) {
+      CZ_CUDA_TRY(cudaFuncSetAttribute(czk::cdf_stats_tma_kernel<MODE, OP>, cudaFuncAttributeMaxDynamicSharedMemorySize, czk::StCfg<MODE>::SMEM));
+      attr = true;
+    }
+    const unsigned g = (unsigned)ceil_div(M, (size_t)czk::ST_COLS);
+    CZ_LAUNCH(ctx, CZ_K_CDF,
+              (czk::cdf_stats_tma_kernel<MODE, OP><<<g, czk::ST_COLS + 32, czk::StCfg<MODE>::SMEM, stream>>>(
+                  tm, lg, (int)V, M, ld, colmax_dev, stats, ctx->err_flag_dev, syms_dev, eoff, ecache, eflag)));
   } else {
-    if (op == czk::OP_BOUNDS) CZ_CDF_CASE(CZ_CDF_SMOLLM_FLOOR, czk::OP_BOUNDS);
-    else CZ_CDF_CASE(CZ_CDF_SMOLLM_FLOOR, czk::OP_SEARCH);  // (OP_XE runs as mode 0)
+    const unsigned g = (unsigned)ceil_div(M, 128);
+    CZ_LAUNCH(ctx, CZ_K_CDF, (czk::cdf_stats_kernel<MODE, OP><<<g, 128, 0, stream>>>(lg, (int)V, M, ld, colmax_dev, stats, ctx->err_flag_dev)));
   }
-#undef CZ_CDF_CASE
+  CZ_CHECK_LAUNCH();
+  if constexpr (OP == czk::OP_BOUNDS) {
+    // persistent warps pulling columns from a counter in the ctx's status block (word 12; the attention kernel's is word 8)
+    unsigned int *counter = reinterpret_cast<unsigned int *>(ctx->err_flag_dev + 12);
+    CZ_CUDA_TRY(cudaMemsetAsync(counter, 0, sizeof(unsigned int), stream));
+    const size_t want_ctas = ceil_div(M, 8);
+    const unsigned g = (unsigned)std::min<size_t>(want_ctas, (size_t)ctx->sm_count * 8);
+    auto prefix = [&](auto cached) {
+      CZ_LAUNCH(ctx, CZ_K_CDF_PREFIX,
+                (czk::cdf_bounds_warp_kernel<MODE, decltype(cached)::value><<<g, 256, 0, stream>>>(
+                    logits_dev, (int)V, M, ld, syms_dev, stats, c_lo_dev, c_hi_dev, ctx->err_flag_dev, counter, eoff, ecache, eflag)));
+    };
+    // with an e-cache both variants are issued: the flag the offsets kernel wrote decides on the device which one works
+    if (ecache) prefix(std::true_type{});
+    prefix(std::false_type{});
+  } else {
+    const unsigned g = (unsigned)ceil_div(M, 128);
+    CZ_LAUNCH(ctx, CZ_K_CDF, (czk::cdf_xe_final_kernel<MODE><<<g, 128, 0, stream>>>(logits_dev, (int)V, M, ld, syms_dev, stats, xe_dev)));
+  }
   CZ_CHECK_LAUNCH();
   return CZ_OK;
 }
 
+// Device-pointer launchers (used by the executor and by the host-buffer C-ABI wrappers in api.cu)
+int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size_t V, size_t M, size_t ld,
+                    const uint32_t *arg_dev, uint32_t *sym_out_dev, uint32_t *c_lo_dev, uint32_t *c_hi_dev,
+                    double *xe_dev, cudaStream_t stream, const int *colmax_dev) {
+  // OP_XE evaluates the floored pdf for SmolLM whatever the coding alphabet (src/main.rs:1745): mode 2 IS mode 0 there
+  if (op == czk::OP_XE && mode == CZ_CDF_SMOLLM_FLOOR) mode = CZ_CDF_SMOLLM;
+  return with_cdf_mode(mode, [&](auto mode_c) -> int {
+    constexpr int MODE = decltype(mode_c)::value;
+    if (M == 0) return CZ_OK;
+    if (V == 0 || V > (1u << 24) || ld < M) {
+      set_error("cdf: bad shape");
+      return CZ_ERR_INVALID;
+    }
+    if (op == czk::OP_SEARCH) {  // warp per column
+      const unsigned g = (unsigned)ceil_div(M, 8);  // 4 warps x 2 columns
+      CZ_LAUNCH(ctx, CZ_K_CDF,
+                (czk::cdf_search_warp_kernel<MODE><<<g, 128, 0, stream>>>(logits_dev, (int)V, M, ld, arg_dev, sym_out_dev, c_lo_dev, c_hi_dev,
+                                                                         ctx->err_flag_dev, colmax_dev)));
+      CZ_CHECK_LAUNCH();
+      return CZ_OK;
+    }
+    if constexpr (MODE != CZ_CDF_SMOLLM_FLOOR)  // (mode 2's XE runs as mode 0: no such kernels)
+      if (op == czk::OP_XE)
+        return launch_cdf_encode<MODE, czk::OP_XE>(ctx, logits_dev, V, M, ld, arg_dev, c_lo_dev, c_hi_dev, xe_dev, stream, colmax_dev);
+    return launch_cdf_encode<MODE, czk::OP_BOUNDS>(ctx, logits_dev, V, M, ld, arg_dev, c_lo_dev, c_hi_dev, xe_dev, stream, colmax_dev);
+  });
+}
+
 int launch_cdf_full(cz_ctx *ctx, int mode, const float *logits_dev, size_t V, uint32_t *cdf_dev, cudaStream_t stream) {
-  if (mode == CZ_CDF_SMOLLM)
-    CZ_LAUNCH(ctx, CZ_K_CDF, (czk::cdf_full_kernel<CZ_CDF_SMOLLM><<<1, 32, 0, stream>>>(logits_dev, (int)V, cdf_dev)));
-  else if (mode == CZ_CDF_RWKV_LITERALS)
-    CZ_LAUNCH(ctx, CZ_K_CDF,
-              (czk::cdf_full_kernel<CZ_CDF_RWKV_LITERALS><<<1, 32, 0, stream>>>(logits_dev, (int)V, cdf_dev)));
-  else if (mode == CZ_CDF_SMOLLM_FLOOR)
-    CZ_LAUNCH(ctx, CZ_K_CDF, (czk::cdf_full_kernel<CZ_CDF_SMOLLM_FLOOR><<<1, 32, 0, stream>>>(logits_dev, (int)V, cdf_dev)));
-  else {
-    set_error("cdf: unknown mode");
-    return CZ_ERR_INVALID;
-  }
-  CZ_CHECK_LAUNCH();
-  return CZ_OK;
+  return with_cdf_mode(mode, [&](auto mode_c) -> int {
+    CZ_LAUNCH(ctx, CZ_K_CDF, (czk::cdf_full_kernel<decltype(mode_c)::value><<<1, 32, 0, stream>>>(logits_dev, (int)V, cdf_dev)));
+    CZ_CHECK_LAUNCH();
+    return CZ_OK;
+  });
 }
 
 }  // namespace cz

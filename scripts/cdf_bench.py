@@ -2,8 +2,9 @@
 """Micro-benchmark of the encode-side CDF kernels on a device-resident logits batch (GPU box only).
     python scripts/cdf_bench.py [mode=0] [cols=131072]
 Times cz_cdf_bounds_dev with CUDA events for: coded symbol 0 everywhere (the full passes alone), symbols distributed like the
-bench's spread byte ids, and uniform symbols; for each of CZ_CDF_NCOL = 1, 2, 4 and the round-1 kernel (CZ_CDF_LEGACY is read once
-per process, so the legacy numbers come from a second invocation: `CZ_CDF_LEGACY=1 python scripts/cdf_bench.py`)."""
+bench's spread byte ids, and uniform symbols; with the e-cache (`tma`) and without it (`tma_noecache`: the prefix walk reads the
+logits).  The batch's row stride is `cols`.  The TMA-staged stats kernel needs a stride that is a multiple of 4, so an odd `cols`
+(e.g. 131071) times the direct-load stats kernel instead, and without an e-cache in both variants."""
 import ctypes as C
 import json
 import os
@@ -33,17 +34,14 @@ hi = torch.empty(M, dtype=torch.int32, device="cuda")
 data = corpus.load("enwik8_3mib")
 ids = corpus.byte_ids((data * (M // len(data) + 1))[:M], V, True)
 cases = {"sym0": np.zeros(M, np.uint32), "spread_ids": ids, "uniform": np.random.default_rng(0).integers(0, V, M).astype(np.uint32)}
-res = {"mode": mode, "V": V, "cols": M, "legacy": bool(os.environ.get("CZ_CDF_LEGACY"))}
-variants = ("legacy",) if res["legacy"] else ("tma", "tma_noecache", "ncol1")
+res = {"mode": mode, "V": V, "cols": M}
+variants = ("tma", "tma_noecache")
 if os.environ.get("CDF_BENCH_VARIANTS"):
     variants = tuple(os.environ["CDF_BENCH_VARIANTS"].split(","))
-for ncol in variants:
-    os.environ.pop("CZ_CDF_NCOL", None)
+for variant in variants:
     os.environ.pop("CZ_CDF_NO_ECACHE", None)
-    if ncol == "tma_noecache":  # the prefix walk reads the vocab-major logits instead of the e-cache the stats pass fills
+    if variant == "tma_noecache":  # the prefix walk reads the vocab-major logits instead of the e-cache the stats pass fills
         os.environ["CZ_CDF_NO_ECACHE"] = "1"
-    if ncol == "ncol1":  # the direct-load kernel (a forced column width keeps the TMA-staged variant off)
-        os.environ["CZ_CDF_NCOL"] = "1"
     for name, syms in cases.items():
         s_dev = torch.from_numpy(syms.astype(np.int64)).to(torch.int32).cuda()
         ts = []
@@ -57,6 +55,6 @@ for ncol in variants:
             e1.record(stream)
             torch.cuda.synchronize()
             ts.append(e0.elapsed_time(e1))
-        res[f"{ncol}_{name}_ms"] = round(min(ts), 3)
-        res[f"{ncol}_{name}_GBps_algorithmic"] = round(4.0 * V * M * (1 + syms.astype(np.float64).mean() / V) / min(ts) / 1e6, 1)
+        res[f"{variant}_{name}_ms"] = round(min(ts), 3)
+        res[f"{variant}_{name}_GBps_algorithmic"] = round(4.0 * V * M * (1 + syms.astype(np.float64).mean() / V) / min(ts) / 1e6, 1)
 print(json.dumps(res))

@@ -50,25 +50,19 @@ def _check_k1(gpu_ctx, logits, syms, rng):
 
 
 @pytest.mark.parametrize("v", [1024, 4099, 49152])
-def test_k1_floor_mode_bit_exact_tma_direct_and_vector_widths(gpu_ctx, v):
-    """every kernel family of mode 2: the TMA-staged stats pass (>= 256 aligned columns), the direct-load stats kernel (40 columns, and
-    CZ_CDF_NCOL = 1 / 2 / 4), the warp-per-column prefix walk, the warp search; a column whose entries are mostly > 87 below the max
-    (the fast expf's conversion fallback); symbols at both ends of the alphabet; cz_cdf_full"""
+def test_k1_floor_mode_bit_exact_tma_and_direct(gpu_ctx, v):
+    """every kernel family of mode 2: the TMA-staged stats pass (260 and 1024 columns), the direct-load stats kernel (40 columns, and
+    the odd counts: ld = m is not a multiple of 4), the warp-per-column prefix walk, the warp search (also over more than 8,192
+    columns); a column whose entries are mostly > 87 below the max (the fast expf's conversion fallback); symbols at both ends of
+    the alphabet; cz_cdf_full"""
     rng = np.random.default_rng(v)
-    try:
-        for ncol in (0, 1, 2, 4):
-            if ncol:
-                os.environ["CZ_CDF_NCOL"] = str(ncol)
-            for m in ((40, 260, 1024) if v < 49152 or ncol in (0, 2) else (260,)):
-                logits = adversarial_logits(rng, v, m)
-                logits[:, m // 2] = rng.normal(0, 30, v)
-                syms = rng.integers(0, v, m).astype(np.uint32)
-                syms[:6] = [0, v - 1, 1, v - 2, 5, v // 3]
-                _check_k1(gpu_ctx, logits, syms, rng)
-            os.environ.pop("CZ_CDF_NCOL", None)
-    finally:
-        os.environ.pop("CZ_CDF_NCOL", None)
-    if v == 1024:  # more columns than the warp search takes: the thread-per-column search (cdf_cols_kernel)
+    for m in (40, 260, 261, 1024, 1027):
+        logits = adversarial_logits(rng, v, m)
+        logits[:, m // 2] = rng.normal(0, 30, v)
+        syms = rng.integers(0, v, m).astype(np.uint32)
+        syms[:6] = [0, v - 1, 1, v - 2, 5, v // 3]
+        _check_k1(gpu_ctx, logits, syms, rng)
+    if v == 1024:  # a search over more columns than a decode step has streams: the same warp kernel
         logits = adversarial_logits(rng, v, 8200)
         values = rng.integers(0, 1 << 30, 8200).astype(np.uint32)
         s, slo, shi = gpu_ctx.cdf_search(logits, values, FLOOR)

@@ -339,43 +339,38 @@ def test_cdf_fast_paths_equal_the_originals_exhaustively(gpu_ctx):
         assert m.value == 0, m.value
 
 
-@pytest.mark.parametrize("ncol", [0, 1, 2, 4])
+@pytest.mark.parametrize("m", [40, 260, 261, 1024, 1027])
 @pytest.mark.parametrize("mode", [0, 1])
-def test_cdf_bounds_and_xe_new_kernels_all_vector_widths(gpu_ctx, mode, ncol):
-    """the round-2 stats / sorted-prefix / XE kernels against the oracle for 1, 2 and 4 adjacent columns per thread (forced through
-    CZ_CDF_NCOL; by default the width follows the column count), with symbols at both ends of the alphabet, literal escapes,
-    logits more than 87 below the maximum (the conversion fallback), -inf entries and exact ties; then a model-level encode whose
-    ragged column counts go through the same width, checked against the oracle coder on the GPU's own logits."""
+def test_cdf_bounds_and_xe_tma_and_direct_stats_kernels(gpu_ctx, mode, m):
+    """the round-2 stats / sorted-prefix / XE kernels against the oracle on m columns (ld = m): 260 and 1024 take the TMA-staged
+    full passes, 40 (too few columns) and the odd counts (ld % 4 != 0) the direct-load kernel; with symbols at both ends of the
+    alphabet, literal escapes, logits more than 87 below the maximum (the conversion fallback), -inf entries and exact ties; then
+    (once) a model-level encode whose ragged column counts go through the same kernels, checked against the oracle coder on the
+    GPU's own logits."""
     import test_gpu_parity as tgp
 
-    if ncol:  # 0: the default path (TMA-staged full passes for >= 256 columns; 40 columns stay on the direct-load kernel)
-        os.environ["CZ_CDF_NCOL"] = str(ncol)
-    try:
-        rng = np.random.default_rng(100 + mode)
-        v = 2309 if mode else 2304
-        n_sym = v + 256 if mode else v
-        for m in (40, 260, 1024):
-            logits = tgp._adversarial_logits(rng, v, m)
-            logits[:, m // 2] = rng.normal(0, 30, v)      # most entries > 87 below the max: slow conversion path, tiny / zero terms
-            syms = rng.integers(0, n_sym, m).astype(np.uint32)
-            syms[:6] = [0, n_sym - 1, 1, v - 1, min(v, n_sym - 1), n_sym - 2]
-            lo, hi = gpu_ctx.cdf_bounds(logits, syms, mode)
-            xe = gpu_ctx.xe_bits_cols(logits, syms, mode)
-            for j in range(m):
-                cdf = oracle.logits_to_cdf(logits[:, j], mode)
-                assert (int(lo[j]), int(hi[j])) == (int(cdf[syms[j]]), int(cdf[syms[j] + 1])), (m, j, syms[j])
-                pdf = oracle.combined_pdf_with_literals(logits[:, j]) if mode else oracle.softmax_pdf_floor(logits[:, j])
-                want = -np.log2(max(pdf[syms[j]], 1e-300))
-                assert abs(xe[j] - want) <= 1e-12 * max(1.0, abs(want)), (m, j)
-        if mode == 0:
-            model = _tiny(gpu_ctx)
-            ids = rng.integers(0, 1024, 701).astype(np.uint32)
-            pays, seg = model.encode(ids, n_segments=1)
-            lg = np.concatenate([model.chunk_logits([0], ids[:512]), model.chunk_logits(np.concatenate([[0], ids])[2:513], ids[512:])])
-            bounds = [tuple(int(x) for x in oracle.logits_to_cdf(lg[j], 0)[[ids[j], ids[j] + 1]]) for j in range(701)]
-            assert oracle.ac_encode(bounds) == pays[0]
-    finally:
-        os.environ.pop("CZ_CDF_NCOL", None)
+    rng = np.random.default_rng([100 + mode, m])
+    v = 2309 if mode else 2304
+    n_sym = v + 256 if mode else v
+    logits = tgp._adversarial_logits(rng, v, m)
+    logits[:, m // 2] = rng.normal(0, 30, v)      # most entries > 87 below the max: slow conversion path, tiny / zero terms
+    syms = rng.integers(0, n_sym, m).astype(np.uint32)
+    syms[:6] = [0, n_sym - 1, 1, v - 1, min(v, n_sym - 1), n_sym - 2]
+    lo, hi = gpu_ctx.cdf_bounds(logits, syms, mode)
+    xe = gpu_ctx.xe_bits_cols(logits, syms, mode)
+    for j in range(m):
+        cdf = oracle.logits_to_cdf(logits[:, j], mode)
+        assert (int(lo[j]), int(hi[j])) == (int(cdf[syms[j]]), int(cdf[syms[j] + 1])), (m, j, syms[j])
+        pdf = oracle.combined_pdf_with_literals(logits[:, j]) if mode else oracle.softmax_pdf_floor(logits[:, j])
+        want = -np.log2(max(pdf[syms[j]], 1e-300))
+        assert abs(xe[j] - want) <= 1e-12 * max(1.0, abs(want)), (m, j)
+    if mode == 0 and m == 40:
+        model = _tiny(gpu_ctx)
+        ids = rng.integers(0, 1024, 701).astype(np.uint32)
+        pays, seg = model.encode(ids, n_segments=1)
+        lg = np.concatenate([model.chunk_logits([0], ids[:512]), model.chunk_logits(np.concatenate([[0], ids])[2:513], ids[512:])])
+        bounds = [tuple(int(x) for x in oracle.logits_to_cdf(lg[j], 0)[[ids[j], ids[j] + 1]]) for j in range(701)]
+        assert oracle.ac_encode(bounds) == pays[0]
 
 
 @pytest.mark.parametrize("mode", [0, 1])
