@@ -8,8 +8,12 @@ every input).  --segments N > 1 writes the SEG1 container extension (parallel de
 --on-zero-width {stored,floor}: what compress does when the SmolLM coder meets a token of mass < 2^-30 (codec.compress).
 compress-many / decompress-many IN... [--out-dir DIR]: many files through one encode call and lock-step decode waves of at most
 --max-streams streams (codec.compress_many / decompress_many); each .canz is the one `compress` writes for that file.
+analyze INPUT [OUTPUT]: per-token code lengths, coding-distribution entropies and positions (codec.analyze), tokenised and split as
+`compress` does, into OUTPUT (default INPUT.analysis.npz: the arrays, plus the summary as JSON under "summary"); prints the summary.
+--pdf-floor (analyze, SmolLM only) codes with the floored pdf.
 """
 import argparse
+import json
 import sys
 import time
 
@@ -124,9 +128,36 @@ def _main_many(args, ap):
     return 0
 
 
+def _print_summary(s):
+    bpb = lambda x: "n/a" if x is None else f"{x:.4f}"  # noqa: E731
+    print(f"{s['tokens']} tokens, {s['bytes']} bytes: {s['bits']:.1f} bits of code length ({bpb(s['bits_per_byte'])} bits/byte), "
+          f"{s['payload_bits']} payload bits ({bpb(s['payload_bits_per_byte'])} bits/byte)")
+    print(f"mean code length {s['mean_bits'] if s['mean_bits'] is None else round(s['mean_bits'], 4)} bits/token, "
+          f"mean entropy {s['mean_entropy'] if s['mean_entropy'] is None else round(s['mean_entropy'], 4)} bits/token, "
+          f"{s['zero_width']} zero-width tokens" + (f" (first: {s['first_zero_width']})" if s["zero_width"] else ""))
+    for g, seg in enumerate(s["segments"]):
+        print(f"  segment {g}: {seg['tokens']} tokens, {seg['bits']:.1f} bits, {seg['payload_bits']} payload bits")
+    for name, key in (("position in chunk", "by_chunk_position"), ("position in segment", "by_segment_position")):
+        print(f"  by {name}: " + ", ".join(f"{b['bucket']}: {'-' if b['mean_bits'] is None else format(b['mean_bits'], '.3f')}"
+                                          f"/{b['mean_entropy']:.3f}" for b in s[key]) + "  (mean bits / mean entropy)")
+
+
+def _analyze(args):
+    model, tok = _model(args)
+    data = open(args.input, "rb").read()
+    arrays, summary = codec.analyze(model, data, tok, args.segments, context=args.context, reprime_interval=args.reprime_interval,
+                                    pdf_floor=args.pdf_floor)
+    out = args.output or args.input + ".analysis.npz"
+    with open(out, "wb") as f:  # (a file object: np.savez would append .npz to a name without it)
+        np.savez(f, summary=np.array(json.dumps(summary)), **arrays)
+    _print_summary(summary)
+    print(f"wrote {out}")
+    return 0
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(prog="candlezip_b200")
-    ap.add_argument("command", choices=["compress", "decompress", "self-test", "compress-many", "decompress-many"])
+    ap.add_argument("command", choices=["compress", "decompress", "self-test", "compress-many", "decompress-many", "analyze"])
     ap.add_argument("input", nargs="+", help="INPUT [OUTPUT]; compress-many / decompress-many: one or more inputs")
     ap.add_argument("--backend", choices=["smollm", "rwkv7"], default="smollm")
     ap.add_argument("--context", type=int, default=512)
@@ -148,12 +179,20 @@ def main(argv=None):
     ap.add_argument("--scan-output-dir", help="where the proof.csv ledger of a scan goes")
     ap.add_argument("--out-dir", help="compress-many / decompress-many: where NAME.canz / NAME.out go (default: beside each input)")
     ap.add_argument("--max-streams", type=int, help="decompress-many: most segments decoded together in one lock-step wave; default 2048")
+    ap.add_argument("--pdf-floor", action="store_true", help="analyze: code with the floored SmolLM pdf (no token is zero-width)")
     args = ap.parse_args(argv)
     # flags that only one side uses are refused on the other instead of being ignored
     if args.command == "decompress-many" and (args.segments is not None or args.on_zero_width):
         ap.error("--segments and --on-zero-width are compress settings: a container carries its own (decompress-many)")
     if args.command != "decompress-many" and args.max_streams is not None:
         ap.error("--max-streams applies to decompress-many only")
+    if args.pdf_floor and (args.command != "analyze" or args.backend != "smollm"):
+        ap.error("--pdf-floor applies to analyze on the SmolLM backend only (RWKV-7 codes with a floored alphabet already)")
+    if args.command == "analyze":
+        for flag, val in (("--reuse-scan-dir", args.reuse_scan_dir), ("--on-zero-width", args.on_zero_width), ("--out-dir", args.out_dir),
+                          ("--max-streams", args.max_streams)):
+            if val is not None:
+                ap.error(f"{flag} is not available with analyze")
     if args.segments is None:
         args.segments = 1
     if args.command.endswith("-many"):
@@ -167,6 +206,8 @@ def main(argv=None):
     if len(args.input) > 2:
         ap.error(f"{args.command} takes INPUT [OUTPUT]")
     args.input, args.output = args.input[0], (args.input[1] if len(args.input) > 1 else None)
+    if args.command == "analyze":
+        return _analyze(args)
     scan = bool(args.reuse_scan_dir)
     if scan and (args.backend != "smollm" or args.segments != 1):
         ap.error("--reuse-scan-dir works on the SmolLM backend with one AC stream (--segments 1), like the reference's container")

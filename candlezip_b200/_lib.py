@@ -103,6 +103,7 @@ SIGNATURES = {
     "cz_cdf_search": (C.c_int, [_vp, f32p, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, u32p, u32p, u32p, u32p]),
     "cz_cdf_full": (C.c_int, [_vp, f32p, C.c_size_t, C.c_int, u32p]),
     "cz_xe_bits_cols": (C.c_int, [_vp, f32p, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, u32p, f64p]),
+    "cz_cdf_entropy": (C.c_int, [_vp, f32p, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, f64p]),
     "cz_ac_encode_lanes": (C.c_int, [_vp, u32p, u32p, u64p, C.c_size_t, u8p, u64p, u64p]),
     "cz_ac_decode_lanes": (C.c_int, [_vp, u8p, u64p, u64p, u64p, C.c_size_t, u32p, C.c_size_t, u32p]),
     "cz_model_config_smollm_135m": (None, [C.POINTER(ModelConfig)]),
@@ -129,6 +130,7 @@ SIGNATURES = {
     "cz_model_set_digest_out": (C.c_int, [_vp, u8p, C.c_size_t]),
     "cz_model_set_pdf_floor": (C.c_int, [_vp, C.c_int]),
     "cz_model_set_zero_width_out": (C.c_int, [_vp, u64p, C.c_size_t]),
+    "cz_model_set_code_length_out": (C.c_int, [_vp, u32p, u32p, f64p, C.c_size_t]),
     "cz_xe_bits": (C.c_int, [_vp, C.POINTER(XeJob), C.c_size_t, f64p]),
     "cz_chunk_logits": (C.c_int, [_vp, u32p, C.c_size_t, u32p, C.c_size_t, f32p]),
     "cz_container_header_size": (C.c_size_t, [C.POINTER(HeaderV2)]),

@@ -115,6 +115,15 @@ class Context:
         check(lib.cz_xe_bits_cols(self._h, p, v, m, m, mode, sp, out.ctypes.data_as(_lib.f64p)))
         return out
 
+    def cdf_entropy(self, logits_vm, mode=_lib.CZ_CDF_SMOLLM):
+        """logits_vm: [V, M] vocab-major float32.  Returns float64 [M]: the expected code length in bits of each column's quantised coding
+        distribution, 2^-30 sum_s w_s (30 - log2 w_s) over the widths w_s of the CDF the coder uses in `mode` (cz_cdf_entropy)."""
+        a, p = _f32(logits_vm)
+        v, m = a.shape
+        out = np.empty(m, np.float64)
+        check(lib.cz_cdf_entropy(self._h, p, v, m, m, mode, out.ctypes.data_as(_lib.f64p)))
+        return out
+
     # ---- K2 / K3 ----
     def ac_encode_lanes(self, c_lo, c_hi, lane_off):
         """Returns a list of payload bytes, one per lane."""
@@ -284,6 +293,53 @@ class Model:
         pay = [data[int(seg_off[g]) : int(seg_off[g + 1])].tobytes() for g in range(int(s.n_segments))]
         return (pay, seg_start, first_zw[: int(s.n_segments)]) if zero_width_out else (pay, seg_start)
 
+    def analyze(self, ids, n_segments=1, seg_start=None, bos=0, context=512, reprime_interval=512, pdf_floor=False, max_batch_tokens=0):
+        """Where the bits go: encodes ids as encode() does, with the code-length and zero-width sinks set (cleared again afterwards).
+        Returns a dict with
+          payloads, seg_start   as encode() returns them
+          first_zw              per segment, its first zero-width token (segment-relative) or _lib.NO_ZERO_WIDTH (that segment's
+                                payload is unspecified)
+          c_lo, c_hi            uint32 [n]: the interval each token was coded with
+          bits                  float64 [n]: 30 - log2(c_hi - c_lo), the token's exact code length before coder overhead; +inf where the
+                                interval is empty (a zero-width token)
+          entropy               float64 [n]: the expected code length of the distribution the token was coded from (cz_cdf_entropy), in
+                                the alphabet of the call (pdf_floor applies)"""
+        a, p = _u32(ids)
+        n = a.shape[0]
+        if self.cfg.get("arch", 0) == _lib.CZ_ARCH_RWKV7 and pdf_floor:
+            raise ValueError("pdf_floor: RWKV-7 codes with a floored alphabet already")
+        if context < 1 or reprime_interval < 1:
+            raise ValueError("context and reprime_interval must be >= 1")
+        if seg_start is None:
+            if n_segments < 1:
+                raise ValueError("n_segments must be >= 1")
+            seg_start = split_segments(n, n_segments)
+        else:
+            seg_start = np.asarray(seg_start, np.uint64)
+            if seg_start.ndim != 1 or seg_start.shape[0] < 2 or int(seg_start[0]) != 0 or int(seg_start[-1]) != n or np.any(np.diff(seg_start.astype(np.int64)) < 0):
+                raise ValueError(f"seg_start must run from 0 to len(ids) = {n}, non-decreasing")
+        self.set_pdf_floor(pdf_floor)
+        s, keep = self._schedule(n, seg_start, bos, context, reprime_interval, None, max_batch_tokens)
+        n_seg = int(s.n_segments)
+        cap = 4 * n + 8 * n_seg + 16
+        data = np.empty(cap, np.uint8)
+        seg_off = np.zeros(n_seg + 1, np.uint64)
+        bs = _lib.Bitstreams(data.ctypes.data_as(_lib.u8p), cap, seg_off.ctypes.data_as(_lib.u64p))
+        c_lo, c_hi, ent = np.zeros(max(n, 1), np.uint32), np.zeros(max(n, 1), np.uint32), np.zeros(max(n, 1), np.float64)
+        first_zw = np.zeros(max(1, n_seg), np.uint64)
+        check(lib.cz_model_set_zero_width_out(self._h, first_zw.ctypes.data_as(_lib.u64p), first_zw.shape[0]))
+        try:
+            check(lib.cz_model_set_code_length_out(self._h, c_lo.ctypes.data_as(_lib.u32p), c_hi.ctypes.data_as(_lib.u32p),
+                                                   ent.ctypes.data_as(_lib.f64p), c_lo.shape[0]))
+            check(lib.cz_encode(self._h, p, n, C.byref(s), C.byref(bs)))
+        finally:
+            check(lib.cz_model_set_code_length_out(self._h, None, None, None, 0))
+            check(lib.cz_model_set_zero_width_out(self._h, None, 0))
+        pay = [data[int(seg_off[g]) : int(seg_off[g + 1])].tobytes() for g in range(n_seg)]
+        c_lo, c_hi, ent = c_lo[:n], c_hi[:n], ent[:n]
+        return dict(payloads=pay, seg_start=seg_start, first_zw=first_zw[:n_seg], c_lo=c_lo, c_hi=c_hi, bits=code_length_bits(c_lo, c_hi),
+                    entropy=ent)
+
     def decode(self, payloads, seg_start, bos=0, context=512, reprime_interval=512, max_batch_tokens=0, events=None, pdf_floor=False):
         """events: the same gated hint primes the encoder was given (src/main.rs:2586-2614), single segment only;
         pdf_floor: the setting the stream was encoded with"""
@@ -326,6 +382,13 @@ def xe_make_prime(history, hint, max_ctx=511):
     hb = min(len(hint), max_ctx)
     take = min(max_ctx - hb, len(history))
     return np.concatenate([history[len(history) - take :], hint[:hb]]).astype(np.uint32)
+
+
+def code_length_bits(c_lo, c_hi):
+    """30 - log2(c_hi - c_lo) per interval of total 2^30 (float64), +inf for an empty interval"""
+    w = np.asarray(c_hi, np.int64) - np.asarray(c_lo, np.int64)
+    with np.errstate(divide="ignore"):
+        return 30.0 - np.log2(w.astype(np.float64))
 
 
 class Session:

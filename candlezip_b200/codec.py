@@ -350,3 +350,103 @@ def decompress_many(model, blobs, tokenizer=None, max_streams=2048, verify=True)
         except ValueError as e:
             raise ValueError(f"blob {i}: {e}") from None
     return out
+
+
+# ---- per-token code lengths ----------------------------------------------------------------------------------------------------------
+# analyze() reports where in a file the bits go: each token's exact code length (from the interval it was coded with), the entropy of
+# the distribution it was coded from (the model's uncertainty, as opposed to its surprise at the actual token), and where the token sits
+# in its segment and in its reprime chunk.  Everything below except analyze() itself is pure and needs no device.
+
+def schedule_chunks(n_tokens, context, reprime_interval):
+    """(first coded index, number coded) of each chunk of one segment of n_tokens (cz_schedule_chunks, host-only): a chunk starts from
+    BOS or from a reprime of the last min(context, 511) tokens"""
+    k = int(_lib.lib.cz_schedule_chunks(int(n_tokens), int(context), int(reprime_interval), None, None, None, None, 0))
+    first, n_coded = np.zeros(max(k, 1), np.uint64), np.zeros(max(k, 1), np.uint32)
+    _lib.lib.cz_schedule_chunks(int(n_tokens), int(context), int(reprime_interval), first.ctypes.data_as(_lib.u64p),
+                                n_coded.ctypes.data_as(_lib.u32p), None, None, k)
+    return first[:k].astype(np.int64), n_coded[:k].astype(np.int64)
+
+
+def token_positions(seg_start, context, reprime_interval, reprime=True):
+    """per coded token: segment index, position in the segment, reprime-chunk index in the segment and position in the chunk.
+    reprime=False (RWKV-7, whose state runs over the whole segment): one chunk per segment."""
+    seg_start = np.asarray(seg_start, np.int64)
+    n = int(seg_start[-1])
+    seg, pos, chunk, cpos = (np.zeros(n, np.int64) for _ in range(4))
+    for g in range(len(seg_start) - 1):
+        a, b = int(seg_start[g]), int(seg_start[g + 1])
+        seg[a:b] = g
+        pos[a:b] = np.arange(b - a)
+        if b == a:
+            continue
+        first, n_coded = schedule_chunks(b - a, context, reprime_interval) if reprime else (np.zeros(1, np.int64), np.array([b - a]))
+        for c, (f, k) in enumerate(zip(first, n_coded)):
+            chunk[a + f:a + f + k] = c
+            cpos[a + f:a + f + k] = np.arange(k)
+    return seg, pos, chunk, cpos
+
+
+def pos_bucket(pos):
+    """power-of-two bucket of a position: 0 -> 0, 1 -> 1, 2-3 -> 2, 4-7 -> 3, ..."""
+    p = np.array(pos, np.int64)
+    out = np.zeros(p.shape, np.int64)
+    while np.any(p > 0):  # bit length
+        out += p > 0
+        p >>= 1
+    return out
+
+
+def bucket_label(b):
+    return "0" if b == 0 else "1" if b == 1 else f"{1 << (b - 1)}-{(1 << b) - 1}"
+
+
+def bucket_means(pos, bits, entropy):
+    """mean code length (finite bits only) and mean entropy per power-of-two position bucket"""
+    bk = pos_bucket(pos)
+    bits, entropy = np.asarray(bits, np.float64), np.asarray(entropy, np.float64)
+    out = []
+    for b in range(int(bk.max()) + 1 if bk.size else 0):
+        sel = bk == b
+        if not sel.any():
+            continue
+        fin = sel & np.isfinite(bits)
+        out.append(dict(bucket=bucket_label(b), tokens=int(sel.sum()), zero_width=int((sel & ~np.isfinite(bits)).sum()),
+                        mean_bits=float(bits[fin].mean()) if fin.any() else None, mean_entropy=float(entropy[sel].mean())))
+    return out
+
+
+def summarize(bits, entropy, seg, seg_pos, chunk_pos, payload_lens, n_bytes, max_zw_listed=16):
+    """the summary of analyze()'s per-token arrays (payload_lens: bytes per segment)"""
+    bits, entropy = np.asarray(bits, np.float64), np.asarray(entropy, np.float64)
+    seg = np.asarray(seg, np.int64)
+    fin = np.isfinite(bits)
+    zw = np.nonzero(~fin)[0]
+    n = int(bits.shape[0])
+    pay_bits = 8 * int(sum(int(x) for x in payload_lens))
+    per_byte = lambda x: x / n_bytes if n_bytes else None  # noqa: E731
+    bits_total = float(bits[fin].sum())
+    segments = []
+    for g, plen in enumerate(payload_lens):
+        sel = seg == g
+        sf = sel & fin
+        segments.append(dict(tokens=int(sel.sum()), bits=float(bits[sf].sum()), zero_width=int((sel & ~fin).sum()),
+                             payload_bits=8 * int(plen), entropy=float(entropy[sel].sum())))
+    return dict(tokens=n, bytes=int(n_bytes), bits=bits_total, bits_per_byte=per_byte(bits_total), payload_bits=pay_bits,
+                payload_bits_per_byte=per_byte(pay_bits), mean_bits=float(bits[fin].mean()) if fin.any() else None,
+                mean_entropy=float(entropy.mean()) if n else None, zero_width=int(zw.size), first_zero_width=[int(i) for i in zw[:max_zw_listed]],
+                segments=segments, by_chunk_position=bucket_means(chunk_pos, bits, entropy), by_segment_position=bucket_means(seg_pos, bits, entropy))
+
+
+def analyze(model, data: bytes, tokenizer=None, n_segments=1, bos=0, context=512, reprime_interval=512, pdf_floor=False):
+    """per-token code lengths of `data`, tokenised and split as compress() does.  Returns (arrays, summary): arrays holds, per coded
+    token, ids, bits (its exact code length: 30 - log2 of its interval width, +inf for a zero-width token), entropy (the expected code
+    length of the distribution it was coded from), segment, segment_position, chunk, chunk_position; plus seg_start, first_zw and
+    payload_lens per segment.  pdf_floor codes with the floored SmolLM pdf (as compress(on_zero_width="floor") would)."""
+    tokenizer = tokenizer or ByteTokenizer()
+    ids = tokenize(model, data, tokenizer)
+    r = model.analyze(ids, n_segments=n_segments, bos=bos, context=context, reprime_interval=reprime_interval, pdf_floor=pdf_floor)
+    seg, pos, chunk, cpos = token_positions(r["seg_start"], context, reprime_interval, reprime=model.cfg.get("arch", 0) != 1)
+    payload_lens = np.array([len(p) for p in r["payloads"]], np.int64)
+    arrays = dict(ids=np.asarray(ids, np.uint32), bits=r["bits"], entropy=r["entropy"], segment=seg, segment_position=pos, chunk=chunk,
+                  chunk_position=cpos, seg_start=np.asarray(r["seg_start"], np.uint64), first_zw=r["first_zw"], payload_lens=payload_lens)
+    return arrays, summarize(r["bits"], r["entropy"], seg, pos, cpos, payload_lens, len(data))

@@ -28,6 +28,7 @@ int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size
                     const uint32_t *arg_dev, uint32_t *sym_out_dev, uint32_t *c_lo_dev, uint32_t *c_hi_dev,
                     double *xe_dev, cudaStream_t stream, const int *colmax_dev = nullptr);
 int launch_cdf_full(cz_ctx *ctx, int mode, const float *logits_dev, size_t V, uint32_t *cdf_dev, cudaStream_t stream);
+int launch_cdf_entropy(cz_ctx *ctx, int mode, const float *logits_dev, size_t V, size_t M, size_t ld, double *h_dev, cudaStream_t stream);
 int launch_ac_encode_lanes(cz_ctx *ctx, const uint32_t *c_lo_dev, const uint32_t *c_hi_dev, const uint64_t *lane_off_dev,
                            size_t n_lanes, uint8_t *out_dev, const uint64_t *out_off_dev, uint64_t *out_len_dev,
                            unsigned long long *err_index_dev, cudaStream_t stream, unsigned long long *lane_zw_dev = nullptr);
@@ -216,6 +217,31 @@ int cz_cdf_search(cz_ctx *ctx, const float *logits, size_t vocab, size_t m, size
 int cz_xe_bits_cols(cz_ctx *ctx, const float *logits, size_t vocab, size_t m, size_t ld, int mode, const uint32_t *syms,
                     double *bits_out) {
   return cdf_cols_host(ctx, 2, logits, vocab, m, ld, mode, syms, nullptr, nullptr, nullptr, bits_out);
+}
+// the stats pass of the bounds kernels (every column coded as symbol 0), then the entropy walk over the stats it left
+int cz_cdf_entropy(cz_ctx *ctx, const float *logits, size_t vocab, size_t m, size_t ld, int mode, double *bits_out) {
+  CZ_TRY(require_device(ctx));
+  if (m == 0) return CZ_OK;
+  if (!logits || !bits_out || ld < m) {
+    set_error("cdf: null pointer or ld < m");
+    return CZ_ERR_INVALID;
+  }
+  CZ_CUDA_TRY(cudaSetDevice(ctx->device));
+  const size_t b_log = vocab * ld * sizeof(float), b_u = m * sizeof(uint32_t), b_d = m * sizeof(double);
+  auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
+  CZ_TRY(ensure_scratch(ctx, al(b_log) + 3 * al(b_u) + al(b_d)));
+  char *base = (char *)ctx->scratch;
+  float *d_log = (float *)base;
+  uint32_t *d_sym = (uint32_t *)(base + al(b_log));
+  uint32_t *d_lo = (uint32_t *)((char *)d_sym + al(b_u));
+  uint32_t *d_hi = (uint32_t *)((char *)d_lo + al(b_u));
+  double *d_h = (double *)((char *)d_hi + al(b_u));
+  CZ_CUDA_TRY(cudaMemcpyAsync(d_log, logits, b_log, cudaMemcpyHostToDevice, ctx->stream));
+  CZ_CUDA_TRY(cudaMemsetAsync(d_sym, 0, b_u, ctx->stream));
+  CZ_TRY(launch_cdf_cols(ctx, 0, mode, d_log, vocab, m, ld, d_sym, nullptr, d_lo, d_hi, nullptr, ctx->stream));
+  CZ_TRY(launch_cdf_entropy(ctx, mode, d_log, vocab, m, ld, d_h, ctx->stream));
+  CZ_CUDA_TRY(cudaMemcpyAsync(bits_out, d_h, b_d, cudaMemcpyDeviceToHost, ctx->stream));
+  return fetch_device_status(ctx, nullptr, nullptr);
 }
 int cz_cdf_bounds_dev(cz_ctx *ctx, const float *logits_dev, size_t vocab, size_t m, size_t ld, int mode,
                       const uint32_t *syms_dev, uint32_t *c_lo_dev, uint32_t *c_hi_dev) {

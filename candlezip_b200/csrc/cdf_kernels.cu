@@ -629,6 +629,78 @@ __global__ void __launch_bounds__(128) cdf_xe_final_kernel(const float *__restri
   xe_out[col] = -log2(fmax(pr, 1e-300));
 }
 
+// w (30 - log2 w), one term of H below; 0 for w = 0 (the limit: a zero-width symbol contributes nothing).  For w > 2^29 the factor is below 1 and 30 - log2(w) would lose up to 2^-22 of it to cancellation
+// (w near 2^30: the coded token of a confident model); -log2(1 - d 2^-30) through log1p keeps it to a few ulp (d = 2^30 - w is exact).
+__device__ __forceinline__ double code_len_term(uint32_t w) {
+  const double bits = w > (1u << 29) ? __dmul_rn(-log1p(-(double)(CZ_AC_CDF_TOTAL - w) * 0x1p-30), 1.4426950408889634)  // log2(e)
+                                     : __dsub_rn(30.0, log2(fmax((double)w, 1.0)));  // (w = 0: 0 x 30, not 0 x inf = NaN)
+  return __dmul_rn((double)w, bits);
+}
+
+// Expected code length of every column's coding distribution, from the stats the stats pass left:
+//   H = 2^-30 sum_{s < n, w_s > 0} w_s (30 - log2 w_s),   w_s = cdf[s + 1] - cdf[s]
+// with cdf exactly the coder's (cdf_full_kernel's accumulation, quant, monotone clamp, cdf[n] = 2^30), summed in f64 in ascending s.
+// One thread per column (its own sequential walk: no cross-thread reduction, so H is a pure function of the column), direct coalesced
+// loads of the vocab-major rows.  The rows hold logits (SmolLM) or the e_v the stats pass left in their slots (RWKV alphabet).  The
+// last width is 2^30 - cdf[n - 1], so the last row of the SmolLM alphabets is never read.  A width equal to the previous one reuses its
+// term: in the tail of a real distribution the widths repeat, and log2 is the most expensive operation of the walk.
+template <int MODE>
+__global__ void __launch_bounds__(128) cdf_entropy_kernel(const float *__restrict__ logits, int V, size_t M, size_t ld,
+                                                          const CdfStats *__restrict__ stats, double *__restrict__ h_out) {
+  constexpr bool kLit = MODE == CZ_CDF_RWKV_LITERALS;
+  __shared__ uint64_t s_tab[kLit ? 1 : 32 * 32];
+  if (!kLit) exp_tab64_init(s_tab);
+  const ExpTab64 tab{s_tab + (threadIdx.x & 31)};
+  const size_t col = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (col >= M) return;
+  const CdfStats st = stats[col];
+  PdfOf<MODE, MODE == CZ_CDF_SMOLLM_FLOOR> pdf;
+  pdf.init(st, V);
+  const float mx = st.mx;
+  double acc = 0.0, h = 0.0, term = 0.0;
+  uint32_t prev = 0, last_w = 0;  // (term = code_len_term(0) = 0)
+  auto add = [&](double q) {
+    acc = __dadd_rn(acc, q);
+    uint32_t cur = quant(acc);
+    if (cur < prev) cur = prev;
+    const uint32_t w = cur - prev;
+    prev = cur;
+    if (w != last_w) {
+      last_w = w;
+      term = code_len_term(w);
+    }
+    h = __dadd_rn(h, term);
+  };
+  const int n_rows = kLit ? V : V - 1;
+  auto walk = [&](auto fast_tag) {
+    constexpr bool kFast = decltype(fast_tag)::value;
+    cdf_walk_groups<true>(logits + col, ld, n_rows, [&](int, const float(&x)[CDF_GRP], int cnt) {
+      double d[CDF_GRP];
+      if (kLit) {
+#pragma unroll
+        for (int k = 0; k < CDF_GRP; k++) d[k] = kFast ? cz_widen_pos(x[k]) : (double)x[k];  // (values below 2^-126 are floored either way)
+      } else {
+        float a[CDF_GRP], ef[CDF_GRP];
+#pragma unroll
+        for (int k = 0; k < CDF_GRP; k++) a[k] = __fsub_rn(mx, x[k]);
+        exp_group<CDF_GRP, false>(a, tab, d, ef);
+      }
+#pragma unroll
+      for (int k = 0; k < CDF_GRP; k++)
+        if (k < cnt) add(pdf.template get<kFast>(d[k]));
+    });
+  };
+  if (pdf.fast) walk(std::true_type{});
+  else walk(std::false_type{});
+  if (kLit) {  // literal symbols V .. V + 254 (the last one's width is what is left)
+    const double pl = pdf.literal();
+    for (int j = 0; j < 255; j++) add(pl);
+  }
+  const uint32_t w = CZ_AC_CDF_TOTAL - prev;  // cdf[n] = 2^30
+  h = __dadd_rn(h, code_len_term(w));
+  h_out[col] = __dmul_rn(h, 0x1p-30);
+}
+
 // ---- test hooks: the fast paths of cdf_fast.cuh against the originals -----------------------------------------------------------
 // every non-negative f32 bit pattern b (a = max - logit >= 0, +inf, NaNs): fast == original wherever exp_group takes the fast path,
 // and a checksum of the ORIGINAL expf over the whole domain that the CPU oracle reproduces from glibc-verified code
@@ -1013,6 +1085,20 @@ int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size
       if (op == czk::OP_XE)
         return launch_cdf_encode<MODE, czk::OP_XE>(ctx, logits_dev, V, M, ld, arg_dev, c_lo_dev, c_hi_dev, xe_dev, stream, colmax_dev);
     return launch_cdf_encode<MODE, czk::OP_BOUNDS>(ctx, logits_dev, V, M, ld, arg_dev, c_lo_dev, c_hi_dev, xe_dev, stream, colmax_dev);
+  });
+}
+
+// Expected code length of each column (cdf_entropy_kernel).  Reads the per-column stats in ctx->cdf_stats, so it must follow, on the
+// same stream, the OP_BOUNDS launch_cdf_cols of the same batch in the same mode (which, in the RWKV alphabet, also left e_v in the
+// logits' slots), before anything else overwrites the logits or the stats.
+int launch_cdf_entropy(cz_ctx *ctx, int mode, const float *logits_dev, size_t V, size_t M, size_t ld, double *h_dev, cudaStream_t stream) {
+  return with_cdf_mode(mode, [&](auto mode_c) -> int {
+    if (M == 0) return CZ_OK;
+    const unsigned g = (unsigned)ceil_div(M, 128);
+    CZ_LAUNCH(ctx, CZ_K_CDF, (czk::cdf_entropy_kernel<decltype(mode_c)::value><<<g, 128, 0, stream>>>(
+                                 logits_dev, (int)V, M, ld, (const czk::CdfStats *)ctx->cdf_stats, h_dev)));
+    CZ_CHECK_LAUNCH();
+    return CZ_OK;
   });
 }
 

@@ -18,6 +18,7 @@ namespace cz {
 int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size_t V, size_t M, size_t ld,
                     const uint32_t *arg_dev, uint32_t *sym_out_dev, uint32_t *c_lo_dev, uint32_t *c_hi_dev,
                     double *xe_dev, cudaStream_t stream, const int *colmax_dev = nullptr);
+int launch_cdf_entropy(cz_ctx *ctx, int mode, const float *logits_dev, size_t V, size_t M, size_t ld, double *h_dev, cudaStream_t stream);
 int launch_ac_encode_lanes(cz_ctx *ctx, const uint32_t *c_lo_dev, const uint32_t *c_hi_dev, const uint64_t *lane_off_dev,
                            size_t n_lanes, uint8_t *out_dev, const uint64_t *out_off_dev, uint64_t *out_len_dev,
                            unsigned long long *err_index_dev, cudaStream_t stream, unsigned long long *lane_zw_dev = nullptr);
@@ -26,7 +27,8 @@ int fetch_device_status(cz_ctx *ctx, unsigned long long *err_index_dev, unsigned
 int fetch_device_status_masked(cz_ctx *ctx, unsigned long long *err_index_dev, unsigned long long *err_index_out, int ignore_bits);
 // exec_rwkv.cu
 int rwkv_encode_bounds(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids_host, size_t n_tokens, const cz_schedule *sched,
-                       const uint32_t *extra_dev, const std::vector<size_t> &ev_off, uint32_t *lo_dev, uint32_t *hi_dev, cudaStream_t st);
+                       const uint32_t *extra_dev, const std::vector<size_t> &ev_off, uint32_t *lo_dev, uint32_t *hi_dev, double *ent_dev,
+                       cudaStream_t st);
 int rwkv_xe_bits(cz_model *m, const cz_xe_job *jobs, size_t n_jobs, double *bits_out);
 int rwkv_chunk_logits(cz_model *m, const uint32_t *prime, size_t prime_len, const uint32_t *targets, size_t n_targets, float *logits_out);
 int rwkv_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, size_t n_tokens, const cz_schedule *sched, uint32_t *ids_out);
@@ -343,8 +345,9 @@ static int run_wave_trunk(cz_model *m, const Wave &w, const uint32_t *ids_dev, c
 // LM head + CDF op over the wave's logit columns, in sub-batches of ws.ld_sub columns.
 // syms_dev[j] is the symbol of column j; results go to lo_out/hi_out (OP_BOUNDS) or xe_out (OP_XE), indexed by column.
 // digest_first >= 0: the model has a digest sink and column j is coded token digest_first + j (f-4, digest_kernels.cu).
+// ent_out (OP_BOUNDS): also the expected code length of column j's coding distribution (cdf_entropy_kernel), indexed by column.
 static int run_wave_head(cz_model *m, size_t n_logit, int op, int mode, const uint32_t *syms_dev, uint32_t *lo_out, uint32_t *hi_out,
-                         double *xe_out, cudaStream_t st, long long digest_first = -1) {
+                         double *xe_out, cudaStream_t st, long long digest_first = -1, double *ent_out = nullptr) {
   CZ_TRY(ensure_logits(m, n_logit));
   Workspace &ws = m->ws;
   cz_ctx *ctx = m->ctx;
@@ -381,6 +384,9 @@ static int run_wave_head(cz_model *m, size_t n_logit, int op, int mode, const ui
       rc = launch_cdf_cols(ctx, op, mode, ws.logits[buf], (size_t)m->cfg.vocab, nc, ws.ld_sub, syms_dev + c0, nullptr,
                            lo_out ? lo_out + c0 : nullptr, hi_out ? hi_out + c0 : nullptr, xe_out ? xe_out + c0 : nullptr, cst,
                            have_max ? colmax : nullptr);
+    // (before ev_cdf: the next LM head into this buffer and the next batch's stats pass must not overwrite what it reads)
+    if (rc == CZ_OK && ent_out)
+      rc = launch_cdf_entropy(ctx, mode, ws.logits[buf], (size_t)m->cfg.vocab, nc, ws.ld_sub, ent_out + c0, cst);
     ctx->prof_stream = nullptr;
     CZ_TRY(rc);
     if (overlap) {
@@ -449,8 +455,9 @@ static double host_ms() {
   return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6;
 }
 
+// host_cap: what the caller can take of the payload (cz_encode's cz_bitstreams.cap); checked before the code-length sinks are written.
 static int encode_core(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids_host, size_t n_tokens, const cz_schedule *sched,
-                       uint8_t *out_dev, size_t out_cap, uint64_t *seg_off_host) {
+                       uint8_t *out_dev, size_t out_cap, uint64_t *seg_off_host, size_t host_cap = SIZE_MAX) {
   cz_ctx *ctx = m->ctx;
   cudaStream_t st = ctx->stream;
   static const bool dbg = getenv("CZ_DEBUG_TIMING") != nullptr;
@@ -461,12 +468,21 @@ static int encode_core(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
     set_error("zero-width sink too small: " + std::to_string(m->zw_cap) + " < " + std::to_string(S) + " segments");
     return CZ_ERR_INVALID;
   }
+  if ((m->cl_lo_host || m->cl_hi_host || m->cl_ent_host) && m->cl_cap < n_tokens) {
+    set_error("code-length sink too small: " + std::to_string(m->cl_cap) + " < " + std::to_string(n_tokens) + " tokens");
+    return CZ_ERR_INVALID;
+  }
   static const size_t env_rows = getenv("CZ_WAVE_ROWS") ? (size_t)atoll(getenv("CZ_WAVE_ROWS")) : 0;  // tuning aid
   const size_t max_rows = sched->max_batch_tokens ? sched->max_batch_tokens : (env_rows ? env_rows : (size_t)262144);
   GrowBuf &d_lo = m->sb[SB_LO], &d_hi = m->sb[SB_HI], &d_src = m->sb[SB_SRC], &d_extra = m->sb[SB_EXTRA], &d_lane = m->sb[SB_LANE],
           &d_raw = m->sb[SB_RAW];
   CZ_TRY(d_lo.reserve(n_tokens * 4, st));
   CZ_TRY(d_hi.reserve(n_tokens * 4, st));
+  double *ent_dev = nullptr;
+  if (m->cl_ent_host) {
+    CZ_TRY(m->sb[SB_ENT].reserve(n_tokens * 8 + 16, st));
+    ent_dev = m->sb[SB_ENT].as<double>();
+  }
   CZ_TRY(digest_begin(m, n_tokens, 262144, st));
   // explicit prime token lists of the hint events
   std::vector<uint32_t> extra;
@@ -490,7 +506,8 @@ static int encode_core(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
     CZ_TRY(d_src.reserve(w.n_rows() * 8, st));
     CZ_TRY(run_wave_trunk(m, w, ids_dev, d_extra.as<uint32_t>(), sched->bos, d_src.as<long long>(), st));
     CZ_TRY(run_wave_head(m, w.n_logit(), czk::OP_BOUNDS, coded_mode(m), ids_dev + wave_first, d_lo.as<uint32_t>() + wave_first,
-                         d_hi.as<uint32_t>() + wave_first, nullptr, st, m->digest_host ? (long long)wave_first : -1));
+                         d_hi.as<uint32_t>() + wave_first, nullptr, st, m->digest_host ? (long long)wave_first : -1,
+                         ent_dev ? ent_dev + wave_first : nullptr));
     wave_first += w.n_logit();
     w.clear();
     t_wave0 = host_ms();
@@ -499,7 +516,8 @@ static int encode_core(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
   };
   std::vector<Chunk> chunks;
   if (m->cfg.arch == CZ_ARCH_RWKV7) {
-    CZ_TRY(rwkv_encode_bounds(m, ids_dev, ids_host, n_tokens, sched, d_extra.as<uint32_t>(), ev_off, d_lo.as<uint32_t>(), d_hi.as<uint32_t>(), st));
+    CZ_TRY(rwkv_encode_bounds(m, ids_dev, ids_host, n_tokens, sched, d_extra.as<uint32_t>(), ev_off, d_lo.as<uint32_t>(), d_hi.as<uint32_t>(),
+                              ent_dev, st));
     coded_done = wave_first = n_tokens;
   }
   for (uint32_t g = 0; g < S && m->cfg.arch != CZ_ARCH_RWKV7; g++) {
@@ -568,6 +586,15 @@ static int encode_core(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
   CZ_LAUNCH(ctx, CZ_K_CODER, (czk::compact_payload_kernel<<<S, 128, 0, st>>>(d_raw.as<uint8_t>(), d_raw_off, d_dst_off, out_dev)));
   CZ_CHECK_LAUNCH();
   CZ_TRY(digest_end(m, n_tokens, st));
+  if (seg_off_host[S] > host_cap) {
+    CZ_CUDA_TRY(cudaStreamSynchronize(st));
+    set_error("cz_encode: output capacity " + std::to_string(host_cap) + " < payload " + std::to_string(seg_off_host[S]));
+    return CZ_ERR_NOMEM;
+  }
+  // code-length sinks: the intervals the lanes coded and the entropies the CDF passes left, indexed by global coded index
+  if (n_tokens && m->cl_lo_host) CZ_CUDA_TRY(cudaMemcpyAsync(m->cl_lo_host, d_lo.p, n_tokens * 4, cudaMemcpyDeviceToHost, st));
+  if (n_tokens && m->cl_hi_host) CZ_CUDA_TRY(cudaMemcpyAsync(m->cl_hi_host, d_hi.p, n_tokens * 4, cudaMemcpyDeviceToHost, st));
+  if (n_tokens && ent_dev) CZ_CUDA_TRY(cudaMemcpyAsync(m->cl_ent_host, ent_dev, n_tokens * 8, cudaMemcpyDeviceToHost, st));
   const double t_pre_sync = host_ms();
   CZ_CUDA_TRY(cudaStreamSynchronize(st));
   if (dbg)
@@ -731,12 +758,8 @@ int cz_encode(cz_model *m, const uint32_t *ids, size_t n_tokens, const cz_schedu
   if (n_tokens) CZ_CUDA_TRY(cudaMemcpyAsync(d_ids.p, ids, n_tokens * 4, cudaMemcpyHostToDevice, ctx->stream));
   const size_t cap = 4 * n_tokens + 8 * (size_t)sched->n_segments + 16;
   CZ_TRY(d_out.reserve(cap, ctx->stream));
-  CZ_TRY(encode_core(m, d_ids.as<uint32_t>(), ids, n_tokens, sched, d_out.as<uint8_t>(), cap, out->seg_off));
+  CZ_TRY(encode_core(m, d_ids.as<uint32_t>(), ids, n_tokens, sched, d_out.as<uint8_t>(), cap, out->seg_off, out->cap));
   const uint64_t total = out->seg_off[sched->n_segments];
-  if (total > out->cap) {
-    set_error("cz_encode: output capacity " + std::to_string(out->cap) + " < payload " + std::to_string(total));
-    return CZ_ERR_NOMEM;
-  }
   CZ_CUDA_TRY(cudaMemcpyAsync(out->data, d_out.p, total, cudaMemcpyDeviceToHost, ctx->stream));
   CZ_CUDA_TRY(cudaStreamSynchronize(ctx->stream));
   return CZ_OK;

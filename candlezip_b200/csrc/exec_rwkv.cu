@@ -22,6 +22,7 @@ namespace cz {
 int launch_cdf_cols(cz_ctx *ctx, int op, int mode, const float *logits_dev, size_t V, size_t M, size_t ld,
                     const uint32_t *arg_dev, uint32_t *sym_out_dev, uint32_t *c_lo_dev, uint32_t *c_hi_dev,
                     double *xe_dev, cudaStream_t stream, const int *colmax_dev = nullptr);
+int launch_cdf_entropy(cz_ctx *ctx, int mode, const float *logits_dev, size_t V, size_t M, size_t ld, double *h_dev, cudaStream_t stream);
 int fetch_device_status(cz_ctx *ctx, unsigned long long *err_index_dev, unsigned long long *err_index_out);
 int launch_decode_step(cz_ctx *ctx, int mode, const float *logits, int V, size_t ld, int n_lanes, const uint8_t *payload,
                        const uint64_t *seg_off, const uint64_t *seg_start, uint64_t coded_index, void *decoder_state, uint32_t *ids_out,
@@ -118,6 +119,7 @@ struct RwOut {
   const uint32_t *col_sym = nullptr;  // device, indexed by global column id
   uint32_t *lo = nullptr, *hi = nullptr;
   double *xe = nullptr;
+  double *ent = nullptr;         // OP_BOUNDS: also each column's coding-distribution entropy (cdf_entropy_kernel), by global column id
   float *logits_host = nullptr;  // test hook: [n_cols][V] row-major on the host (single unit)
   bool digest = false;           // f-4: hash every column's logits into the model's digest buffer at its global coded index
 };
@@ -236,11 +238,14 @@ static int rwkv_run_units(cz_model *m, std::vector<RwUnit> &units, const uint32_
       CZ_TRY(launch_cdf_cols(ctx, o.op, CZ_CDF_RWKV_LITERALS, ws.logits[0], V, nc, ws.ld_sub, d_syms.as<uint32_t>() + c0, nullptr,
                              d_lo.as<uint32_t>() + c0, d_hi.as<uint32_t>() + c0, d_xe.as<double>() + c0, st,
                              have_max ? ws.colmax : nullptr));
+      if (o.ent)  // (the per-column results of the encode pass are unused there: d_xe holds the entropies until the scatter)
+        CZ_TRY(launch_cdf_entropy(ctx, CZ_CDF_RWKV_LITERALS, ws.logits[0], V, nc, ws.ld_sub, d_xe.as<double>() + c0, st));
     }
-    if (o.op == czk::OP_XE)
+    if (o.op == czk::OP_XE || o.ent)
       CZ_LAUNCH(ctx, CZ_K_OTHER,
-                (czk::rw_scatter_xe_kernel<<<(unsigned)ceil_div(NL, 256), 256, 0, st>>>(d_xe.as<double>(), d_oidx.as<unsigned long long>(), o.xe, (int)NL)));
-    else
+                (czk::rw_scatter_xe_kernel<<<(unsigned)ceil_div(NL, 256), 256, 0, st>>>(d_xe.as<double>(), d_oidx.as<unsigned long long>(),
+                                                                                       o.op == czk::OP_XE ? o.xe : o.ent, (int)NL)));
+    if (o.op != czk::OP_XE)
       CZ_LAUNCH(ctx, CZ_K_OTHER,
                 (czk::rw_scatter_bounds_kernel<<<(unsigned)ceil_div(NL, 256), 256, 0, st>>>(d_lo.as<uint32_t>(), d_hi.as<uint32_t>(),
                                                                                            d_oidx.as<unsigned long long>(), o.lo, o.hi, (int)NL)));
@@ -251,7 +256,8 @@ static int rwkv_run_units(cz_model *m, std::vector<RwUnit> &units, const uint32_
 
 // ---- encode: fills lo/hi for every coded token (device arrays indexed by global coded index) -------------------------------
 int rwkv_encode_bounds(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids_host, size_t n_tokens, const cz_schedule *sched,
-                       const uint32_t *extra_dev, const std::vector<size_t> &ev_off, uint32_t *lo_dev, uint32_t *hi_dev, cudaStream_t st) {
+                       const uint32_t *extra_dev, const std::vector<size_t> &ev_off, uint32_t *lo_dev, uint32_t *hi_dev, double *ent_dev,
+                       cudaStream_t st) {
   const uint32_t V = (uint32_t)m->cfg.vocab;
   std::vector<uint32_t> host_copy;
   if (!ids_host) {  // device-resident entry point: the host needs the ids to see which symbols are literal escapes
@@ -300,6 +306,7 @@ int rwkv_encode_bounds(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
   o.col_sym = ids_dev;
   o.lo = lo_dev;
   o.hi = hi_dev;
+  o.ent = ent_dev;
   o.digest = m->digest_host != nullptr;  // (encode_core reserved the buffers: digest_begin)
   return rwkv_run_units(m, units, ids_dev, extra_dev, sched->bos, o, sched->max_batch_tokens, st);
 }

@@ -61,7 +61,7 @@ struct GrowBuf {
 };
 enum { SB_LO = 0, SB_HI, SB_SRC, SB_EXTRA, SB_LANE, SB_RAW, SB_IDS, SB_OUT, SB_PAY, SB_OFF, SB_START, SB_STATE, SB_DIDS, SB_K, SB_V,
        SB_LOGITS, SB_KVB, SB_TGT, SB_BITS, SB_JOFF, SB_XOUT, SB_RW_OIDX, SB_RW_SYMS, SB_RW_LO, SB_RW_HI, SB_RW_XE, SB_RW_FRESH,
-       SB_DIGEST, SB_CV,
+       SB_DIGEST, SB_CV, SB_ENT,
        SB_COUNT };
 
 // ---- RWKV-7 (rwkv7.cu) ----
@@ -130,6 +130,10 @@ struct cz_model {
   // cz_model_set_zero_width_out: per-segment first zero-width index of cz_encode / cz_encode_dev (exec.cu, encode_core)
   uint64_t *zw_host = nullptr;
   size_t zw_cap = 0;
+  // cz_model_set_code_length_out: per-token interval and coding-distribution entropy of cz_encode / cz_encode_dev (exec.cu, encode_core)
+  uint32_t *cl_lo_host = nullptr, *cl_hi_host = nullptr;
+  double *cl_ent_host = nullptr;
+  size_t cl_cap = 0;
 };
 
 namespace cz {

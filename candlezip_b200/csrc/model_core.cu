@@ -540,6 +540,19 @@ int cz_model_set_zero_width_out(cz_model *m, uint64_t *first_zw_out, size_t cap_
   m->zw_cap = first_zw_out ? cap_segments : 0;
   return CZ_OK;
 }
+int cz_model_set_code_length_out(cz_model *m, uint32_t *c_lo_out, uint32_t *c_hi_out, double *entropy_out, size_t cap_tokens) {
+  const bool any = c_lo_out || c_hi_out || entropy_out;
+  if (!m) return CZ_ERR_INVALID;
+  if (any && cap_tokens == 0) {
+    set_error("code-length sink: cap_tokens == 0 with a sink set");
+    return CZ_ERR_INVALID;
+  }
+  m->cl_lo_host = c_lo_out;
+  m->cl_hi_host = c_hi_out;
+  m->cl_ent_host = entropy_out;
+  m->cl_cap = any ? cap_tokens : 0;
+  return CZ_OK;
+}
 int cz_model_tensor_count(const cz_model *m) { return m ? (int)m->tensors.size() : 0; }
 int cz_model_tensor_info(const cz_model *m, int idx, const char **name, size_t *n_elems) {
   if (!m || idx < 0 || idx >= (int)m->tensors.size()) return CZ_ERR_INVALID;

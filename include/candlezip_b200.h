@@ -99,6 +99,11 @@ int cz_cdf_full(cz_ctx *ctx, const float *logits, size_t vocab, int mode, uint32
 /* K9: -log2(max(p_floor(sym), 1e-300)) per column (src/main.rs:1745-1747 / 1778-1781) */
 int cz_xe_bits_cols(cz_ctx *ctx, const float *logits, size_t vocab, size_t m, size_t ld, int mode,
                     const uint32_t *syms, double *bits_out);
+/* Expected code length, in bits, of each column's coding distribution in `mode` (0, 1 or 2; else CZ_ERR_INVALID):
+ *   bits_out[m] = 2^-30 * sum_{s < n, w_s > 0} w_s * (30 - log2 w_s),   w_s = cdf[s+1] - cdf[s]
+ * with cdf[0..n] exactly the quantised CDF the coder uses (cz_cdf_full's; n = vocab, or vocab + 256 with CZ_CDF_RWKV_LITERALS),
+ * summed in f64 in ascending s by one thread per column: a pure function of the column, whatever the batch.  Arguments as cz_cdf_bounds. */
+int cz_cdf_entropy(cz_ctx *ctx, const float *logits, size_t vocab, size_t m, size_t ld, int mode, double *bits_out);
 
 /* ---------------------------------------------------------------- K2/K3: arithmetic coder lanes */
 /* Lane l codes the interval list [lane_off[l], lane_off[l+1]) of (c_lo, c_hi) with total 2^30, then finish().
@@ -233,6 +238,17 @@ int cz_model_set_pdf_floor(cz_model *m, int enabled);
  * n_segments makes the call return CZ_ERR_INVALID.  NULL (the default when the model is created) restores failing with
  * CZ_ERR_ZERO_WIDTH; first_zw_out != NULL with cap_segments == 0 is CZ_ERR_INVALID. */
 int cz_model_set_zero_width_out(cz_model *m, uint64_t *first_zw_out, size_t cap_segments);
+
+/* Per-token code lengths.  With a sink set, cz_encode / cz_encode_dev write, for every global coded index i of the call:
+ *   c_lo_out[i], c_hi_out[i]  the interval token i was coded with (c_lo == c_hi for a zero-width token, which only a call with the
+ *                             zero-width sink set can return);  30 - log2(c_hi - c_lo) is its exact code length before coder overhead;
+ *   entropy_out[i]            the expected code length of the distribution token i was coded from (cz_cdf_entropy), in the alphabet the
+ *                             call codes with (cz_model_set_pdf_floor applies).
+ * Any of the three may be NULL; all NULL (the default when the model is created) is off, and then the call launches exactly what it
+ * launches without this function.  The sinks are written only when the call returns CZ_OK.  cap_tokens < the call's n_tokens makes the
+ * call return CZ_ERR_INVALID; a non-NULL pointer with cap_tokens == 0 is CZ_ERR_INVALID.  Both architectures.  cz_decode, cz_xe_bits,
+ * the session shim and cz_chunk_logits are unaffected. */
+int cz_model_set_code_length_out(cz_model *m, uint32_t *c_lo_out, uint32_t *c_hi_out, double *entropy_out, size_t cap_tokens);
 
 typedef struct {
   const uint32_t *prime;     /* tail(history, 511-|hint|) ++ hint, built by the caller or cz_xe_make_prime */
