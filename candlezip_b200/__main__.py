@@ -66,7 +66,7 @@ def _scan_compress(model, tok, data, args):
     prime the main stream; the container carries the AGT2 records; a proof.csv in the reference's format goes to --scan-output-dir."""
     import os
 
-    ids = (tok or codec.ByteTokenizer()).encode_bytes(data)
+    ids = codec.tokenize(model, data, tok or codec.ByteTokenizer())  # RWKV-7: literal escapes for what the vocabulary cannot cover
     texts, calls, decisions, _ = gate.load_replay(args.reuse_scan_dir)
     hint_tok = _hint_tokenizer(tok, model.cfg["vocab"])
     pays, seg, records, rows, events = gate.scan_encode(model, ids, texts, hint_tok, agent_chunk=args.agent_chunk,
@@ -93,13 +93,10 @@ def _scan_decompress(model, tok, blob, args):
     texts, _, _, _ = gate.load_replay(args.reuse_scan_dir)
     hint_tok = _hint_tokenizer(tok, model.cfg["vocab"])
     hints = [[np.asarray(hint_tok(c, 512), np.uint32) for c in gate.build_candidates(texts.get(k + 1, ""))] for k in range(len(records or []))]
-    events = gate.events_from_records(records or [], hints, chunk, n, scan_lookahead=args.scan_lookahead)
+    events = gate.events_from_records(records or [], hints, chunk, n, scan_lookahead=args.scan_lookahead, max_ctx=gate.max_ctx_for(model))
     ids = model.decode(pays, np.array([0, n], np.uint64), bos=int(f["bos_token_id"]), context=int(f["context_window"]),
                        reprime_interval=int(f["reprime_interval"]), events=events or None)
-    data = (tok or codec.ByteTokenizer()).decode_bytes(ids)
-    if container.blake3_16(data) != f["orig_hash16"]:
-        raise ValueError("decoded bytes do not match the container's BLAKE3-128 of the original")
-    return data
+    return codec._finish(model, tok or codec.ByteTokenizer(), f, ids, verify=True)
 
 
 def _main_many(args, ap):
@@ -170,7 +167,7 @@ def main(argv=None):
     ap.add_argument("--on-zero-width", choices=["stored", "floor"],
                     help="compress / self-test: a token the SmolLM coder cannot code stores the input uncoded (stored) or codes it "
                          "again with the floored pdf (floor); default stored")
-    # the agentic gate, replay only (src/main.rs:74-118: --scan, --scan-lookahead, --reuse-scan-dir, gate thresholds); SmolLM backend
+    # the agentic gate, replay only (src/main.rs:74-118: --scan, --scan-lookahead, --reuse-scan-dir, gate thresholds); both backends
     ap.add_argument("--reuse-scan-dir", help="directory with agent_cache.jsonl (+ proof.csv) of a finished run: replay the gate scan")
     ap.add_argument("--scan-lookahead", type=int, default=512)
     ap.add_argument("--agent-chunk", type=int, default=512, help="tokens between gate boundaries (the reference's --scan-chunk-size in tokens)")
@@ -209,8 +206,8 @@ def main(argv=None):
     if args.command == "analyze":
         return _analyze(args)
     scan = bool(args.reuse_scan_dir)
-    if scan and (args.backend != "smollm" or args.segments != 1):
-        ap.error("--reuse-scan-dir works on the SmolLM backend with one AC stream (--segments 1), like the reference's container")
+    if scan and args.segments != 1:
+        ap.error("--reuse-scan-dir works on one AC stream (--segments 1), like the reference's container")
     if scan and args.on_zero_width:
         ap.error("--on-zero-width is not available with --reuse-scan-dir (the gated stream has no fallback of either kind)")
     model, tok = _model(args)

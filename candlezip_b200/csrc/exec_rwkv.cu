@@ -114,6 +114,54 @@ static void build_unit(RwUnit &u, const std::vector<long long> &first_src, const
   }
 }
 
+// rows of one slab when the schedule sets no max_batch_tokens (encode), and the bound on a decode prime slab
+static const size_t kSlabRows = 262144;
+
+// The units of one stream of n coded tokens under the schedule's hint-prime events (n_segments == 1 when there are any): unit u
+// covers coded indices [begin, next unit's begin) and starts from a zero state primed with BOS (event -1) or with the prime of
+// `event`.  Of several events at one index the last wins; an event at an index already passed (out of order) is skipped and one at
+// i >= n never applies.  The encoder and the decoder both plan with this, so they apply the same event at the same index.
+struct RwCut {
+  uint64_t begin;
+  int event;
+};
+static int rwkv_plan_units(const cz_schedule *s, uint64_t n, uint32_t V, std::vector<RwCut> &cuts) {
+  cuts.clear();
+  uint32_t ev = 0;
+  for (uint64_t cur = 0; cur < n;) {
+    int at = -1;
+    for (; ev < s->n_events && s->events[ev].i <= cur; ev++) {
+      const cz_prime_event &e = s->events[ev];
+      if (e.i != cur) continue;
+      bool any = e.hist_take > 0;  // a history tail is never empty: BOS pads it
+      for (uint32_t k = 0; k < e.prime_len && !any; k++) any = e.prime[k] < V;
+      if (!any) {
+        set_error("rwkv: hint prime has no in-vocabulary token");
+        return CZ_ERR_INVALID;
+      }
+      at = (int)ev;
+    }
+    cuts.push_back({cur, at});
+    cur = ev < s->n_events && s->events[ev].i < n ? s->events[ev].i : n;
+  }
+  return CZ_OK;
+}
+
+// Gather codes (rw_gather_tokens_kernel) of the prime of hint event e applied at coded index cur of a stream that starts at a: the
+// last hist_take symbols below V among ids[a, cur) in order, preceded by BOS when there are fewer (S[0] = BOS), then the event's
+// explicit tokens below V, which the caller holds at extra[ev_off ..).  Literal escapes are filtered out (main.rs:2139-2141).
+// ids: the host's copy of at least ids[a, cur).
+static void rwkv_event_prime(const cz_prime_event &e, const uint32_t *ids, uint64_t a, uint64_t cur, uint32_t V, size_t ev_off,
+                             std::vector<long long> &first) {
+  first.clear();
+  for (uint64_t t = cur; t > a && first.size() < e.hist_take; t--)
+    if (ids[t - 1] < V) first.push_back((long long)(t - 1));
+  if (first.size() < e.hist_take) first.push_back(-1ll);
+  std::reverse(first.begin(), first.end());
+  for (uint32_t k = 0; k < e.prime_len; k++)
+    if (e.prime[k] < V) first.push_back(-2 - (long long)(ev_off + k));
+}
+
 struct RwOut {
   int op = czk::OP_BOUNDS;
   const uint32_t *col_sym = nullptr;  // device, indexed by global column id
@@ -132,7 +180,7 @@ static int rwkv_run_units(cz_model *m, std::vector<RwUnit> &units, const uint32_
   if (U == 0) return CZ_OK;
   size_t max_steps = 0;
   for (auto &u : units) max_steps = std::max(max_steps, u.step_src.size());
-  if (max_rows == 0) max_rows = 262144;
+  if (max_rows == 0) max_rows = kSlabRows;
   const size_t Tw = std::max<size_t>(1, std::min(max_steps, max_rows / U));
   CZ_TRY(rwkv_state_reset(m, m->rstate, U, st));
   std::vector<long long> src;
@@ -267,38 +315,18 @@ int rwkv_encode_bounds(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
     ids_host = host_copy.data();
   }
   std::vector<RwUnit> units;
+  std::vector<RwCut> cuts;
+  std::vector<long long> first;
   for (uint32_t g = 0; g < sched->n_segments; g++) {
     const uint64_t a = sched->seg_start[g], b = sched->seg_start[g + 1];
-    if (a == b) continue;
-    uint64_t cur = a;
-    std::vector<long long> first{-1ll};  // BOS (main.rs:1916)
-    uint32_t ev = 0;
-    while (cur < b) {
-      uint64_t end = b;
-      // a gated hint prime at coded index i restarts the state from the prime (main.rs:2137-2149 -> models.rs:162-170)
-      while (ev < sched->n_events && a + sched->events[ev].i < cur) ev++;
-      if (ev < sched->n_events && a + sched->events[ev].i == cur) {
-        first.clear();
-        {  // tail of the in-vocabulary history (literals filtered out, main.rs:2139-2141), then the explicit hint tokens
-          std::vector<long long> hist;
-          const uint64_t want = sched->events[ev].hist_take;
-          for (uint64_t t = cur; t > a && hist.size() < want; t--)
-            if (ids_host[t - 1] < V) hist.push_back((long long)(t - 1));
-          if (hist.size() < want) hist.push_back(-1ll);  // BOS is S[0]
-          first.assign(hist.rbegin(), hist.rend());
-        }
-        for (uint32_t k = 0; k < sched->events[ev].prime_len; k++)
-          if (sched->events[ev].prime[k] < V) first.push_back(-2 - (long long)(ev_off[ev] + k));
-        if (first.empty()) {
-          set_error("rwkv: hint prime has no in-vocabulary token");
-          return CZ_ERR_INVALID;
-        }
-        ev++;
-      }
-      if (ev < sched->n_events && a + sched->events[ev].i < b) end = a + sched->events[ev].i;
+    CZ_TRY(rwkv_plan_units(sched, b - a, V, cuts));
+    for (size_t u = 0; u < cuts.size(); u++) {
+      const uint64_t cur = a + cuts[u].begin, end = u + 1 < cuts.size() ? a + cuts[u + 1].begin : b;
+      // BOS (main.rs:1916), or a gated hint prime, which restarts the state (main.rs:2137-2149 -> models.rs:162-170)
+      if (cuts[u].event < 0) first.assign(1, -1ll);
+      else rwkv_event_prime(sched->events[cuts[u].event], ids_host, a, cur, V, ev_off[cuts[u].event], first);
       units.emplace_back();
       build_unit(units.back(), first, ids_host + cur, (size_t)(end - cur), V, cur, [&](size_t j) { return (long long)(cur + j); });
-      cur = end;
     }
   }
   RwOut o;
@@ -386,7 +414,7 @@ int rwkv_chunk_logits(cz_model *m, const uint32_t *prime, size_t prime_len, cons
   return rwkv_run_units(m, units, nullptr, d_extra.as<uint32_t>(), 0, o, 0, st);
 }
 
-// ---- lock-step batched decode (main.rs:2706-2864 without the agent blocks) ----------------------------------------------------
+// ---- lock-step batched decode (main.rs:2706-2864; gated hint primes as at 2803-2812, rebuilt from the decoded history) ---------
 int rwkv_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, size_t n_tokens, const cz_schedule *sched, uint32_t *ids_out) {
   cz_ctx *ctx = m->ctx;
   cudaStream_t st = ctx->stream;
@@ -410,6 +438,7 @@ int rwkv_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, si
   CZ_TRY(ensure_workspace(m, S, S, 0));
   CZ_TRY(rwkv_ensure_ws(m, S, S));
   CZ_TRY(ensure_logits(m, S));
+  CZ_TRY(digest_begin(m, n_tokens, S, st));
   Workspace &ws = m->ws;
   RwkvWs &rw = m->rws;
   int *d_active = d_meta.as<int>(), *d_cm_keep = d_active + S, *d_sym = d_cm_keep + S;
@@ -438,36 +467,43 @@ int rwkv_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, si
     return CZ_OK;
   };
   // (re)start every stream from a zero state and feed `first` (BOS, or a gated hint prime: main.rs:2803-2812 ->
-  // models.rs:162-170), leaving the logits of its last token in d_keep; then restore the single-row step metadata
+  // models.rs:162-170), leaving the logits of its last token in d_keep; then restore the single-row step metadata.  A long prime
+  // goes in slabs of at most max_rows rows (the encoder's bound), the state carried from slab to slab, so the workspace does not
+  // grow with the history; any split gives the same logits bit for bit (DESIGN §3).
+  const size_t max_rows = sched->max_batch_tokens ? sched->max_batch_tokens : kSlabRows, Tw = std::max<size_t>(1, max_rows / S);
   auto prime_all = [&](const std::vector<uint32_t> &first) -> int {
-    const size_t n = first.size(), R = (size_t)S * n;
-    CZ_TRY(ensure_workspace(m, R, S, 0));
-    CZ_TRY(rwkv_ensure_ws(m, R, S));
-    std::vector<uint32_t> tok(R);
-    std::vector<int> prev(R), slot(R), flags(R, 0), rb(S), re(S), lrows(S);
-    for (uint32_t g = 0; g < S; g++) {
-      for (size_t k = 0; k < n; k++) {
-        const size_t r = (size_t)g * n + k;
-        tok[r] = first[k];
-        prev[r] = k == 0 ? -1 : (int)r - 1;
-        slot[r] = (int)g;
-      }
-      flags[(size_t)g * n + n - 1] = 1;
-      rb[g] = (int)(g * n);
-      re[g] = (int)(g * n + n);
-      lrows[g] = (int)(g * n + n - 1);
-    }
-    CZ_CUDA_TRY(cudaMemcpyAsync(ws.tok, tok.data(), R * 4, cudaMemcpyHostToDevice, st));
-    CZ_CUDA_TRY(cudaMemcpyAsync(rw.prev_row, prev.data(), R * 4, cudaMemcpyHostToDevice, st));
-    CZ_CUDA_TRY(cudaMemcpyAsync(rw.slot, slot.data(), R * 4, cudaMemcpyHostToDevice, st));
-    CZ_CUDA_TRY(cudaMemcpyAsync(rw.flags, flags.data(), R * 4, cudaMemcpyHostToDevice, st));
-    CZ_CUDA_TRY(cudaMemcpyAsync(rw.row_begin, rb.data(), S * 4, cudaMemcpyHostToDevice, st));
-    CZ_CUDA_TRY(cudaMemcpyAsync(rw.row_end, re.data(), S * 4, cudaMemcpyHostToDevice, st));
-    CZ_CUDA_TRY(cudaMemcpyAsync(rw.stream_slot, iota.data(), S * 4, cudaMemcpyHostToDevice, st));
-    CZ_CUDA_TRY(cudaMemcpyAsync(ws.logit_rows, lrows.data(), S * 4, cudaMemcpyHostToDevice, st));
+    const size_t n = first.size();
     CZ_CUDA_TRY(cudaMemcpyAsync(d_active, ones.data(), S * 4, cudaMemcpyHostToDevice, st));
     CZ_TRY(rwkv_state_reset(m, m->rstate, S, st));
-    CZ_TRY(rwkv_forward(m, (int)R, (int)S, m->rstate, /*in_place=*/n == 1, nullptr, st));
+    for (size_t k0 = 0; k0 < n; k0 += Tw) {
+      const size_t T = std::min(Tw, n - k0), R = (size_t)S * T;
+      CZ_TRY(ensure_workspace(m, R, S, 0));
+      CZ_TRY(rwkv_ensure_ws(m, R, S));
+      std::vector<uint32_t> tok(R);
+      std::vector<int> prev(R), slot(R), flags(R, 0), rb(S), re(S), lrows(S);
+      for (uint32_t g = 0; g < S; g++) {
+        for (size_t k = 0; k < T; k++) {
+          const size_t r = (size_t)g * T + k;
+          tok[r] = first[k0 + k];
+          prev[r] = k == 0 ? -1 : (int)r - 1;
+          slot[r] = (int)g;
+        }
+        flags[(size_t)g * T + T - 1] = 1;
+        rb[g] = (int)(g * T);
+        re[g] = (int)(g * T + T);
+        lrows[g] = (int)(g * T + T - 1);
+      }
+      CZ_CUDA_TRY(cudaMemcpyAsync(ws.tok, tok.data(), R * 4, cudaMemcpyHostToDevice, st));
+      CZ_CUDA_TRY(cudaMemcpyAsync(rw.prev_row, prev.data(), R * 4, cudaMemcpyHostToDevice, st));
+      CZ_CUDA_TRY(cudaMemcpyAsync(rw.slot, slot.data(), R * 4, cudaMemcpyHostToDevice, st));
+      CZ_CUDA_TRY(cudaMemcpyAsync(rw.flags, flags.data(), R * 4, cudaMemcpyHostToDevice, st));
+      CZ_CUDA_TRY(cudaMemcpyAsync(rw.row_begin, rb.data(), S * 4, cudaMemcpyHostToDevice, st));
+      CZ_CUDA_TRY(cudaMemcpyAsync(rw.row_end, re.data(), S * 4, cudaMemcpyHostToDevice, st));
+      CZ_CUDA_TRY(cudaMemcpyAsync(rw.stream_slot, iota.data(), S * 4, cudaMemcpyHostToDevice, st));
+      CZ_CUDA_TRY(cudaMemcpyAsync(ws.logit_rows, lrows.data(), S * 4, cudaMemcpyHostToDevice, st));
+      CZ_TRY(rwkv_forward(m, (int)R, (int)S, m->rstate, /*in_place=*/n == 1, nullptr, st));
+      if (k0 + T < n) CZ_CUDA_TRY(cudaStreamSynchronize(st));  // the staging vectors are stack-owned
+    }
     CZ_TRY(head_commit());
     // single-row step metadata: row s = stream s, state slot s
     CZ_CUDA_TRY(cudaMemcpyAsync(rw.prev_row, minus1.data(), S * 4, cudaMemcpyHostToDevice, st));
@@ -480,6 +516,11 @@ int rwkv_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, si
     return CZ_OK;
   };
   auto decode_syms = [&]() -> int {
+    // f-4: digest of the logits column each live stream is about to decode from, at index seg_start[g] + ctr[0].  A stream that
+    // decoded a literal escape did not step, so its kept column is the one the encoder coded the next symbol from.
+    if (m->digest_host)
+      CZ_TRY(launch_logits_digest(ctx, d_keep.as<float>(), V, S, S_pad, m->sb[SB_CV].p, m->sb[SB_DIGEST].as<uint8_t>(), 0, nullptr,
+                                  d_start.as<uint64_t>(), d_ctr, st));
     return launch_decode_step(ctx, CZ_CDF_RWKV_LITERALS, d_keep.as<float>(), (int)V, S_pad, (int)S, d_pay.as<uint8_t>(), d_off.as<uint64_t>(),
                               d_start.as<uint64_t>(), 0, d_state.p, d_ids.as<uint32_t>(), (uint32_t *)d_sym, use_cm ? d_cm_keep : nullptr, st,
                               d_ctr);
@@ -498,31 +539,38 @@ int rwkv_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, si
     CZ_TRY(launch_advance_ctr(ctx, d_ctr, st));
     return CZ_OK;
   };
-  for (uint32_t e = 0; e < sched->n_events; e++)
-    if (sched->events[e].hist_take) {
-      set_error("rwkv decode: hint primes with a history tail (hist_take > 0) need the decoded tokens on the host; pass explicit primes");
-      return CZ_ERR_UNSUPPORTED;
-    }
-  // units: [0, e_0), [e_0, e_1), ... ; each starts from a fresh state primed with BOS / the event's prime (events: S == 1)
-  std::vector<uint64_t> cut{0};
-  for (uint32_t e = 0; e < sched->n_events; e++)
-    if (sched->events[e].i > cut.back() && sched->events[e].i < max_len) cut.push_back(sched->events[e].i);
-  cut.push_back(max_len);
-  for (size_t u = 0; u + 1 < cut.size(); u++) {
-    std::vector<uint32_t> first{sched->bos};
-    for (uint32_t e = 0; e < sched->n_events; e++)
-      if (sched->events[e].i == cut[u] && (u > 0 || cut[u] == 0) && sched->events[e].i == cut[u]) {
-        std::vector<uint32_t> pr;
-        for (uint32_t k = 0; k < sched->events[e].prime_len; k++)
-          if (sched->events[e].prime[k] < V) pr.push_back(sched->events[e].prime[k]);
-        if (!pr.empty()) first = pr;
+  // units as the encoder plans them; each starts from a fresh state primed with BOS / the event's prime (events: S == 1)
+  std::vector<RwCut> cut;
+  CZ_TRY(rwkv_plan_units(sched, max_len, (uint32_t)V, cut));
+  std::vector<uint32_t> extra, ids_host, first;  // explicit prime tokens of the events; decoded ids [0, n_host) of the one stream
+  std::vector<size_t> ev_off(sched->n_events + 1, 0);
+  for (uint32_t e = 0; e < sched->n_events; e++) {
+    ev_off[e] = extra.size();
+    extra.insert(extra.end(), sched->events[e].prime, sched->events[e].prime + sched->events[e].prime_len);
+  }
+  std::vector<long long> src;
+  uint64_t n_host = 0;
+  for (size_t u = 0; u < cut.size(); u++) {
+    const uint64_t c0 = cut[u].begin, c1 = u + 1 < cut.size() ? cut[u + 1].begin : max_len;
+    first.assign(1, sched->bos);
+    if (cut[u].event >= 0) {
+      const cz_prime_event &ev = sched->events[cut[u].event];
+      if (ev.hist_take && n_host < c0) {  // the history tail needs what has been decoded so far on the host: one copy per event
+        ids_host.resize(c0);
+        CZ_CUDA_TRY(cudaMemcpyAsync(ids_host.data() + n_host, d_ids.as<uint32_t>() + n_host, (c0 - n_host) * 4, cudaMemcpyDeviceToHost, st));
+        CZ_CUDA_TRY(cudaStreamSynchronize(st));
+        n_host = c0;
       }
+      rwkv_event_prime(ev, ids_host.data(), 0, c0, (uint32_t)V, ev_off[cut[u].event], src);
+      first.resize(src.size());
+      for (size_t k = 0; k < src.size(); k++) first[k] = src[k] >= 0 ? ids_host[src[k]] : (src[k] == -1 ? sched->bos : extra[-2 - src[k]]);
+    }
     CZ_TRY(prime_all(first));
-    CZ_TRY(launch_set_ctr(ctx, d_ctr, cut[u], 0, st));
+    CZ_TRY(launch_set_ctr(ctx, d_ctr, c0, 0, st));
     cudaGraphExec_t gexec = nullptr;
     uint64_t nodes = 0;
     int rc = CZ_OK;
-    const uint64_t n_steps = cut[u + 1] - cut[u] - (u + 2 == cut.size() ? 1 : 0);  // the very last symbol needs no step after it
+    const uint64_t n_steps = c1 - c0 - (u + 1 == cut.size() ? 1 : 0);  // the very last symbol needs no step after it
     for (uint64_t i = 0; i < n_steps && rc == CZ_OK; i++) {
       if (i == 0 || !use_graph || n_steps < 4) {
         rc = step();
@@ -559,6 +607,7 @@ int rwkv_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, si
   CZ_TRY(decode_syms());  // every stream's last symbol
   CZ_TRY(fetch_device_status(ctx, nullptr, nullptr));
   CZ_CUDA_TRY(cudaMemcpyAsync(ids_out, d_ids.p, n_tokens * 4, cudaMemcpyDeviceToHost, st));
+  CZ_TRY(digest_end(m, n_tokens, st));
   CZ_CUDA_TRY(cudaStreamSynchronize(st));
   return CZ_OK;
 }

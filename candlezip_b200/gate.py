@@ -7,7 +7,7 @@ texts are an input (replayed from `agent_cache.jsonl`, src/main.rs:1152-1195, or
   -------------------------------------------------------------  ------------------------------------------------------------
   candidates = [normalized, first 2000 bytes, digit lines,       build_candidates()
                 Capitalised words]            (main.rs:2018-2032)
-  budgets = [max_ctx/8, /4, /2, 3/4]          (main.rs:2034-2035)  BUDGETS (max_ctx = 511 for SmolLM)
+  budgets = [max_ctx/8, /4, /2, 3/4]          (main.rs:2034-2035)  budgets(max_ctx): 511 for SmolLM, the whole history for RWKV-7
   baseline XE + up to 16 conditioned XE passes (2043-2054)       ONE cz_xe_bits call for ALL boundaries: every (boundary,
                                                                   candidate, budget) is an independent paired stream
   best = argmax saved; gate = saved > 0 (+ thresholds) (2068-72)  same selection order (first maximum wins)
@@ -18,7 +18,17 @@ texts are an input (replayed from `agent_cache.jsonl`, src/main.rs:1152-1195, or
 """
 import numpy as np
 
+from . import _lib
+
 MAX_CTX_SMOLLM = 511  # max_context_length() - 1, src/models.rs:91, main.rs:2034
+# RWKV-7's max_context_length() is usize::MAX (src/models.rs:150): every budget covers the whole hint, every history tail the whole
+# history (BOS first), so a gated prime re-feeds everything before the boundary (models.rs:162-170)
+MAX_CTX_RWKV7 = (1 << 64) - 1
+
+
+def max_ctx_for(model):
+    """the gate's max_ctx for a model: SmolLM's 511, or the whole history on RWKV-7"""
+    return MAX_CTX_RWKV7 if model.cfg.get("arch", _lib.CZ_ARCH_SMOLLM) == _lib.CZ_ARCH_RWKV7 else MAX_CTX_SMOLLM
 
 
 def build_candidates(agent_text: str):
@@ -36,14 +46,18 @@ def budgets(max_ctx=MAX_CTX_SMOLLM):
 
 
 def plan_scan(ids, agent_texts, tokenize_hint, agent_chunk, scan_lookahead=512, scan_max_hint_tokens=512, bos=0,
-              max_ctx=MAX_CTX_SMOLLM):
+              max_ctx=MAX_CTX_SMOLLM, share_jobs=None):
     """Builds the XE jobs of every boundary.  ids: coded tokens (no BOS).  agent_texts: {chunk_index: text} (1-based chunk
-    index = boundary / agent_chunk, main.rs:1985).  Returns (jobs, plan) with plan[k] = dict(i, chunk_index, job0, hints)
-    where jobs[job0] is the baseline and jobs[job0 + 1 + cid*4 + bid] the conditioned stream (or None when it equals the
-    baseline: empty hint, main.rs:2050)."""
+    index = boundary / agent_chunk, main.rs:1985).  Returns (jobs, plan) with plan[k] = dict(i, chunk_index, job0, hints, slots)
+    where jobs[job0] is the baseline and jobs[slots[cid*4 + bid]] the conditioned stream (slot None when it equals the
+    baseline: empty hint, main.rs:2050).
+    share_jobs: conditioned jobs of a boundary with the same prime share one stream (several slots name the same job).  The
+    default shares under the whole-history rule (max_ctx = MAX_CTX_RWKV7), where the four budgets of a candidate always give the
+    same prime; with SmolLM's 511 every slot keeps a stream of its own, one per XE pass of the reference."""
     seq = np.concatenate([[bos], np.asarray(ids, np.uint32)]).astype(np.uint32)  # the reference's `ids` (BOS first)
     n = len(seq) - 1
     bud = budgets(max_ctx)
+    share = max_ctx == MAX_CTX_RWKV7 if share_jobs is None else bool(share_jobs)
     jobs, plan = [], []
     boundary = agent_chunk
     for i in range(n):
@@ -60,14 +74,19 @@ def plan_scan(ids, agent_texts, tokenize_hint, agent_chunk, scan_lookahead=512, 
         hints = [np.asarray(tokenize_hint(c, scan_max_hint_tokens), np.uint32) for c in cands]
         entry = dict(i=i, chunk_index=chunk_index, job0=len(jobs), hints=hints, slots=[])
         jobs.append((xe_prime(hist, None, max_ctx), targets))
+        seen = {}  # prime bytes -> job index (same boundary, so the same targets)
         for cid in range(4):
             for bid in range(4):
                 h = hints[cid][: bud[bid]]
                 if len(h) == 0:
                     entry["slots"].append(None)
-                else:
-                    entry["slots"].append(len(jobs))
-                    jobs.append((xe_prime(hist, h, max_ctx), targets))
+                    continue
+                prime = xe_prime(hist, h, max_ctx)
+                key = prime.tobytes()
+                if not share or key not in seen:
+                    seen[key] = len(jobs)
+                    jobs.append((prime, targets))
+                entry["slots"].append(seen[key])
         plan.append(entry)
     return jobs, plan
 
@@ -132,15 +151,17 @@ def events_from_records(records, hints_by_boundary, agent_chunk, n_tokens, scan_
     return events
 
 
-def scan_encode(model, ids, agent_texts, tokenize_hint, agent_chunk, n_segments=1, **kw):
+def scan_encode(model, ids, agent_texts, tokenize_hint, agent_chunk, n_segments=1, max_ctx=None, **kw):
     """compress with the agentic gate: one batched XE scan, then one batched encode with the gated hint primes.
-    Returns (payloads, seg_start, records, rows, events)."""
+    max_ctx: default max_ctx_for(model).  Returns (payloads, seg_start, records, rows, events)."""
     if n_segments != 1:
         raise ValueError("the gate works on a single AC stream (the reference's container has one)")
+    max_ctx = max_ctx_for(model) if max_ctx is None else max_ctx
     look = kw.get("scan_lookahead", 512)
-    jobs, plan = plan_scan(ids, agent_texts, tokenize_hint, agent_chunk, look, kw.get("scan_max_hint_tokens", 512), kw.get("bos", 0))
+    jobs, plan = plan_scan(ids, agent_texts, tokenize_hint, agent_chunk, look, kw.get("scan_max_hint_tokens", 512), kw.get("bos", 0),
+                           max_ctx=max_ctx)
     bits = model.xe_bits(jobs) if jobs else np.zeros(0)
-    records, events, rows = decide(plan, bits, look, kw.get("thr_abs_bits", 0.0), kw.get("thr_pct", 0.0))
+    records, events, rows = decide(plan, bits, look, kw.get("thr_abs_bits", 0.0), kw.get("thr_pct", 0.0), max_ctx=max_ctx)
     pays, seg = model.encode(ids, n_segments=1, bos=kw.get("bos", 0), events=events or None)
     return pays, seg, records, rows, events
 

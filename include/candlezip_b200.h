@@ -178,7 +178,8 @@ typedef struct {
   uint64_t hold_until;       /* src/main.rs:2149 */
   uint32_t hist_take;        /* tokens taken from the stream itself before `prime`: tail(ids[..=i], hist_take) with ids[0] = BOS
                                 (src/main.rs:2132-2134, 2596-2600).  The decoder rebuilds this part from what it has decoded, so a
-                                gated stream decodes in one call.  0: `prime` is the whole prime (SmolLM only when > 0). */
+                                gated stream decodes in one call.  0: `prime` is the whole prime.  RWKV-7: the last hist_take
+                                symbols below vocab before index i (literal escapes skipped), BOS first when there are fewer. */
 } cz_prime_event;
 
 typedef struct {
@@ -207,7 +208,11 @@ int cz_encode(cz_model *m, const uint32_t *ids, size_t n_tokens, const cz_schedu
  * the remainder on the first segments) so that the live streams are always a prefix of the batch; otherwise CZ_ERR_UNSUPPORTED.
  * Memory: the KV arenas are allocated up front, 2 * n_layers * n_segments * max_pos * n_kv_heads * 64 bf16 elements with
  * max_pos = 1024 at --context 512 / --reprime-interval 512 (SmolLM-135M: 23.6 MB per segment, 48 GB at 2048 segments);
- * CZ_ERR_CUDA (out of memory) if that does not fit. */
+ * CZ_ERR_CUDA (out of memory) if that does not fit.
+ * Hint-prime events (n_segments == 1) are applied at the same coded index as cz_encode applies them, on both backends; an event's
+ * history tail (hist_take) is rebuilt from the symbols decoded so far.  RWKV-7 feeds a prime in slabs of at most max_batch_tokens
+ * rows (262,144 when 0), so its memory does not grow with the history; an event whose prime has no in-vocabulary token is
+ * CZ_ERR_INVALID, as in cz_encode. */
 int cz_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, size_t n_tokens,
               const cz_schedule *sched, uint32_t *ids_out);
 /* device-resident variant of the encode step used by bench.py for the kernel-only number: ids already in HBM (an id outside
@@ -219,7 +224,8 @@ int cz_encode_dev(cz_model *m, const uint32_t *ids_dev, size_t n_tokens, const c
  * `pdf_digest` per encode / decode step, :2328-2342, :2629-2647).  With a sink set, cz_encode / cz_encode_dev / cz_decode hash
  * every coded token's logits vector (the V f32 values, little-endian) ON THE DEVICE next to the CDF pass and copy the 16-byte
  * BLAKE3-128 digests to digests_out[i * 16 .. i * 16 + 16), i = global coded index.  Encode and decode digests of a stream are
- * equal byte for byte (decode safety), whatever the wave size, batch size or GPU count.  NULL disables.  (RWKV-7: encode only.) */
+ * equal byte for byte (decode safety), whatever the wave size, batch size or GPU count.  NULL disables.  Both backends; on RWKV-7 a
+ * literal-escape symbol does not step the model, so its digest is that of the logits the previous symbol was coded from. */
 int cz_model_set_digest_out(cz_model *m, uint8_t *digests_out, size_t cap_tokens);
 
 /* enabled != 0: cz_encode / cz_encode_dev / cz_decode code SmolLM streams with CZ_CDF_SMOLLM_FLOOR instead of CZ_CDF_SMOLLM, so no
