@@ -11,6 +11,8 @@ compress-many / decompress-many IN... [--out-dir DIR]: many files through one en
 analyze INPUT [OUTPUT]: per-token code lengths, coding-distribution entropies and positions (codec.analyze), tokenised and split as
 `compress` does, into OUTPUT (default INPUT.analysis.npz: the arrays, plus the summary as JSON under "summary"); prints the summary.
 --pdf-floor (analyze, SmolLM only) codes with the floored pdf.
+--dictionary FILE (every command but the gate replay): code each segment as if it followed FILE's contents (a preset dictionary, never
+stored in the container); decompress needs the same FILE.
 """
 import argparse
 import json
@@ -112,9 +114,9 @@ def _main_many(args, ap):
     t0 = time.perf_counter()
     if args.command == "compress-many":
         res = codec.compress_many(model, datas, tok, args.segments, context=args.context, reprime_interval=args.reprime_interval,
-                                  on_zero_width=args.on_zero_width or "stored")
+                                  on_zero_width=args.on_zero_width or "stored", dictionary=args.dictionary_bytes)
     else:
-        res = codec.decompress_many(model, datas, tok, max_streams=args.max_streams)
+        res = codec.decompress_many(model, datas, tok, max_streams=args.max_streams, dictionary=args.dictionary_bytes)
     dt = time.perf_counter() - t0
     if args.out_dir:
         os.makedirs(args.out_dir, exist_ok=True)
@@ -143,7 +145,7 @@ def _analyze(args):
     model, tok = _model(args)
     data = open(args.input, "rb").read()
     arrays, summary = codec.analyze(model, data, tok, args.segments, context=args.context, reprime_interval=args.reprime_interval,
-                                    pdf_floor=args.pdf_floor)
+                                    pdf_floor=args.pdf_floor, dictionary=args.dictionary_bytes)
     out = args.output or args.input + ".analysis.npz"
     with open(out, "wb") as f:  # (a file object: np.savez would append .npz to a name without it)
         np.savez(f, summary=np.array(json.dumps(summary)), **arrays)
@@ -177,7 +179,11 @@ def main(argv=None):
     ap.add_argument("--out-dir", help="compress-many / decompress-many: where NAME.canz / NAME.out go (default: beside each input)")
     ap.add_argument("--max-streams", type=int, help="decompress-many: most segments decoded together in one lock-step wave; default 2048")
     ap.add_argument("--pdf-floor", action="store_true", help="analyze: code with the floored SmolLM pdf (no token is zero-width)")
+    ap.add_argument("--dictionary", metavar="FILE", help="preset dictionary: code every segment as if it followed FILE's contents; "
+                                                         "decompressing needs the same FILE")
     args = ap.parse_args(argv)
+    if args.dictionary and args.reuse_scan_dir:
+        ap.error("--dictionary is not available with --reuse-scan-dir (gated hint primes and a dictionary do not combine)")
     # flags that only one side uses are refused on the other instead of being ignored
     if args.command == "decompress-many" and (args.segments is not None or args.on_zero_width):
         ap.error("--segments and --on-zero-width are compress settings: a container carries its own (decompress-many)")
@@ -192,6 +198,10 @@ def main(argv=None):
                 ap.error(f"{flag} is not available with analyze")
     if args.segments is None:
         args.segments = 1
+    args.dictionary_bytes = None
+    if args.dictionary:
+        with open(args.dictionary, "rb") as f:
+            args.dictionary_bytes = f.read()
     if args.command.endswith("-many"):
         if args.reuse_scan_dir:
             ap.error("--reuse-scan-dir codes one file at a time: not available with compress-many / decompress-many")
@@ -215,20 +225,20 @@ def main(argv=None):
     if args.command == "compress":
         blob = _scan_compress(model, tok, data, args) if scan else \
             codec.compress(model, data, tok, args.segments, context=args.context, reprime_interval=args.reprime_interval,
-                           on_zero_width=args.on_zero_width or "stored")
+                           on_zero_width=args.on_zero_width or "stored", dictionary=args.dictionary_bytes)
         open(args.output or args.input + ".canz", "wb").write(blob)
         print(f"{len(data)} -> {len(blob)} bytes ({8 * len(blob) / max(1, len(data)):.4f} bits/byte)")
     elif args.command == "decompress":
-        out = _scan_decompress(model, tok, data, args) if scan else codec.decompress(model, data, tok)
+        out = _scan_decompress(model, tok, data, args) if scan else codec.decompress(model, data, tok, dictionary=args.dictionary_bytes)
         open(args.output or args.input + ".out", "wb").write(out)
         print(f"{len(data)} -> {len(out)} bytes")
     else:  # self-test: encode + decode round trip with timings (src/main.rs:156-221)
         t0 = time.perf_counter()
         blob = _scan_compress(model, tok, data, args) if scan else \
             codec.compress(model, data, tok, args.segments, context=args.context, reprime_interval=args.reprime_interval,
-                           on_zero_width=args.on_zero_width or "stored")
+                           on_zero_width=args.on_zero_width or "stored", dictionary=args.dictionary_bytes)
         t1 = time.perf_counter()
-        out = _scan_decompress(model, tok, blob, args) if scan else codec.decompress(model, blob, tok)
+        out = _scan_decompress(model, tok, blob, args) if scan else codec.decompress(model, blob, tok, dictionary=args.dictionary_bytes)
         t2 = time.perf_counter()
         ok = out == data
         print(f"Compression: {t1 - t0:.3f} s  Decompression: {t2 - t1:.3f} s  {8 * len(blob) / max(1, len(data)):.4f} bits/byte  "

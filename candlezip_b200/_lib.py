@@ -29,6 +29,7 @@ CZ_ENGINE_TCGEN05, CZ_ENGINE_SIMT = 0, 1
 CZ_FLAG_SEGMENTS = 1 << 8
 CZ_FLAG_STORED = 1 << 9
 CZ_FLAG_PDF_FLOOR = 1 << 10
+CZ_FLAG_DICTIONARY = 1 << 11
 NO_ZERO_WIDTH = 2 ** 64 - 1  # cz_model_set_zero_width_out: the segment has no zero-width token
 K_FAMILIES = ("gemm_qkv", "attn", "elemwise", "cdf", "coder", "other", "gemm_o", "gemm_gu", "gemm_down", "gemm_head", "cdf_prefix")
 
@@ -131,6 +132,7 @@ SIGNATURES = {
     "cz_model_set_pdf_floor": (C.c_int, [_vp, C.c_int]),
     "cz_model_set_zero_width_out": (C.c_int, [_vp, u64p, C.c_size_t]),
     "cz_model_set_code_length_out": (C.c_int, [_vp, u32p, u32p, f64p, C.c_size_t]),
+    "cz_model_set_dictionary": (C.c_int, [_vp, u32p, C.c_size_t]),
     "cz_xe_bits": (C.c_int, [_vp, C.POINTER(XeJob), C.c_size_t, f64p]),
     "cz_chunk_logits": (C.c_int, [_vp, u32p, C.c_size_t, u32p, C.c_size_t, f32p]),
     "cz_container_header_size": (C.c_size_t, [C.POINTER(HeaderV2)]),
@@ -140,6 +142,8 @@ SIGNATURES = {
     "cz_container_read_gates": (C.c_size_t, [u8p, C.c_size_t, u8p, C.c_size_t, szp]),
     "cz_container_write_segments": (C.c_size_t, [u8p, C.c_size_t, C.c_int, u64p, u64p, C.c_size_t]),
     "cz_container_read_segments": (C.c_size_t, [u8p, C.c_size_t, C.POINTER(C.c_int), u64p, u64p, C.c_size_t, szp]),
+    "cz_container_write_dictionary": (C.c_size_t, [u8p, C.c_size_t, C.c_uint64, u8p]),
+    "cz_container_read_dictionary": (C.c_size_t, [u8p, C.c_size_t, u64p, u8p]),
     "cz_flags_pack": (C.c_uint32, [C.c_int, C.c_int, C.c_int, C.c_uint32]),
     "cz_blake3_16": (None, [u8p, C.c_size_t, u8p]),
     "cz_test_gemm": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_uint16), C.POINTER(C.c_uint16), C.c_int, C.c_int, _vp,
@@ -153,6 +157,7 @@ SIGNATURES = {
     "cz_test_div_random": (C.c_int, [_vp, C.c_uint64, C.c_uint64, u64p]),
     "cz_test_cdf_ecache_state": (C.c_int, [_vp, C.POINTER(C.c_int), u64p]),
     "cz_schedule_chunks": (C.c_size_t, [C.c_uint64, C.c_uint32, C.c_uint32, u64p, u32p, u64p, u32p, C.c_size_t]),
+    "cz_schedule_chunks_prefixed": (C.c_size_t, [C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, u64p, u32p, u64p, u32p, C.c_size_t]),
 }
 
 

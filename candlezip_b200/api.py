@@ -265,13 +265,33 @@ class Model:
         """code SmolLM streams with the floored pdf (CZ_CDF_SMOLLM_FLOOR) in the following encode / decode calls; RWKV-7 refuses"""
         check(lib.cz_model_set_pdf_floor(self._h, 1 if enabled else 0))
 
+    def set_dictionary(self, symbols):
+        """code every segment of the following encode / decode calls as if it followed `symbols` (cz_model_set_dictionary); None or an
+        empty list clears it"""
+        if symbols is None or len(symbols) == 0:
+            check(lib.cz_model_set_dictionary(self._h, None, 0))
+            return
+        a, p = _u32(symbols)
+        check(lib.cz_model_set_dictionary(self._h, p, a.shape[0]))
+
+    def _with_dictionary(self, dictionary, call):
+        """call() with the dictionary set, cleared again afterwards (no dictionary: nothing is set)"""
+        if dictionary is None:
+            return call()
+        self.set_dictionary(dictionary)
+        try:
+            return call()
+        finally:
+            self.set_dictionary(None)
+
     def encode(self, ids, n_segments=1, bos=0, context=512, reprime_interval=512, events=None, seg_start=None, max_batch_tokens=0,
-               pdf_floor=False, zero_width_out=False):
+               pdf_floor=False, zero_width_out=False, dictionary=None):
         """ids: coded tokens (no BOS). Returns (list of per-segment payload bytes, seg_start).
         pdf_floor: code with softmax_pdf_floor (no token is zero-width); the stream must be decoded with pdf_floor=True too.
         zero_width_out: a zero-width token does not raise CZ_ERR_ZERO_WIDTH; returns (payloads, seg_start, first_zw) instead, first_zw
         a uint64 array with each segment's segment-relative index of its first zero-width token or _lib.NO_ZERO_WIDTH (a segment with
-        an index has an unspecified payload: cz_model_set_zero_width_out)."""
+        an index has an unspecified payload: cz_model_set_zero_width_out).
+        dictionary: symbols every segment is coded as if it followed (cz_model_set_dictionary); decode with the same ones."""
         self.set_pdf_floor(pdf_floor)
         a, p = _u32(ids)
         n = a.shape[0]
@@ -281,19 +301,21 @@ class Model:
         data = np.empty(cap, np.uint8)
         seg_off = np.zeros(int(s.n_segments) + 1, np.uint64)
         bs = _lib.Bitstreams(data.ctypes.data_as(_lib.u8p), cap, seg_off.ctypes.data_as(_lib.u64p))
+        run = lambda: check(lib.cz_encode(self._h, p, n, C.byref(s), C.byref(bs)))  # noqa: E731
         if not zero_width_out:
-            check(lib.cz_encode(self._h, p, n, C.byref(s), C.byref(bs)))
+            self._with_dictionary(dictionary, run)
         else:
             first_zw = np.zeros(max(1, int(s.n_segments)), np.uint64)
             check(lib.cz_model_set_zero_width_out(self._h, first_zw.ctypes.data_as(_lib.u64p), first_zw.shape[0]))
             try:
-                check(lib.cz_encode(self._h, p, n, C.byref(s), C.byref(bs)))
+                self._with_dictionary(dictionary, run)
             finally:
                 check(lib.cz_model_set_zero_width_out(self._h, None, 0))
         pay = [data[int(seg_off[g]) : int(seg_off[g + 1])].tobytes() for g in range(int(s.n_segments))]
         return (pay, seg_start, first_zw[: int(s.n_segments)]) if zero_width_out else (pay, seg_start)
 
-    def analyze(self, ids, n_segments=1, seg_start=None, bos=0, context=512, reprime_interval=512, pdf_floor=False, max_batch_tokens=0):
+    def analyze(self, ids, n_segments=1, seg_start=None, bos=0, context=512, reprime_interval=512, pdf_floor=False, max_batch_tokens=0,
+                dictionary=None):
         """Where the bits go: encodes ids as encode() does, with the code-length and zero-width sinks set (cleared again afterwards).
         Returns a dict with
           payloads, seg_start   as encode() returns them
@@ -303,7 +325,8 @@ class Model:
           bits                  float64 [n]: 30 - log2(c_hi - c_lo), the token's exact code length before coder overhead; +inf where the
                                 interval is empty (a zero-width token)
           entropy               float64 [n]: the expected code length of the distribution the token was coded from (cz_cdf_entropy), in
-                                the alphabet of the call (pdf_floor applies)"""
+                                the alphabet of the call (pdf_floor applies)
+        dictionary as in encode()."""
         a, p = _u32(ids)
         n = a.shape[0]
         if self.cfg.get("arch", 0) == _lib.CZ_ARCH_RWKV7 and pdf_floor:
@@ -331,7 +354,7 @@ class Model:
         try:
             check(lib.cz_model_set_code_length_out(self._h, c_lo.ctypes.data_as(_lib.u32p), c_hi.ctypes.data_as(_lib.u32p),
                                                    ent.ctypes.data_as(_lib.f64p), c_lo.shape[0]))
-            check(lib.cz_encode(self._h, p, n, C.byref(s), C.byref(bs)))
+            self._with_dictionary(dictionary, lambda: check(lib.cz_encode(self._h, p, n, C.byref(s), C.byref(bs))))
         finally:
             check(lib.cz_model_set_code_length_out(self._h, None, None, None, 0))
             check(lib.cz_model_set_zero_width_out(self._h, None, 0))
@@ -340,9 +363,10 @@ class Model:
         return dict(payloads=pay, seg_start=seg_start, first_zw=first_zw[:n_seg], c_lo=c_lo, c_hi=c_hi, bits=code_length_bits(c_lo, c_hi),
                     entropy=ent)
 
-    def decode(self, payloads, seg_start, bos=0, context=512, reprime_interval=512, max_batch_tokens=0, events=None, pdf_floor=False):
+    def decode(self, payloads, seg_start, bos=0, context=512, reprime_interval=512, max_batch_tokens=0, events=None, pdf_floor=False,
+               dictionary=None):
         """events: the same gated hint primes the encoder was given (src/main.rs:2586-2614), single segment only;
-        pdf_floor: the setting the stream was encoded with"""
+        pdf_floor, dictionary: the settings the stream was encoded with"""
         self.set_pdf_floor(pdf_floor)
         seg_start = np.asarray(seg_start, np.uint64)
         n = int(seg_start[-1])
@@ -351,7 +375,8 @@ class Model:
         seg_off = np.concatenate([[0], np.cumsum(lens)]).astype(np.uint64)
         blob, blobp = _u8(np.frombuffer(b"".join(payloads) + b"\0", dtype=np.uint8))
         out = np.empty(max(n, 1), np.uint32)
-        check(lib.cz_decode(self._h, blobp, seg_off.ctypes.data_as(_lib.u64p), n, C.byref(s), out.ctypes.data_as(_lib.u32p)))
+        self._with_dictionary(dictionary, lambda: check(lib.cz_decode(self._h, blobp, seg_off.ctypes.data_as(_lib.u64p), n, C.byref(s),
+                                                                      out.ctypes.data_as(_lib.u32p))))
         return out[:n]
 
     def xe_bits(self, jobs):

@@ -11,6 +11,10 @@
       -- lossy for non-UTF-8 input                                   offline: byte-exact for EVERY input (SURVEY 7.3c)
   encode_file / decode_file container assembly (1793-2405,         compress() / decompress(): header v2 (+ SEG1 segment table,
       2407-2660)                                                     + AGT2 gates), BLAKE3-128 ids, orig hash VERIFIED on decode
+
+dictionary= (bytes, every entry point): a preset dictionary.  Each segment is coded as if it followed the dictionary's symbols
+(cz_model_set_dictionary), which are never stored: the container records their count and BLAKE3-128 (DIC1), and decoding needs the same
+dictionary.  Small files, which are all cold start, gain the most.
 """
 import json
 import sys
@@ -103,6 +107,19 @@ def tokenize(model, data: bytes, tokenizer):
     return tokenizer.encode_bytes(data)
 
 
+def dictionary_symbols(model, dictionary, tokenizer):
+    """the coded symbols of a dictionary (bytes, tokenised like the file, literal escapes included), or None for no dictionary"""
+    if not dictionary:
+        return None
+    d = np.asarray(tokenize(model, bytes(dictionary), tokenizer), np.uint32)
+    return d if d.shape[0] else None
+
+
+def _dict_kw(d):
+    """keyword arguments of a Model call: only with a dictionary, so that models without the keyword work as before"""
+    return {} if d is None else dict(dictionary=d)
+
+
 def header_fields(model, data: bytes, n_tokens, bos, context, reprime_interval, model_hash16, tokenizer_hash16):
     return dict(bos_token_id=bos, token_count=n_tokens, orig_len_bytes=len(data), model_hash16=model_hash16,
                 tokenizer_hash16=tokenizer_hash16, orig_hash16=container.blake3_16(data), context_window=context,
@@ -113,24 +130,27 @@ def stored_container(fields, model_repr, data: bytes) -> bytes:
     return container.write_container(dict(fields, reserved_flags=_lib.CZ_FLAG_STORED), model_repr, [bytes(data)])
 
 
-def coded_container(model, fields, model_repr, pays, seg) -> bytes:
-    """one payload: the reference's v2 layout; several: the SEG1 table"""
+def coded_container(model, fields, model_repr, pays, seg, dictionary=None) -> bytes:
+    """one payload: the reference's v2 layout; several: the SEG1 table; a dictionary (its symbols): the DIC1 section"""
     seg_tokens = np.diff(seg) if len(pays) > 1 else None
-    return container.write_container(fields, model_repr, pays, seg_tokens=seg_tokens, engine=model.engine)
+    return container.write_container(fields, model_repr, pays, seg_tokens=seg_tokens, engine=model.engine,
+                                     dictionary=None if dictionary is None else container.dictionary_id(dictionary))
 
 
 def compress(model, data: bytes, tokenizer=None, n_segments=1, bos=0, context=512, reprime_interval=512, model_repr=b"model.safetensors",
-             model_hash16=b"\0" * 16, tokenizer_hash16=b"\0" * 16, on_zero_width="stored"):
+             model_hash16=b"\0" * 16, tokenizer_hash16=b"\0" * 16, on_zero_width="stored", dictionary=None):
     """bytes -> .canz container bytes.  n_segments == 1 gives the reference's v2 layout (header | payload).
     on_zero_width: what to do when the SmolLM coder meets a token it cannot code (CZ_ERR_ZERO_WIDTH): "stored" writes the bytes
     uncoded (CZ_FLAG_STORED), "floor" codes the whole input again with the floored pdf (CZ_FLAG_PDF_FLOOR).  An input that codes
-    without such a token gives the same container either way."""
+    without such a token gives the same container either way.  dictionary: bytes every segment is coded as if it followed (module
+    docstring); None or empty writes a container without one."""
     _check_policy(on_zero_width)
     tokenizer = tokenizer or ByteTokenizer()
     ids = tokenize(model, data, tokenizer)
+    d = dictionary_symbols(model, dictionary, tokenizer)
     fields = header_fields(model, data, len(ids), bos, context, reprime_interval, model_hash16, tokenizer_hash16)
     try:
-        pays, seg = model.encode(ids, n_segments=n_segments, bos=bos, context=context, reprime_interval=reprime_interval)
+        pays, seg = model.encode(ids, n_segments=n_segments, bos=bos, context=context, reprime_interval=reprime_interval, **_dict_kw(d))
     except _lib.CzError as e:
         if e.code != _lib.CZ_ERR_ZERO_WIDTH:
             raise
@@ -140,12 +160,13 @@ def compress(model, data: bytes, tokenizer=None, n_segments=1, bos=0, context=51
         # (the message names the offending token index for whoever wants to know why).
         if on_zero_width == "floor":
             sys.stderr.write(f"candlezip_b200: {e}; coding with the floored pdf\n")
-            pays, seg = model.encode(ids, n_segments=n_segments, bos=bos, context=context, reprime_interval=reprime_interval, pdf_floor=True)
+            pays, seg = model.encode(ids, n_segments=n_segments, bos=bos, context=context, reprime_interval=reprime_interval, pdf_floor=True,
+                                     **_dict_kw(d))
             fields["reserved_flags"] = _lib.CZ_FLAG_PDF_FLOOR
         else:
             sys.stderr.write(f"candlezip_b200: {e}; writing a STORED container\n")
             return stored_container(fields, model_repr, data)
-    return coded_container(model, fields, model_repr, pays, seg)
+    return coded_container(model, fields, model_repr, pays, seg, d)
 
 
 class _Parsed:
@@ -155,7 +176,9 @@ class _Parsed:
         self.f, self.pays, self.seg, self.key, self.data = f, pays, seg, key, data
 
 
-def _parse(model, blob: bytes, verify) -> _Parsed:
+def _parse(model, blob: bytes, verify, dictionary=None) -> _Parsed:
+    """dictionary: the symbols the caller offers (dictionary_symbols); used only where the container names a dictionary, which must
+    then be this one"""
     f, _, gates, _, seg_tokens, pays = container.read_container(blob)
     n = int(f["token_count"])
     pdf_floor = bool(f["reserved_flags"] & _lib.CZ_FLAG_PDF_FLOOR)
@@ -171,7 +194,13 @@ def _parse(model, blob: bytes, verify) -> _Parsed:
     seg = np.concatenate([[0], np.cumsum(seg_tokens)]).astype(np.uint64) if seg_tokens is not None else np.array([0, n], np.uint64)
     if int(seg[-1]) != n:
         raise ValueError("segment table does not add up to token_count")
-    key = (int(f["bos_token_id"]), int(f["context_window"]), int(f["reprime_interval"]), pdf_floor)
+    named = f.get("dictionary")
+    if named is not None:
+        if dictionary is None:
+            raise ValueError(f"the container was coded with a dictionary of {named[0]} symbols; none was given")
+        if container.dictionary_id(dictionary) != named:
+            raise ValueError("the container was coded with a different dictionary than the one given")
+    key = (int(f["bos_token_id"]), int(f["context_window"]), int(f["reprime_interval"]), pdf_floor, None if named is None else named[1])
     return _Parsed(f, pays=pays, seg=seg, key=key)
 
 
@@ -190,13 +219,16 @@ def _finish(model, tokenizer, f, ids, verify) -> bytes:
     return data
 
 
-def decompress(model, blob: bytes, tokenizer=None, verify=True) -> bytes:
+def decompress(model, blob: bytes, tokenizer=None, verify=True, dictionary=None) -> bytes:
+    """dictionary: the one the container was compressed with; it is checked against the container's DIC1 record before any decoding"""
     tokenizer = tokenizer or ByteTokenizer()
-    p = _parse(model, blob, verify)
+    d = dictionary_symbols(model, dictionary, tokenizer)
+    p = _parse(model, blob, verify, d)
     if p.data is not None:
         return p.data
-    bos, context, reprime_interval, pdf_floor = p.key
-    ids = model.decode(p.pays, p.seg, bos=bos, context=context, reprime_interval=reprime_interval, pdf_floor=pdf_floor)
+    bos, context, reprime_interval, pdf_floor, dict_hash = p.key
+    ids = model.decode(p.pays, p.seg, bos=bos, context=context, reprime_interval=reprime_interval, pdf_floor=pdf_floor,
+                       **_dict_kw(None if dict_hash is None else d))
     return _finish(model, tokenizer, p.f, ids, verify)
 
 
@@ -260,18 +292,19 @@ def encode_many(id_lists, n_segments, encode_fn, on_zero_width="stored"):
 
 
 def compress_many(model, datas, tokenizer=None, n_segments=1, bos=0, context=512, reprime_interval=512, model_repr=b"model.safetensors",
-                  model_hash16=b"\0" * 16, tokenizer_hash16=b"\0" * 16, on_zero_width="stored"):
+                  model_hash16=b"\0" * 16, tokenizer_hash16=b"\0" * 16, on_zero_width="stored", dictionary=None):
     """[bytes] -> [container bytes], element i equal byte for byte to compress(model, datas[i], <same arguments>).  The segments of all
     files are coded in one Model.encode call with the per-segment zero-width report on; the files that report a zero-width token get
-    the on_zero_width fallback (all "floor" files in one more call)."""
+    the on_zero_width fallback (all "floor" files in one more call, with the same dictionary)."""
     _check_policy(on_zero_width)
     tokenizer = tokenizer or ByteTokenizer()
     id_lists = [tokenize(model, d, tokenizer) for d in datas]
+    dsym = dictionary_symbols(model, dictionary, tokenizer)
 
     def encode_fn(ids, seg_start, pdf_floor):
         # the sink is set on the floored call too: no token can be zero-width there, and encode_many checks that none was
         pays, _, first_zw = model.encode(ids, seg_start=seg_start, bos=bos, context=context, reprime_interval=reprime_interval,
-                                         pdf_floor=pdf_floor, zero_width_out=True)
+                                         pdf_floor=pdf_floor, zero_width_out=True, **_dict_kw(dsym))
         return pays, first_zw
 
     out = []
@@ -283,13 +316,13 @@ def compress_many(model, datas, tokenizer=None, n_segments=1, bos=0, context=512
             continue
         if flag == _lib.CZ_FLAG_PDF_FLOOR:
             sys.stderr.write(f"candlezip_b200: file {i}: zero-width coding interval; coded with the floored pdf\n")
-        out.append(coded_container(model, dict(fields, reserved_flags=flag), model_repr, pays, loc))
+        out.append(coded_container(model, dict(fields, reserved_flags=flag), model_repr, pays, loc, dsym))
     return out
 
 
 def decode_waves(jobs, max_streams):
     """jobs[i]: None (nothing to decode) or (key, segment lengths) of file i.  Segments of files with the same key (bos, context,
-    reprime_interval, pdf_floor) share calls; within a key they are sorted by length, longest first (stable), which is the lock-step
+    reprime_interval, pdf_floor, dictionary hash or None) share calls; within a key they are sorted by length, longest first (stable), which is the lock-step
     decoder's precondition, and cut into waves of at most max_streams.  Zero-length segments decode to nothing and are left out.
     Returns [(key, [(file, segment, length)])], one entry per decode call."""
     if max_streams < 1:
@@ -320,24 +353,27 @@ def decode_many(jobs, payloads, decode_fn, max_streams):
     return [None if p is None else np.concatenate(p).astype(np.uint32) for p in parts]
 
 
-def decompress_many(model, blobs, tokenizer=None, max_streams=2048, verify=True) -> list:
+def decompress_many(model, blobs, tokenizer=None, max_streams=2048, verify=True, dictionary=None) -> list:
     """[container bytes] -> [bytes], element i equal to decompress(model, blobs[i], tokenizer).  STORED containers and empty files need
     no GPU work; the segments of all other containers are decoded in lock-step waves of at most max_streams streams (decode_waves).
     The default of 2,048 streams decodes at nearly the 4,096-stream rate with half the KV memory (48 GB for SmolLM-135M), and lets a
     container with more segments than one cz_decode call could hold decode too.  A gated (AGT2) container, a bad header or a hash
-    mismatch raises ValueError naming the index of the blob."""
+    mismatch raises ValueError naming the index of the blob, as does a container that names a dictionary other than `dictionary` (all
+    before any decoding).  Containers without a dictionary decode without it, in calls of their own."""
     tokenizer = tokenizer or ByteTokenizer()
+    d = dictionary_symbols(model, dictionary, tokenizer)
     parsed = []
     for i, blob in enumerate(blobs):
         try:
-            parsed.append(_parse(model, blob, verify))
+            parsed.append(_parse(model, blob, verify, d))
         except ValueError as e:
             raise ValueError(f"blob {i}: {e}") from None
     jobs = [None if p.data is not None or int(p.f["token_count"]) == 0 else (p.key, np.diff(p.seg)) for p in parsed]
 
     def decode_fn(key, pays, seg_start):
-        bos, context, reprime_interval, pdf_floor = key
-        return model.decode(pays, seg_start, bos=bos, context=context, reprime_interval=reprime_interval, pdf_floor=pdf_floor)
+        bos, context, reprime_interval, pdf_floor, dict_hash = key
+        return model.decode(pays, seg_start, bos=bos, context=context, reprime_interval=reprime_interval, pdf_floor=pdf_floor,
+                            **_dict_kw(None if dict_hash is None else d))
 
     ids = decode_many(jobs, [p.pays for p in parsed], decode_fn, max_streams)
     out = []
@@ -357,18 +393,20 @@ def decompress_many(model, blobs, tokenizer=None, max_streams=2048, verify=True)
 # the distribution it was coded from (the model's uncertainty, as opposed to its surprise at the actual token), and where the token sits
 # in its segment and in its reprime chunk.  Everything below except analyze() itself is pure and needs no device.
 
-def schedule_chunks(n_tokens, context, reprime_interval):
+def schedule_chunks(n_tokens, context, reprime_interval, n_prefix=0):
     """(first coded index, number coded) of each chunk of one segment of n_tokens (cz_schedule_chunks, host-only): a chunk starts from
-    BOS or from a reprime of the last min(context, 511) tokens"""
-    k = int(_lib.lib.cz_schedule_chunks(int(n_tokens), int(context), int(reprime_interval), None, None, None, None, 0))
+    BOS or from a reprime of the last min(context, 511) tokens.  n_prefix: the segment follows a dictionary of that many symbols
+    (cz_schedule_chunks_prefixed)"""
+    args = (int(n_tokens), int(n_prefix), int(context), int(reprime_interval))
+    k = int(_lib.lib.cz_schedule_chunks_prefixed(*args, None, None, None, None, 0))
     first, n_coded = np.zeros(max(k, 1), np.uint64), np.zeros(max(k, 1), np.uint32)
-    _lib.lib.cz_schedule_chunks(int(n_tokens), int(context), int(reprime_interval), first.ctypes.data_as(_lib.u64p),
-                                n_coded.ctypes.data_as(_lib.u32p), None, None, k)
+    _lib.lib.cz_schedule_chunks_prefixed(*args, first.ctypes.data_as(_lib.u64p), n_coded.ctypes.data_as(_lib.u32p), None, None, k)
     return first[:k].astype(np.int64), n_coded[:k].astype(np.int64)
 
 
-def token_positions(seg_start, context, reprime_interval, reprime=True):
-    """per coded token: segment index, position in the segment, reprime-chunk index in the segment and position in the chunk.
+def token_positions(seg_start, context, reprime_interval, reprime=True, n_prefix=0):
+    """per coded token: segment index, position in the segment, reprime-chunk index in the segment and position in the chunk (the chunk
+    in which a dictionary of n_prefix symbols ends counts from its first coded token).
     reprime=False (RWKV-7, whose state runs over the whole segment): one chunk per segment."""
     seg_start = np.asarray(seg_start, np.int64)
     n = int(seg_start[-1])
@@ -379,7 +417,7 @@ def token_positions(seg_start, context, reprime_interval, reprime=True):
         pos[a:b] = np.arange(b - a)
         if b == a:
             continue
-        first, n_coded = schedule_chunks(b - a, context, reprime_interval) if reprime else (np.zeros(1, np.int64), np.array([b - a]))
+        first, n_coded = schedule_chunks(b - a, context, reprime_interval, n_prefix) if reprime else (np.zeros(1, np.int64), np.array([b - a]))
         for c, (f, k) in enumerate(zip(first, n_coded)):
             chunk[a + f:a + f + k] = c
             cpos[a + f:a + f + k] = np.arange(k)
@@ -437,15 +475,19 @@ def summarize(bits, entropy, seg, seg_pos, chunk_pos, payload_lens, n_bytes, max
                 segments=segments, by_chunk_position=bucket_means(chunk_pos, bits, entropy), by_segment_position=bucket_means(seg_pos, bits, entropy))
 
 
-def analyze(model, data: bytes, tokenizer=None, n_segments=1, bos=0, context=512, reprime_interval=512, pdf_floor=False):
+def analyze(model, data: bytes, tokenizer=None, n_segments=1, bos=0, context=512, reprime_interval=512, pdf_floor=False, dictionary=None):
     """per-token code lengths of `data`, tokenised and split as compress() does.  Returns (arrays, summary): arrays holds, per coded
     token, ids, bits (its exact code length: 30 - log2 of its interval width, +inf for a zero-width token), entropy (the expected code
     length of the distribution it was coded from), segment, segment_position, chunk, chunk_position; plus seg_start, first_zw and
-    payload_lens per segment.  pdf_floor codes with the floored SmolLM pdf (as compress(on_zero_width="floor") would)."""
+    payload_lens per segment.  pdf_floor codes with the floored SmolLM pdf (as compress(on_zero_width="floor") would); dictionary as
+    compress() takes it."""
     tokenizer = tokenizer or ByteTokenizer()
     ids = tokenize(model, data, tokenizer)
-    r = model.analyze(ids, n_segments=n_segments, bos=bos, context=context, reprime_interval=reprime_interval, pdf_floor=pdf_floor)
-    seg, pos, chunk, cpos = token_positions(r["seg_start"], context, reprime_interval, reprime=model.cfg.get("arch", 0) != 1)
+    d = dictionary_symbols(model, dictionary, tokenizer)
+    r = model.analyze(ids, n_segments=n_segments, bos=bos, context=context, reprime_interval=reprime_interval, pdf_floor=pdf_floor,
+                      **_dict_kw(d))
+    seg, pos, chunk, cpos = token_positions(r["seg_start"], context, reprime_interval, reprime=model.cfg.get("arch", 0) != 1,
+                                            n_prefix=0 if d is None else d.shape[0])
     payload_lens = np.array([len(p) for p in r["payloads"]], np.int64)
     arrays = dict(ids=np.asarray(ids, np.uint32), bits=r["bits"], entropy=r["entropy"], segment=seg, segment_position=pos, chunk=chunk,
                   chunk_position=cpos, seg_start=np.asarray(r["seg_start"], np.uint64), first_zw=r["first_zw"], payload_lens=payload_lens)

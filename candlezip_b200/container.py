@@ -1,4 +1,4 @@
-"""Container v2 (+ segment-table extension) over the C ABI: src/main.rs:227-259, 551-677."""
+"""Container v2 (+ segment-table and dictionary extensions) over the C ABI: src/main.rs:227-259, 551-677."""
 import ctypes as C
 
 import numpy as np
@@ -7,6 +7,7 @@ from . import _lib
 from ._lib import lib
 
 CZ_FLAG_SEGMENTS = _lib.CZ_FLAG_SEGMENTS
+CZ_FLAG_DICTIONARY = _lib.CZ_FLAG_DICTIONARY
 
 
 def blake3_16(data: bytes) -> bytes:
@@ -14,6 +15,12 @@ def blake3_16(data: bytes) -> bytes:
     out = (C.c_uint8 * 16)()
     lib.cz_blake3_16(buf, len(data), out)
     return bytes(out)
+
+
+def dictionary_id(symbols):
+    """(n_symbols, BLAKE3-128 of the symbols as little-endian u32): what a DIC1 section records of a dictionary"""
+    a = np.asarray(symbols, np.uint32)
+    return int(a.shape[0]), blake3_16(a.astype("<u4").tobytes())
 
 
 def _hdr(fields: dict, repr_len: int):
@@ -32,9 +39,14 @@ def _hdr(fields: dict, repr_len: int):
     return h
 
 
-def write_container(fields: dict, model_file_repr: bytes, payloads, seg_tokens=None, gates=None, engine=0) -> bytes:
-    """One payload and no seg_tokens -> byte-identical layout to the reference (header | [AGT2] | payload)."""
+def write_container(fields: dict, model_file_repr: bytes, payloads, seg_tokens=None, gates=None, engine=0, dictionary=None) -> bytes:
+    """One payload and no seg_tokens -> byte-identical layout to the reference (header | [AGT2] | payload).
+    dictionary: dictionary_id() of the dictionary the payloads were coded with (CZ_FLAG_DICTIONARY + a DIC1 section), or None."""
     flags = fields.get("reserved_flags", 0)
+    if dictionary is not None:
+        if flags & _lib.CZ_FLAG_STORED:
+            raise ValueError("a STORED payload is not coded: it has no dictionary")
+        flags |= CZ_FLAG_DICTIONARY
     segmented = seg_tokens is not None and len(payloads) >= 1 and not (len(payloads) == 1 and seg_tokens is None)
     if seg_tokens is not None:
         flags |= CZ_FLAG_SEGMENTS
@@ -60,13 +72,20 @@ def write_container(fields: dict, model_file_repr: bytes, payloads, seg_tokens=N
         k = lib.cz_container_write_segments(sbuf, len(sbuf), engine, st.ctypes.data_as(_lib.u64p), sb.ctypes.data_as(_lib.u64p), len(payloads))
         assert k, "segment table write failed"
         out += bytes(sbuf[:k])
+    if dictionary is not None:
+        n_sym, h16 = dictionary
+        db = (C.c_uint8 * 32)()
+        k = lib.cz_container_write_dictionary(db, len(db), int(n_sym), (C.c_uint8 * 16)(*h16))
+        assert k, "dictionary section write failed"
+        out += bytes(db[:k])
     for p in payloads:
         out += p
     return bytes(out)
 
 
 def read_container(blob: bytes):
-    """Returns (fields dict, repr bytes, gates list or None, engine, seg_tokens, payload list)."""
+    """Returns (fields dict, repr bytes, gates list or None, engine, seg_tokens, payload list).  A container with CZ_FLAG_DICTIONARY
+    has fields["dictionary"] = (n_symbols, BLAKE3-128 of the symbols), as dictionary_id() gives them."""
     buf = (C.c_uint8 * len(blob)).from_buffer_copy(blob)
     h = _lib.HeaderV2()
     ro = C.c_size_t()
@@ -101,6 +120,7 @@ def read_container(blob: bytes):
                                        C.byref(cnt))
         n += k
         engine, seg_tokens = eng.value, st
+        n = _read_dictionary(blob, n, h, fields)
         if int(sb.sum()) != len(blob) - n:
             raise ValueError(f"segment table declares {int(sb.sum())} payload bytes but {len(blob) - n} follow it")
         if int(st.sum()) != int(h.token_count):
@@ -110,5 +130,22 @@ def read_container(blob: bytes):
             payloads.append(blob[n : n + int(b)])
             n += int(b)
     else:
+        n = _read_dictionary(blob, n, h, fields)
         payloads = [blob[n:]]
     return fields, rep, gates, engine, seg_tokens, payloads
+
+
+def _read_dictionary(blob, n, h, fields):
+    """the DIC1 section at blob[n:] when the header has CZ_FLAG_DICTIONARY: fills fields["dictionary"], returns the offset after it"""
+    if not h.reserved_flags & CZ_FLAG_DICTIONARY:
+        return n
+    if h.reserved_flags & _lib.CZ_FLAG_STORED:
+        raise ValueError("DICTIONARY marks a coded payload: invalid with STORED")
+    sub = (C.c_uint8 * max(1, len(blob) - n)).from_buffer_copy(blob[n:] or b"\0")
+    cnt = C.c_uint64()
+    h16 = (C.c_uint8 * 16)()
+    k = lib.cz_container_read_dictionary(sub, len(blob) - n, C.byref(cnt), h16)
+    if not k:
+        raise ValueError("bad dictionary section")
+    fields["dictionary"] = (int(cnt.value), bytes(h16))
+    return n + k

@@ -309,4 +309,25 @@ size_t cz_container_read_segments(const uint8_t *buf, size_t len, int *engine, u
   return k;
 }
 
+size_t cz_container_write_dictionary(uint8_t *buf, size_t cap, uint64_t n_symbols, const uint8_t hash16[16]) {
+  const size_t need = 4 + var_len(n_symbols) + 16;
+  if (!buf || !hash16 || cap < need) return 0;
+  memcpy(buf, "DIC1", 4);
+  size_t k = 4 + put_var(buf + 4, n_symbols);
+  memcpy(buf + k, hash16, 16);
+  return k + 16;
+}
+
+size_t cz_container_read_dictionary(const uint8_t *buf, size_t len, uint64_t *n_symbols, uint8_t hash16[16]) {
+  if (!buf || len < 5 || memcmp(buf, "DIC1", 4)) return 0;
+  uint64_t n;
+  const size_t r = get_var(buf + 4, len - 4, &n);
+  if (!r || n == 0) return 0;  // an empty dictionary is written as no section at all
+  const size_t k = 4 + r;
+  if (len - k < 16) return 0;
+  if (n_symbols) *n_symbols = n;
+  if (hash16) memcpy(hash16, buf + k, 16);
+  return k + 16;
+}
+
 }  // extern "C"

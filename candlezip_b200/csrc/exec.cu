@@ -152,6 +152,32 @@ __global__ void fill_pos_from_ctr_kernel(int *__restrict__ p, const unsigned lon
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) p[i] = (int)ctr[1];
 }
+// Preset dictionary, SmolLM decode: positions [0, P) of the first chunk's prime are the same for every stream (BOS ++ dictionary), so
+// they are run for stream 0 only.  This copies stream 0's K / V rows of those positions, in every layer, to the arena slots
+// g * max_pos + p of the streams g in [1, n), and stream 0's logits column (and column max) to the others' columns.  A row's K / V and
+// logits do not depend on the batch it was computed in (DESIGN.md §3), so every stream gets what its own prime would have given.
+// blockIdx.y < 2 L: K (even) or V (odd) of layer y / 2, 16-byte pieces; blockIdx.y == 2 L: the logits.
+__global__ void kv_prefix_broadcast_kernel(__nv_bfloat16 *__restrict__ k, __nv_bfloat16 *__restrict__ v, size_t layer_stride, size_t slot_stride,
+                                           size_t n4, int n, float *__restrict__ logits, size_t ld, size_t V, int *__restrict__ colmax) {
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const size_t per = (size_t)(n - 1);
+  if (blockIdx.y < gridDim.y - 1) {
+    uint4 *base = (uint4 *)((blockIdx.y & 1 ? v : k) + (size_t)(blockIdx.y >> 1) * layer_stride);
+    const size_t slot4 = slot_stride / 8;  // bf16 elements -> 16-byte pieces
+    for (; i < n4 * per; i += stride) {
+      const size_t g = 1 + i / n4, e = i % n4;
+      base[g * slot4 + e] = base[e];
+    }
+    return;
+  }
+  for (; i < V * per; i += stride) {
+    const size_t row = i / per, g = 1 + i % per;
+    logits[row * ld + g] = logits[row * ld];
+    if (row == 0 && colmax) colmax[g] = colmax[0];
+  }
+}
+
 __global__ void sum_bits_kernel(const double *__restrict__ bits, const uint64_t *__restrict__ job_off, double *__restrict__ out, int n_jobs) {
   int j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= n_jobs) return;
@@ -433,6 +459,10 @@ static int check_ids(const uint32_t *ids, size_t n, uint32_t limit, const char *
 static uint32_t coded_limit(const cz_model *m) { return (uint32_t)m->cfg.vocab + (m->cfg.arch == CZ_ARCH_RWKV7 ? 256u : 0u); }
 static int check_schedule_ids(const cz_model *m, const cz_schedule *s) {
   CZ_TRY(check_ids(&s->bos, 1, (uint32_t)m->cfg.vocab, "schedule bos"));
+  if (!m->dictionary.empty() && s->n_events) {
+    set_error("schedule: hint prime events are not available with a dictionary");
+    return CZ_ERR_UNSUPPORTED;
+  }
   for (uint32_t e = 0; e < s->n_events; e++) {
     if (s->events[e].prime_len && !s->events[e].prime) {
       set_error("schedule: prime event without tokens");
@@ -453,6 +483,12 @@ static double host_ms() {
   timespec ts;
   clock_gettime(CLOCK_MONOTONIC, &ts);
   return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6;
+}
+
+// gather code (gather_tokens_kernel) of S[si] in a segment whose tokens start at ids[t0], S = BOS ++ dictionary ++ tokens; the
+// dictionary's symbols (n_dict of them) are the whole `extra` buffer, as a dictionary excludes hint-prime events
+static long long prefixed_src(uint64_t si, uint64_t n_dict, uint64_t t0) {
+  return si == 0 ? -1ll : si <= n_dict ? -1ll - (long long)si : (long long)(t0 + si - 1 - n_dict);
 }
 
 // host_cap: what the caller can take of the payload (cz_encode's cz_bitstreams.cap); checked before the code-length sinks are written.
@@ -484,8 +520,9 @@ static int encode_core(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
     ent_dev = m->sb[SB_ENT].as<double>();
   }
   CZ_TRY(digest_begin(m, n_tokens, 262144, st));
-  // explicit prime token lists of the hint events
-  std::vector<uint32_t> extra;
+  // explicit prime token lists of the hint events, or the dictionary (check_schedule_ids: never both)
+  std::vector<uint32_t> extra(m->dictionary);
+  const uint64_t n_dict = m->dictionary.size();
   std::vector<size_t> ev_off(sched->n_events + 1, 0);
   for (uint32_t e = 0; e < sched->n_events; e++) {
     ev_off[e] = extra.size();
@@ -522,7 +559,8 @@ static int encode_core(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
   }
   for (uint32_t g = 0; g < S && m->cfg.arch != CZ_ARCH_RWKV7; g++) {
     const uint64_t t0 = sched->seg_start[g], n = sched->seg_start[g + 1] - t0;
-    build_chunks(n, sched->context, sched->reprime_interval, sched->events, sched->n_events, chunks);
+    if (n_dict) build_chunks_prefixed(n, n_dict, sched->context, sched->reprime_interval, chunks);
+    else build_chunks(n, sched->context, sched->reprime_interval, sched->events, sched->n_events, chunks);
     for (const Chunk &c : chunks) {
       const size_t rows = (size_t)c.prime_len + c.n_coded - 1;
       if (rows > (size_t)m->max_seq()) {
@@ -544,8 +582,7 @@ static int encode_core(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
                     },
                     [&](uint32_t j) { return (long long)(t0 + c.first + j); });
       } else {
-        w.add_chunk(c.prime_len, c.n_coded,
-                    [&](uint32_t k) { uint64_t si = c.prime_start + k; return si == 0 ? -1ll : (long long)(t0 + si - 1); },
+        w.add_chunk(c.prime_len, c.n_coded, [&](uint32_t k) { return prefixed_src(c.prime_start + k, n_dict, t0); },
                     [&](uint32_t j) { return (long long)(t0 + c.first + j); });
       }
       coded_done += c.n_coded;
@@ -785,7 +822,9 @@ int cz_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, size
   uint64_t max_len = 0;
   for (uint32_t g = 0; g < S; g++) max_len = std::max<uint64_t>(max_len, sched->seg_start[g + 1] - sched->seg_start[g]);
   std::vector<Chunk> chunks;  // master timeline = chunk structure of the longest segment
-  build_chunks(max_len, sched->context, sched->reprime_interval, sched->events, sched->n_events, chunks);  // events: S == 1
+  const uint64_t n_dict = m->dictionary.size();
+  if (n_dict) build_chunks_prefixed(max_len, n_dict, sched->context, sched->reprime_interval, chunks);
+  else build_chunks(max_len, sched->context, sched->reprime_interval, sched->events, sched->n_events, chunks);  // events: S == 1
   size_t max_pos = 0;
   for (const Chunk &ch : chunks) max_pos = std::max<size_t>(max_pos, (size_t)ch.prime_len + ch.n_coded);
   max_pos = (max_pos + 63) & ~(size_t)63;
@@ -810,8 +849,8 @@ int cz_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, size
   CZ_CUDA_TRY(cudaMemcpyAsync(d_pay.p, payload, pay_total, cudaMemcpyHostToDevice, st));
   CZ_CUDA_TRY(cudaMemcpyAsync(d_off.p, seg_off, (S + 1) * 8, cudaMemcpyHostToDevice, st));
   CZ_CUDA_TRY(cudaMemcpyAsync(d_start.p, sched->seg_start, (S + 1) * 8, cudaMemcpyHostToDevice, st));
-  // explicit prime token lists of the gated hint events (src/main.rs:2586-2614)
-  std::vector<uint32_t> extra;
+  // explicit prime token lists of the gated hint events (src/main.rs:2586-2614), or the dictionary (never both)
+  std::vector<uint32_t> extra(m->dictionary);
   std::vector<size_t> ev_off(sched->n_events + 1, 0);
   for (uint32_t e = 0; e < sched->n_events; e++) {
     ev_off[e] = extra.size();
@@ -866,7 +905,11 @@ int cz_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, size
         return CZ_ERR_UNSUPPORTED;
       }
     w.clear();
+    // a prime made of BOS and dictionary positions only (the chunk in which the dictionary ends) is the same for every stream: it runs
+    // for stream 0, and kv_prefix_broadcast_kernel gives its K / V rows and logits to the others
+    const bool shared_prime = n_dict && ch.event < 0 && ch.prime_start + ch.prime_len <= 1 + n_dict;
     for (uint32_t g : live) {
+      if (shared_prime && g > 0) break;
       const uint64_t t0 = sched->seg_start[g];
       const int base = (int)(g * max_pos);
       const int r0 = (int)w.src.size();
@@ -878,7 +921,7 @@ int cz_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, size
           if (k >= hist) w.src.push_back(-2 - (long long)(ev_off[ch.event] + (k - hist)));
           else w.src.push_back(sh == 0 ? -1ll : (long long)(t0 + sh - 1));
         } else {
-          w.src.push_back(si == 0 ? -1ll : (long long)(t0 + si - 1));
+          w.src.push_back(prefixed_src(si, n_dict, t0));
         }
         w.pos.push_back((int)k);
         w.kv_base.push_back(base);
@@ -905,6 +948,14 @@ int cz_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, size
       CZ_TRY(lm_head(m, 0, (int)NL, d_logits.as<float>(), S_pad, st, ws.colmax, &have_max));
     }
     const int n_live = (int)live.size();
+    if (shared_prime && n_live > 1) {
+      const size_t n4 = (size_t)ch.prime_len * kvd / 8;  // stream 0's rows [0, prime_len) of one layer, in 16-byte pieces
+      CZ_LAUNCH(ctx, CZ_K_OTHER,
+                (czk::kv_prefix_broadcast_kernel<<<dim3(296, (unsigned)(2 * L + 1)), 256, 0, st>>>(
+                    kv.k, kv.v, kv.layer_stride, max_pos * kvd, n4, n_live, d_logits.as<float>(), S_pad, (size_t)c.vocab,
+                    have_max ? m->ws.colmax : nullptr)));
+      CZ_CHECK_LAUNCH();
+    }
     Workspace &ws = m->ws;
     // per-chunk constants of the single-token steps: row g = stream g, one attention tile per row
     CZ_CUDA_TRY(cudaMemcpyAsync(ws.kv_base, d_kvb_i, (size_t)n_live * 4, cudaMemcpyDeviceToDevice, st));

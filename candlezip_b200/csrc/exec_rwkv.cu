@@ -91,6 +91,22 @@ __global__ void rw_commit_logits_kernel(const float *__restrict__ fresh, float *
   if (col < (size_t)n_lanes && active[col]) keep[i] = fresh[i];
 }
 
+// Preset dictionary: copies the recurrent state of slot 0 -- the WKV state [L][cap][H * 4096] and the token-shift rows xa / xf
+// [L][cap][C] of the current ping-pong side -- to slots [1, n), so every stream starts from the state the dictionary left.
+// 16-byte pieces; blockIdx.y = 0: WKV state, 1: xa, 2: xf.
+__global__ void rwkv_state_broadcast_kernel(float *__restrict__ S, float *__restrict__ xa, float *__restrict__ xf, int L, size_t cap,
+                                            size_t s4, size_t c4, int n) {
+  const size_t per = (size_t)(n - 1);
+  const size_t w4 = blockIdx.y == 0 ? s4 : c4;  // 16-byte pieces per slot and layer
+  float4 *base = (float4 *)(blockIdx.y == 0 ? S : blockIdx.y == 1 ? xa : xf);
+  const size_t total = (size_t)L * per * w4;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+    const size_t e = i % w4, r = i / w4, g = 1 + r % per, l = r / per;
+    float4 *layer = base + l * cap * w4;
+    layer[g * w4 + e] = layer[e];
+  }
+}
+
 }  // namespace czk
 
 namespace cz {
@@ -116,6 +132,61 @@ static void build_unit(RwUnit &u, const std::vector<long long> &first_src, const
 
 // rows of one slab when the schedule sets no max_batch_tokens (encode), and the bound on a decode prime slab
 static const size_t kSlabRows = 262144;
+
+// Preset dictionary (cz_model_set_dictionary): a stream of D ++ T steps BOS and the in-vocabulary symbols of D before it codes T[0]
+// (literal escapes never step the model).  Every stream of a call shares that history, so it runs ONCE: `feed` = BOS and all but the
+// last in-vocabulary symbol, run for one slot; each stream then steps `last` itself (the gather code of that symbol in the dictionary,
+// which is the `extra` buffer, or -1 = BOS when D has no in-vocabulary symbol, in which case `feed` is empty).
+struct RwPrefix {
+  std::vector<uint32_t> feed;
+  long long last = -1;
+};
+static RwPrefix rwkv_prefix(const cz_model *m, uint32_t bos) {
+  RwPrefix p;
+  const std::vector<uint32_t> &d = m->dictionary;
+  for (size_t k = 0; k < d.size(); k++)
+    if (d[k] < (uint32_t)m->cfg.vocab) {
+      p.feed.push_back(p.last == -1 ? bos : d[(size_t)(-2 - p.last)]);  // (a gather code is negative: -1 is BOS, -2 - k is d[k])
+      p.last = -2 - (long long)k;
+    }
+  return p;
+}
+
+// runs p.feed through slot 0 of the freshly reset `stt` in slabs of at most max_rows rows, then copies slot 0's state to slots [1, n)
+static int rwkv_prefix_state(cz_model *m, RwkvState &stt, const RwPrefix &p, size_t n, size_t max_rows, cudaStream_t st) {
+  if (p.feed.empty()) return CZ_OK;  // the zero state
+  cz_ctx *ctx = m->ctx;
+  const cz_model_config &c = m->cfg;
+  Workspace &ws = m->ws;
+  RwkvWs &rw = m->rws;
+  const int zero = 0;
+  for (size_t k0 = 0; k0 < p.feed.size(); k0 += max_rows) {
+    const size_t T = std::min(max_rows, p.feed.size() - k0);
+    CZ_TRY(ensure_workspace(m, T, 1, 0));
+    CZ_TRY(rwkv_ensure_ws(m, T, 1));
+    std::vector<int> prev(T), slot(T, 0), flags(T, 0);
+    for (size_t k = 0; k < T; k++) prev[k] = (int)k - 1;
+    flags[T - 1] = 1;
+    const int re = (int)T;
+    CZ_CUDA_TRY(cudaMemcpyAsync(ws.tok, p.feed.data() + k0, T * 4, cudaMemcpyHostToDevice, st));
+    CZ_CUDA_TRY(cudaMemcpyAsync(rw.prev_row, prev.data(), T * 4, cudaMemcpyHostToDevice, st));
+    CZ_CUDA_TRY(cudaMemcpyAsync(rw.slot, slot.data(), T * 4, cudaMemcpyHostToDevice, st));
+    CZ_CUDA_TRY(cudaMemcpyAsync(rw.flags, flags.data(), T * 4, cudaMemcpyHostToDevice, st));
+    CZ_CUDA_TRY(cudaMemcpyAsync(rw.row_begin, &zero, 4, cudaMemcpyHostToDevice, st));
+    CZ_CUDA_TRY(cudaMemcpyAsync(rw.row_end, &re, 4, cudaMemcpyHostToDevice, st));
+    CZ_CUDA_TRY(cudaMemcpyAsync(rw.stream_slot, &zero, 4, cudaMemcpyHostToDevice, st));
+    CZ_TRY(rwkv_forward(m, (int)T, 1, stt, /*in_place=*/false, nullptr, st));
+    CZ_CUDA_TRY(cudaStreamSynchronize(st));  // the staging vectors are stack-owned
+  }
+  if (n > 1) {
+    const size_t C = c.d_model, H = C / 64;
+    CZ_LAUNCH(ctx, CZ_K_OTHER,
+              (czk::rwkv_state_broadcast_kernel<<<dim3(592, 3), 256, 0, st>>>(stt.S, stt.xa[stt.cur], stt.xf[stt.cur], c.n_layers, stt.cap,
+                                                                             H * 4096 / 4, C / 4, (int)n)));
+    CZ_CHECK_LAUNCH();
+  }
+  return CZ_OK;
+}
 
 // The units of one stream of n coded tokens under the schedule's hint-prime events (n_segments == 1 when there are any): unit u
 // covers coded indices [begin, next unit's begin) and starts from a zero state primed with BOS (event -1) or with the prime of
@@ -172,8 +243,9 @@ struct RwOut {
   bool digest = false;           // f-4: hash every column's logits into the model's digest buffer at its global coded index
 };
 
+// prefix (nullable): the units start from the state it leaves (rwkv_prefix_state) instead of the zero state
 static int rwkv_run_units(cz_model *m, std::vector<RwUnit> &units, const uint32_t *ids_dev, const uint32_t *extra_dev, uint32_t bos,
-                          const RwOut &o, size_t max_rows, cudaStream_t st) {
+                          const RwOut &o, size_t max_rows, cudaStream_t st, const RwPrefix *prefix = nullptr) {
   cz_ctx *ctx = m->ctx;
   const cz_model_config &c = m->cfg;
   const size_t U = units.size(), V = c.vocab;
@@ -183,6 +255,7 @@ static int rwkv_run_units(cz_model *m, std::vector<RwUnit> &units, const uint32_
   if (max_rows == 0) max_rows = kSlabRows;
   const size_t Tw = std::max<size_t>(1, std::min(max_steps, max_rows / U));
   CZ_TRY(rwkv_state_reset(m, m->rstate, U, st));
+  if (prefix) CZ_TRY(rwkv_prefix_state(m, m->rstate, *prefix, U, max_rows, st));
   std::vector<long long> src;
   std::vector<int> prev_row, slot, flags, row_begin, row_end, sslot, logit_rows;
   std::vector<unsigned long long> out_idx;
@@ -317,13 +390,14 @@ int rwkv_encode_bounds(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
   std::vector<RwUnit> units;
   std::vector<RwCut> cuts;
   std::vector<long long> first;
+  const RwPrefix prefix = rwkv_prefix(m, sched->bos);  // (a dictionary excludes events: extra_dev then holds the dictionary)
   for (uint32_t g = 0; g < sched->n_segments; g++) {
     const uint64_t a = sched->seg_start[g], b = sched->seg_start[g + 1];
     CZ_TRY(rwkv_plan_units(sched, b - a, V, cuts));
     for (size_t u = 0; u < cuts.size(); u++) {
       const uint64_t cur = a + cuts[u].begin, end = u + 1 < cuts.size() ? a + cuts[u + 1].begin : b;
       // BOS (main.rs:1916), or a gated hint prime, which restarts the state (main.rs:2137-2149 -> models.rs:162-170)
-      if (cuts[u].event < 0) first.assign(1, -1ll);
+      if (cuts[u].event < 0) first.assign(1, prefix.last);
       else rwkv_event_prime(sched->events[cuts[u].event], ids_host, a, cur, V, ev_off[cuts[u].event], first);
       units.emplace_back();
       build_unit(units.back(), first, ids_host + cur, (size_t)(end - cur), V, cur, [&](size_t j) { return (long long)(cur + j); });
@@ -336,7 +410,7 @@ int rwkv_encode_bounds(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
   o.hi = hi_dev;
   o.ent = ent_dev;
   o.digest = m->digest_host != nullptr;  // (encode_core reserved the buffers: digest_begin)
-  return rwkv_run_units(m, units, ids_dev, extra_dev, sched->bos, o, sched->max_batch_tokens, st);
+  return rwkv_run_units(m, units, ids_dev, extra_dev, sched->bos, o, sched->max_batch_tokens, st, &prefix);
 }
 
 // ---- paired XE scan (main.rs:1753-1787) ---------------------------------------------------------------------------------------
@@ -471,10 +545,13 @@ int rwkv_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, si
   // goes in slabs of at most max_rows rows (the encoder's bound), the state carried from slab to slab, so the workspace does not
   // grow with the history; any split gives the same logits bit for bit (DESIGN §3).
   const size_t max_rows = sched->max_batch_tokens ? sched->max_batch_tokens : kSlabRows, Tw = std::max<size_t>(1, max_rows / S);
+  // with a dictionary, the streams start from the state it leaves (rwkv_prefix: `first` is then its last in-vocabulary symbol)
+  const RwPrefix prefix = rwkv_prefix(m, sched->bos);
   auto prime_all = [&](const std::vector<uint32_t> &first) -> int {
     const size_t n = first.size();
     CZ_CUDA_TRY(cudaMemcpyAsync(d_active, ones.data(), S * 4, cudaMemcpyHostToDevice, st));
     CZ_TRY(rwkv_state_reset(m, m->rstate, S, st));
+    CZ_TRY(rwkv_prefix_state(m, m->rstate, prefix, S, max_rows, st));
     for (size_t k0 = 0; k0 < n; k0 += Tw) {
       const size_t T = std::min(Tw, n - k0), R = (size_t)S * T;
       CZ_TRY(ensure_workspace(m, R, S, 0));
@@ -552,7 +629,7 @@ int rwkv_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, si
   uint64_t n_host = 0;
   for (size_t u = 0; u < cut.size(); u++) {
     const uint64_t c0 = cut[u].begin, c1 = u + 1 < cut.size() ? cut[u + 1].begin : max_len;
-    first.assign(1, sched->bos);
+    first.assign(1, prefix.last == -1 ? sched->bos : m->dictionary[(size_t)(-2 - prefix.last)]);
     if (cut[u].event >= 0) {
       const cz_prime_event &ev = sched->events[cut[u].event];
       if (ev.hist_take && n_host < c0) {  // the history tail needs what has been decoded so far on the host: one copy per event

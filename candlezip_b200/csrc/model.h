@@ -134,6 +134,8 @@ struct cz_model {
   uint32_t *cl_lo_host = nullptr, *cl_hi_host = nullptr;
   double *cl_ent_host = nullptr;
   size_t cl_cap = 0;
+  // cz_model_set_dictionary: every segment of cz_encode / cz_encode_dev / cz_decode is coded as if it followed these symbols
+  std::vector<uint32_t> dictionary;
 };
 
 namespace cz {

@@ -553,6 +553,18 @@ int cz_model_set_code_length_out(cz_model *m, uint32_t *c_lo_out, uint32_t *c_hi
   m->cl_cap = any ? cap_tokens : 0;
   return CZ_OK;
 }
+int cz_model_set_dictionary(cz_model *m, const uint32_t *symbols, size_t n) {
+  if (!m || (n && !symbols)) return CZ_ERR_INVALID;
+  const uint32_t limit = (uint32_t)m->cfg.vocab + (m->cfg.arch == CZ_ARCH_RWKV7 ? 256u : 0u);  // the coded alphabet
+  for (size_t i = 0; i < n; i++)
+    if (symbols[i] >= limit) {
+      set_error("dictionary: symbol " + std::to_string(symbols[i]) + " at index " + std::to_string(i) + " is out of range (< " +
+                std::to_string(limit) + ")");
+      return CZ_ERR_SYMBOL_RANGE;
+    }
+  m->dictionary.assign(symbols, symbols + n);
+  return CZ_OK;
+}
 int cz_model_tensor_count(const cz_model *m) { return m ? (int)m->tensors.size() : 0; }
 int cz_model_tensor_info(const cz_model *m, int idx, const char **name, size_t *n_elems) {
   if (!m || idx < 0 || idx >= (int)m->tensors.size()) return CZ_ERR_INVALID;

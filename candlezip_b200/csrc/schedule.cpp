@@ -65,12 +65,30 @@ void build_chunks(uint64_t n_tokens, uint32_t context, uint32_t reprime_interval
   if (cur.n_coded > 0) out.push_back(cur);
 }
 
+void build_chunks_prefixed(uint64_t n_tokens, uint64_t n_prefix, uint32_t context, uint32_t reprime_interval, std::vector<Chunk> &out) {
+  build_chunks(n_prefix + n_tokens, context, reprime_interval, nullptr, 0, out);
+  size_t k = 0;
+  for (const Chunk &c : out) {
+    if (c.first + c.n_coded <= n_prefix) continue;  // wholly inside the prefix: the next reprime discards its state
+    Chunk d = c;
+    if (d.first < n_prefix) {  // the chunk in which the prefix ends: its prefix positions join the prime
+      const uint64_t skip = n_prefix - d.first;
+      d.prime_len += (uint32_t)skip;
+      d.n_coded -= (uint32_t)skip;
+      d.first = n_prefix;
+    }
+    d.first -= n_prefix;
+    out[k++] = d;
+  }
+  out.resize(k);
+}
+
 }  // namespace cz
 
-extern "C" size_t cz_schedule_chunks(uint64_t n_tokens, uint32_t context, uint32_t reprime_interval, uint64_t *first,
-                                     uint32_t *n_coded, uint64_t *prime_start, uint32_t *prime_len, size_t cap) {
+extern "C" size_t cz_schedule_chunks_prefixed(uint64_t n_tokens, uint64_t n_prefix, uint32_t context, uint32_t reprime_interval,
+                                              uint64_t *first, uint32_t *n_coded, uint64_t *prime_start, uint32_t *prime_len, size_t cap) {
   std::vector<cz::Chunk> chunks;
-  cz::build_chunks(n_tokens, context, reprime_interval, nullptr, 0, chunks);
+  cz::build_chunks_prefixed(n_tokens, n_prefix, context, reprime_interval, chunks);
   for (size_t c = 0; c < chunks.size() && c < cap; c++) {
     if (first) first[c] = chunks[c].first;
     if (n_coded) n_coded[c] = chunks[c].n_coded;
@@ -78,4 +96,9 @@ extern "C" size_t cz_schedule_chunks(uint64_t n_tokens, uint32_t context, uint32
     if (prime_len) prime_len[c] = chunks[c].prime_len;
   }
   return chunks.size();
+}
+
+extern "C" size_t cz_schedule_chunks(uint64_t n_tokens, uint32_t context, uint32_t reprime_interval, uint64_t *first,
+                                     uint32_t *n_coded, uint64_t *prime_start, uint32_t *prime_len, size_t cap) {
+  return cz_schedule_chunks_prefixed(n_tokens, 0, context, reprime_interval, first, n_coded, prime_start, prime_len, cap);
 }

@@ -19,5 +19,9 @@ struct Chunk {
 
 void build_chunks(uint64_t n_tokens, uint32_t context, uint32_t reprime_interval, const cz_prime_event *events,
                   uint32_t n_events, std::vector<Chunk> &out);
+// The chunks of the last n_tokens of a segment S = [bos, p_0 .. p_{n_prefix-1}, t_0 .. t_{n-1}] whose first n_prefix coded
+// positions are a dictionary that is never coded: build_chunks over n_prefix + n_tokens, chunks wholly inside the prefix dropped, the
+// prefix positions of the chunk in which the prefix ends moved into its prime.  `first` counts from t_0; `prime_start` indexes S.
+void build_chunks_prefixed(uint64_t n_tokens, uint64_t n_prefix, uint32_t context, uint32_t reprime_interval, std::vector<Chunk> &out);
 
 }  // namespace cz

@@ -256,6 +256,19 @@ int cz_model_set_zero_width_out(cz_model *m, uint64_t *first_zw_out, size_t cap_
  * the session shim and cz_chunk_logits are unaffected. */
 int cz_model_set_code_length_out(cz_model *m, uint32_t *c_lo_out, uint32_t *c_hi_out, double *entropy_out, size_t cap_tokens);
 
+/* Preset dictionary.  With symbols D set (n > 0), cz_encode / cz_encode_dev / cz_decode code every segment g, coded tokens T_g, exactly
+ * as they would code the token list D ++ T_g without a dictionary, except that the first n positions are not sent to the coder: the
+ * intervals of T_g are, bit for bit, the last |T_g| intervals of a dictionary-less encode of D ++ T_g (BOS first, the reprime schedule
+ * counted from the start of D, RWKV-7's literal escapes not stepping the model).  The stream must be decoded with the same dictionary.
+ * SmolLM runs only the reprime chunk in which D ends and the chunks after it (at most one extra chunk of teacher-forced rows per
+ * segment; that chunk's prime must fit max sequence length, else CZ_ERR_UNSUPPORTED); its decoder primes that chunk once for all
+ * streams and copies the K/V rows.  RWKV-7 runs D once per call and copies the resulting state to every stream.
+ * The symbols are copied and validated against the coded alphabet (CZ_ERR_SYMBOL_RANGE names the index).  NULL / 0 clears it (the
+ * default when the model is created; every call then launches what it launches without this function).  A schedule with hint-prime
+ * events is CZ_ERR_UNSUPPORTED while a dictionary is set.  cz_xe_bits, the session shim and cz_chunk_logits are unaffected; the
+ * digest, code-length, zero-width sinks and the pdf floor work unchanged, indexed by global coded index. */
+int cz_model_set_dictionary(cz_model *m, const uint32_t *symbols, size_t n);
+
 typedef struct {
   const uint32_t *prime;     /* tail(history, 511-|hint|) ++ hint, built by the caller or cz_xe_make_prime */
   uint32_t prime_len;
@@ -294,6 +307,9 @@ typedef struct {
 #define CZ_FLAG_PDF_FLOOR (1u << 10) /* extension: the payload was coded with the floored SmolLM pdf (CZ_CDF_SMOLLM_FLOOR,
                                         cz_model_set_pdf_floor).  Written by compress(on_zero_width="floor") when the unfloored pdf
                                         meets a zero-width symbol; never together with CZ_FLAG_STORED, never on RWKV-7 */
+#define CZ_FLAG_DICTIONARY (1u << 11) /* extension: the payload was coded with a preset dictionary (cz_model_set_dictionary); a "DIC1"
+                                         section names it, after the SEG1 table (or where it would be) and before the payloads.
+                                         Never together with CZ_FLAG_STORED */
 
 size_t cz_container_header_size(const cz_header_v2 *h);
 /* writes header (+repr); returns bytes written or 0 if cap is too small */
@@ -309,6 +325,9 @@ size_t cz_container_write_segments(uint8_t *buf, size_t cap, int engine, const u
                                    const uint64_t *seg_bytes, size_t n);
 size_t cz_container_read_segments(const uint8_t *buf, size_t len, int *engine, uint64_t *seg_tokens,
                                   uint64_t *seg_bytes, size_t cap, size_t *n);
+/* dictionary section: "DIC1" varint n_symbols, then the BLAKE3-128 of the symbols as little-endian u32 (16 bytes) */
+size_t cz_container_write_dictionary(uint8_t *buf, size_t cap, uint64_t n_symbols, const uint8_t hash16[16]);
+size_t cz_container_read_dictionary(const uint8_t *buf, size_t len, uint64_t *n_symbols, uint8_t hash16[16]);
 uint32_t cz_flags_pack(int agent_used, int agent_mock, int gates_present, uint32_t agent_chunk);
 /* BLAKE3-128 of a buffer (src/main.rs:901-920 use blake3 truncated to 16 bytes) */
 void cz_blake3_16(const uint8_t *data, size_t len, uint8_t out16[16]);
@@ -320,6 +339,11 @@ void cz_blake3_16(const uint8_t *data, size_t len, uint8_t out16[16]);
  * segment's token list incl. BOS at 0), prime length. */
 size_t cz_schedule_chunks(uint64_t n_tokens, uint32_t context, uint32_t reprime_interval, uint64_t *first,
                           uint32_t *n_coded, uint64_t *prime_start, uint32_t *prime_len, size_t cap);
+/* The same under a dictionary of n_prefix symbols (cz_model_set_dictionary): the chunks of cz_schedule_chunks(n_prefix + n_tokens)
+ * that code at least one of the n_tokens, first counted from the first of them, and the prefix positions of the chunk in which the
+ * dictionary ends added to its prime.  prime_start indexes the list BOS ++ dictionary ++ tokens. */
+size_t cz_schedule_chunks_prefixed(uint64_t n_tokens, uint64_t n_prefix, uint32_t context, uint32_t reprime_interval, uint64_t *first,
+                                   uint32_t *n_coded, uint64_t *prime_start, uint32_t *prime_len, size_t cap);
 
 /* ---------------------------------------------------------------- test hooks (not part of the drop-in surface) */
 /* one dense contraction C[M,N] (+)= A[M,K] B[N,K]^T through the chosen engine on host buffers; epi: 0 store f32,
