@@ -13,6 +13,8 @@ analyze INPUT [OUTPUT]: per-token code lengths, coding-distribution entropies an
 --pdf-floor (analyze, SmolLM only) codes with the floored pdf.
 --dictionary FILE (every command but the gate replay): code each segment as if it followed FILE's contents (a preset dictionary, never
 stored in the container); decompress needs the same FILE.
+--match-order K (compress, self-test, compress-many; not with the gate replay or analyze): code with the match model of order K (1..16),
+which predicts a token that repeats an earlier context of its segment; the container records K.
 """
 import argparse
 import json
@@ -114,7 +116,7 @@ def _main_many(args, ap):
     t0 = time.perf_counter()
     if args.command == "compress-many":
         res = codec.compress_many(model, datas, tok, args.segments, context=args.context, reprime_interval=args.reprime_interval,
-                                  on_zero_width=args.on_zero_width or "stored", dictionary=args.dictionary_bytes)
+                                  on_zero_width=args.on_zero_width or "stored", dictionary=args.dictionary_bytes, match_order=args.match_order)
     else:
         res = codec.decompress_many(model, datas, tok, max_streams=args.max_streams, dictionary=args.dictionary_bytes)
     dt = time.perf_counter() - t0
@@ -181,6 +183,8 @@ def main(argv=None):
     ap.add_argument("--pdf-floor", action="store_true", help="analyze: code with the floored SmolLM pdf (no token is zero-width)")
     ap.add_argument("--dictionary", metavar="FILE", help="preset dictionary: code every segment as if it followed FILE's contents; "
                                                          "decompressing needs the same FILE")
+    ap.add_argument("--match-order", type=int, metavar="K", help="compress / self-test / compress-many: code with the match model of order "
+                                                                   "K (1..16); the container records it")
     args = ap.parse_args(argv)
     if args.dictionary and args.reuse_scan_dir:
         ap.error("--dictionary is not available with --reuse-scan-dir (gated hint primes and a dictionary do not combine)")
@@ -189,6 +193,14 @@ def main(argv=None):
         ap.error("--segments and --on-zero-width are compress settings: a container carries its own (decompress-many)")
     if args.command != "decompress-many" and args.max_streams is not None:
         ap.error("--max-streams applies to decompress-many only")
+    if args.match_order is not None:
+        if args.command not in ("compress", "self-test", "compress-many"):
+            ap.error(f"--match-order is a compress setting (compress, self-test, compress-many), not available with {args.command}")
+        if args.reuse_scan_dir:
+            ap.error("--match-order is not available with --reuse-scan-dir (gated hint primes and the match model do not combine)")
+        if not 1 <= args.match_order <= 16:
+            ap.error("--match-order must be in [1, 16]")
+    args.match_order = args.match_order or 0
     if args.pdf_floor and (args.command != "analyze" or args.backend != "smollm"):
         ap.error("--pdf-floor applies to analyze on the SmolLM backend only (RWKV-7 codes with a floored alphabet already)")
     if args.command == "analyze":
@@ -225,7 +237,7 @@ def main(argv=None):
     if args.command == "compress":
         blob = _scan_compress(model, tok, data, args) if scan else \
             codec.compress(model, data, tok, args.segments, context=args.context, reprime_interval=args.reprime_interval,
-                           on_zero_width=args.on_zero_width or "stored", dictionary=args.dictionary_bytes)
+                           on_zero_width=args.on_zero_width or "stored", dictionary=args.dictionary_bytes, match_order=args.match_order)
         open(args.output or args.input + ".canz", "wb").write(blob)
         print(f"{len(data)} -> {len(blob)} bytes ({8 * len(blob) / max(1, len(data)):.4f} bits/byte)")
     elif args.command == "decompress":
@@ -236,7 +248,7 @@ def main(argv=None):
         t0 = time.perf_counter()
         blob = _scan_compress(model, tok, data, args) if scan else \
             codec.compress(model, data, tok, args.segments, context=args.context, reprime_interval=args.reprime_interval,
-                           on_zero_width=args.on_zero_width or "stored", dictionary=args.dictionary_bytes)
+                           on_zero_width=args.on_zero_width or "stored", dictionary=args.dictionary_bytes, match_order=args.match_order)
         t1 = time.perf_counter()
         out = _scan_decompress(model, tok, blob, args) if scan else codec.decompress(model, blob, tok, dictionary=args.dictionary_bytes)
         t2 = time.perf_counter()

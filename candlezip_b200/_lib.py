@@ -30,6 +30,8 @@ CZ_FLAG_SEGMENTS = 1 << 8
 CZ_FLAG_STORED = 1 << 9
 CZ_FLAG_PDF_FLOOR = 1 << 10
 CZ_FLAG_DICTIONARY = 1 << 11
+CZ_FLAG_MATCH = 1 << 12
+MATCH_NONE = 2 ** 32 - 1  # cz_model_set_match_out: the token had no prediction
 NO_ZERO_WIDTH = 2 ** 64 - 1  # cz_model_set_zero_width_out: the segment has no zero-width token
 K_FAMILIES = ("gemm_qkv", "attn", "elemwise", "cdf", "coder", "other", "gemm_o", "gemm_gu", "gemm_down", "gemm_head", "cdf_prefix")
 
@@ -133,6 +135,8 @@ SIGNATURES = {
     "cz_model_set_zero_width_out": (C.c_int, [_vp, u64p, C.c_size_t]),
     "cz_model_set_code_length_out": (C.c_int, [_vp, u32p, u32p, f64p, C.c_size_t]),
     "cz_model_set_dictionary": (C.c_int, [_vp, u32p, C.c_size_t]),
+    "cz_model_set_match": (C.c_int, [_vp, C.c_uint32]),
+    "cz_model_set_match_out": (C.c_int, [_vp, u32p, u32p, C.c_size_t]),
     "cz_xe_bits": (C.c_int, [_vp, C.POINTER(XeJob), C.c_size_t, f64p]),
     "cz_chunk_logits": (C.c_int, [_vp, u32p, C.c_size_t, u32p, C.c_size_t, f32p]),
     "cz_container_header_size": (C.c_size_t, [C.POINTER(HeaderV2)]),
@@ -144,6 +148,8 @@ SIGNATURES = {
     "cz_container_read_segments": (C.c_size_t, [u8p, C.c_size_t, C.POINTER(C.c_int), u64p, u64p, C.c_size_t, szp]),
     "cz_container_write_dictionary": (C.c_size_t, [u8p, C.c_size_t, C.c_uint64, u8p]),
     "cz_container_read_dictionary": (C.c_size_t, [u8p, C.c_size_t, u64p, u8p]),
+    "cz_container_write_match": (C.c_size_t, [u8p, C.c_size_t, C.c_uint32]),
+    "cz_container_read_match": (C.c_size_t, [u8p, C.c_size_t, u32p]),
     "cz_flags_pack": (C.c_uint32, [C.c_int, C.c_int, C.c_int, C.c_uint32]),
     "cz_blake3_16": (None, [u8p, C.c_size_t, u8p]),
     "cz_test_gemm": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_uint16), C.POINTER(C.c_uint16), C.c_int, C.c_int, _vp,

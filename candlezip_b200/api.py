@@ -274,6 +274,23 @@ class Model:
         a, p = _u32(symbols)
         check(lib.cz_model_set_dictionary(self._h, p, a.shape[0]))
 
+    def set_match(self, order):
+        """code the following encode / decode calls with the match model of order `order` (1..16; 0 is off): cz_model_set_match"""
+        check(lib.cz_model_set_match(self._h, int(order)))
+
+    def watch_match(self, n_tokens):
+        """The match model's per-token report (cz_model_set_match_out): returns (pred, w), uint32 arrays [n_tokens] that the next encode /
+        decode calls with the match model on fill with each coded token's prediction (_lib.MATCH_NONE if none) and flag weight W (0 if
+        none); watch_match(0) switches it off."""
+        if not n_tokens:
+            check(lib.cz_model_set_match_out(self._h, None, None, 0))
+            self._match_out = None
+            return None
+        self._match_out = (np.zeros(n_tokens, np.uint32), np.zeros(n_tokens, np.uint32))
+        check(lib.cz_model_set_match_out(self._h, self._match_out[0].ctypes.data_as(_lib.u32p), self._match_out[1].ctypes.data_as(_lib.u32p),
+                                         n_tokens))
+        return self._match_out
+
     def _with_dictionary(self, dictionary, call):
         """call() with the dictionary set, cleared again afterwards (no dictionary: nothing is set)"""
         if dictionary is None:
@@ -285,19 +302,21 @@ class Model:
             self.set_dictionary(None)
 
     def encode(self, ids, n_segments=1, bos=0, context=512, reprime_interval=512, events=None, seg_start=None, max_batch_tokens=0,
-               pdf_floor=False, zero_width_out=False, dictionary=None):
+               pdf_floor=False, zero_width_out=False, dictionary=None, match_order=0):
         """ids: coded tokens (no BOS). Returns (list of per-segment payload bytes, seg_start).
         pdf_floor: code with softmax_pdf_floor (no token is zero-width); the stream must be decoded with pdf_floor=True too.
         zero_width_out: a zero-width token does not raise CZ_ERR_ZERO_WIDTH; returns (payloads, seg_start, first_zw) instead, first_zw
         a uint64 array with each segment's segment-relative index of its first zero-width token or _lib.NO_ZERO_WIDTH (a segment with
         an index has an unspecified payload: cz_model_set_zero_width_out).
-        dictionary: symbols every segment is coded as if it followed (cz_model_set_dictionary); decode with the same ones."""
+        dictionary: symbols every segment is coded as if it followed (cz_model_set_dictionary); decode with the same ones.
+        match_order: the match model's order K (1..16; 0 is off: cz_model_set_match); decode with the same order."""
         self.set_pdf_floor(pdf_floor)
+        self.set_match(match_order)
         a, p = _u32(ids)
         n = a.shape[0]
         seg_start = split_segments(n, n_segments) if seg_start is None else np.asarray(seg_start, np.uint64)
         s, keep = self._schedule(n, seg_start, bos, context, reprime_interval, events, max_batch_tokens)
-        cap = 4 * n + 8 * int(s.n_segments) + 16
+        cap = (8 if match_order else 4) * n + 8 * int(s.n_segments) + 16  # (a token codes a flag and a model interval at most)
         data = np.empty(cap, np.uint8)
         seg_off = np.zeros(int(s.n_segments) + 1, np.uint64)
         bs = _lib.Bitstreams(data.ctypes.data_as(_lib.u8p), cap, seg_off.ctypes.data_as(_lib.u64p))
@@ -342,6 +361,7 @@ class Model:
             if seg_start.ndim != 1 or seg_start.shape[0] < 2 or int(seg_start[0]) != 0 or int(seg_start[-1]) != n or np.any(np.diff(seg_start.astype(np.int64)) < 0):
                 raise ValueError(f"seg_start must run from 0 to len(ids) = {n}, non-decreasing")
         self.set_pdf_floor(pdf_floor)
+        self.set_match(0)  # analyze codes without the match model
         s, keep = self._schedule(n, seg_start, bos, context, reprime_interval, None, max_batch_tokens)
         n_seg = int(s.n_segments)
         cap = 4 * n + 8 * n_seg + 16
@@ -364,10 +384,11 @@ class Model:
                     entropy=ent)
 
     def decode(self, payloads, seg_start, bos=0, context=512, reprime_interval=512, max_batch_tokens=0, events=None, pdf_floor=False,
-               dictionary=None):
+               dictionary=None, match_order=0):
         """events: the same gated hint primes the encoder was given (src/main.rs:2586-2614), single segment only;
-        pdf_floor, dictionary: the settings the stream was encoded with"""
+        pdf_floor, dictionary, match_order: the settings the stream was encoded with"""
         self.set_pdf_floor(pdf_floor)
+        self.set_match(match_order)
         seg_start = np.asarray(seg_start, np.uint64)
         n = int(seg_start[-1])
         s, keep = self._schedule(n, seg_start, bos, context, reprime_interval, events, max_batch_tokens)

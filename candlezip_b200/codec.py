@@ -15,6 +15,10 @@
 dictionary= (bytes, every entry point): a preset dictionary.  Each segment is coded as if it followed the dictionary's symbols
 (cz_model_set_dictionary), which are never stored: the container records their count and BLAKE3-128 (DIC1), and decoding needs the same
 dictionary.  Small files, which are all cold start, gain the most.
+
+match_order= (compress / compress_many): the match model of that order K (1..16; cz_model_set_match).  A token whose last K symbols repeat
+an earlier context of its segment is predicted to be the symbol that followed there, and the prediction is coded as a flag in front of
+the model's interval; a right prediction costs a fraction of a bit.  The container records K (MAT1); decompress reads it from there.
 """
 import json
 import sys
@@ -120,6 +124,16 @@ def _dict_kw(d):
     return {} if d is None else dict(dictionary=d)
 
 
+def _match_kw(order):
+    """keyword arguments of a Model call: only with the match model on, so that models without the keyword work as before"""
+    return dict(match_order=int(order)) if order else {}
+
+
+def _check_match_order(order):
+    if not isinstance(order, (int, np.integer)) or not 0 <= int(order) <= 16:
+        raise ValueError(f"match_order must be an integer in [0, 16] (0: off), not {order!r}")
+
+
 def header_fields(model, data: bytes, n_tokens, bos, context, reprime_interval, model_hash16, tokenizer_hash16):
     return dict(bos_token_id=bos, token_count=n_tokens, orig_len_bytes=len(data), model_hash16=model_hash16,
                 tokenizer_hash16=tokenizer_hash16, orig_hash16=container.blake3_16(data), context_window=context,
@@ -130,27 +144,31 @@ def stored_container(fields, model_repr, data: bytes) -> bytes:
     return container.write_container(dict(fields, reserved_flags=_lib.CZ_FLAG_STORED), model_repr, [bytes(data)])
 
 
-def coded_container(model, fields, model_repr, pays, seg, dictionary=None) -> bytes:
-    """one payload: the reference's v2 layout; several: the SEG1 table; a dictionary (its symbols): the DIC1 section"""
+def coded_container(model, fields, model_repr, pays, seg, dictionary=None, match_order=0) -> bytes:
+    """one payload: the reference's v2 layout; several: the SEG1 table; a dictionary (its symbols): the DIC1 section; the match model:
+    the MAT1 section"""
     seg_tokens = np.diff(seg) if len(pays) > 1 else None
     return container.write_container(fields, model_repr, pays, seg_tokens=seg_tokens, engine=model.engine,
-                                     dictionary=None if dictionary is None else container.dictionary_id(dictionary))
+                                     dictionary=None if dictionary is None else container.dictionary_id(dictionary), match_order=match_order)
 
 
 def compress(model, data: bytes, tokenizer=None, n_segments=1, bos=0, context=512, reprime_interval=512, model_repr=b"model.safetensors",
-             model_hash16=b"\0" * 16, tokenizer_hash16=b"\0" * 16, on_zero_width="stored", dictionary=None):
+             model_hash16=b"\0" * 16, tokenizer_hash16=b"\0" * 16, on_zero_width="stored", dictionary=None, match_order=0):
     """bytes -> .canz container bytes.  n_segments == 1 gives the reference's v2 layout (header | payload).
     on_zero_width: what to do when the SmolLM coder meets a token it cannot code (CZ_ERR_ZERO_WIDTH): "stored" writes the bytes
     uncoded (CZ_FLAG_STORED), "floor" codes the whole input again with the floored pdf (CZ_FLAG_PDF_FLOOR).  An input that codes
     without such a token gives the same container either way.  dictionary: bytes every segment is coded as if it followed (module
-    docstring); None or empty writes a container without one."""
+    docstring); None or empty writes a container without one.  match_order: the match model's order (module docstring), 0 for none; the
+    floored re-code keeps it."""
     _check_policy(on_zero_width)
+    _check_match_order(match_order)
     tokenizer = tokenizer or ByteTokenizer()
     ids = tokenize(model, data, tokenizer)
     d = dictionary_symbols(model, dictionary, tokenizer)
     fields = header_fields(model, data, len(ids), bos, context, reprime_interval, model_hash16, tokenizer_hash16)
     try:
-        pays, seg = model.encode(ids, n_segments=n_segments, bos=bos, context=context, reprime_interval=reprime_interval, **_dict_kw(d))
+        pays, seg = model.encode(ids, n_segments=n_segments, bos=bos, context=context, reprime_interval=reprime_interval, **_dict_kw(d),
+                                 **_match_kw(match_order))
     except _lib.CzError as e:
         if e.code != _lib.CZ_ERR_ZERO_WIDTH:
             raise
@@ -161,12 +179,12 @@ def compress(model, data: bytes, tokenizer=None, n_segments=1, bos=0, context=51
         if on_zero_width == "floor":
             sys.stderr.write(f"candlezip_b200: {e}; coding with the floored pdf\n")
             pays, seg = model.encode(ids, n_segments=n_segments, bos=bos, context=context, reprime_interval=reprime_interval, pdf_floor=True,
-                                     **_dict_kw(d))
+                                     **_dict_kw(d), **_match_kw(match_order))
             fields["reserved_flags"] = _lib.CZ_FLAG_PDF_FLOOR
         else:
             sys.stderr.write(f"candlezip_b200: {e}; writing a STORED container\n")
             return stored_container(fields, model_repr, data)
-    return coded_container(model, fields, model_repr, pays, seg, d)
+    return coded_container(model, fields, model_repr, pays, seg, d, match_order)
 
 
 class _Parsed:
@@ -200,7 +218,8 @@ def _parse(model, blob: bytes, verify, dictionary=None) -> _Parsed:
             raise ValueError(f"the container was coded with a dictionary of {named[0]} symbols; none was given")
         if container.dictionary_id(dictionary) != named:
             raise ValueError("the container was coded with a different dictionary than the one given")
-    key = (int(f["bos_token_id"]), int(f["context_window"]), int(f["reprime_interval"]), pdf_floor, None if named is None else named[1])
+    key = (int(f["bos_token_id"]), int(f["context_window"]), int(f["reprime_interval"]), pdf_floor, None if named is None else named[1],
+           int(f.get("match_order", 0)))
     return _Parsed(f, pays=pays, seg=seg, key=key)
 
 
@@ -226,9 +245,9 @@ def decompress(model, blob: bytes, tokenizer=None, verify=True, dictionary=None)
     p = _parse(model, blob, verify, d)
     if p.data is not None:
         return p.data
-    bos, context, reprime_interval, pdf_floor, dict_hash = p.key
+    bos, context, reprime_interval, pdf_floor, dict_hash, match_order = p.key
     ids = model.decode(p.pays, p.seg, bos=bos, context=context, reprime_interval=reprime_interval, pdf_floor=pdf_floor,
-                       **_dict_kw(None if dict_hash is None else d))
+                       **_dict_kw(None if dict_hash is None else d), **_match_kw(match_order))
     return _finish(model, tokenizer, p.f, ids, verify)
 
 
@@ -292,11 +311,12 @@ def encode_many(id_lists, n_segments, encode_fn, on_zero_width="stored"):
 
 
 def compress_many(model, datas, tokenizer=None, n_segments=1, bos=0, context=512, reprime_interval=512, model_repr=b"model.safetensors",
-                  model_hash16=b"\0" * 16, tokenizer_hash16=b"\0" * 16, on_zero_width="stored", dictionary=None):
+                  model_hash16=b"\0" * 16, tokenizer_hash16=b"\0" * 16, on_zero_width="stored", dictionary=None, match_order=0):
     """[bytes] -> [container bytes], element i equal byte for byte to compress(model, datas[i], <same arguments>).  The segments of all
     files are coded in one Model.encode call with the per-segment zero-width report on; the files that report a zero-width token get
-    the on_zero_width fallback (all "floor" files in one more call, with the same dictionary)."""
+    the on_zero_width fallback (all "floor" files in one more call, with the same dictionary and match model)."""
     _check_policy(on_zero_width)
+    _check_match_order(match_order)
     tokenizer = tokenizer or ByteTokenizer()
     id_lists = [tokenize(model, d, tokenizer) for d in datas]
     dsym = dictionary_symbols(model, dictionary, tokenizer)
@@ -304,7 +324,7 @@ def compress_many(model, datas, tokenizer=None, n_segments=1, bos=0, context=512
     def encode_fn(ids, seg_start, pdf_floor):
         # the sink is set on the floored call too: no token can be zero-width there, and encode_many checks that none was
         pays, _, first_zw = model.encode(ids, seg_start=seg_start, bos=bos, context=context, reprime_interval=reprime_interval,
-                                         pdf_floor=pdf_floor, zero_width_out=True, **_dict_kw(dsym))
+                                         pdf_floor=pdf_floor, zero_width_out=True, **_dict_kw(dsym), **_match_kw(match_order))
         return pays, first_zw
 
     out = []
@@ -316,13 +336,13 @@ def compress_many(model, datas, tokenizer=None, n_segments=1, bos=0, context=512
             continue
         if flag == _lib.CZ_FLAG_PDF_FLOOR:
             sys.stderr.write(f"candlezip_b200: file {i}: zero-width coding interval; coded with the floored pdf\n")
-        out.append(coded_container(model, dict(fields, reserved_flags=flag), model_repr, pays, loc, dsym))
+        out.append(coded_container(model, dict(fields, reserved_flags=flag), model_repr, pays, loc, dsym, match_order))
     return out
 
 
 def decode_waves(jobs, max_streams):
     """jobs[i]: None (nothing to decode) or (key, segment lengths) of file i.  Segments of files with the same key (bos, context,
-    reprime_interval, pdf_floor, dictionary hash or None) share calls; within a key they are sorted by length, longest first (stable), which is the lock-step
+    reprime_interval, pdf_floor, dictionary hash or None, match order) share calls; within a key they are sorted by length, longest first (stable), which is the lock-step
     decoder's precondition, and cut into waves of at most max_streams.  Zero-length segments decode to nothing and are left out.
     Returns [(key, [(file, segment, length)])], one entry per decode call."""
     if max_streams < 1:
@@ -371,9 +391,9 @@ def decompress_many(model, blobs, tokenizer=None, max_streams=2048, verify=True,
     jobs = [None if p.data is not None or int(p.f["token_count"]) == 0 else (p.key, np.diff(p.seg)) for p in parsed]
 
     def decode_fn(key, pays, seg_start):
-        bos, context, reprime_interval, pdf_floor, dict_hash = key
+        bos, context, reprime_interval, pdf_floor, dict_hash, match_order = key
         return model.decode(pays, seg_start, bos=bos, context=context, reprime_interval=reprime_interval, pdf_floor=pdf_floor,
-                            **_dict_kw(None if dict_hash is None else d))
+                            **_dict_kw(None if dict_hash is None else d), **_match_kw(match_order))
 
     ids = decode_many(jobs, [p.pays for p in parsed], decode_fn, max_streams)
     out = []

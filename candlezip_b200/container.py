@@ -8,6 +8,7 @@ from ._lib import lib
 
 CZ_FLAG_SEGMENTS = _lib.CZ_FLAG_SEGMENTS
 CZ_FLAG_DICTIONARY = _lib.CZ_FLAG_DICTIONARY
+CZ_FLAG_MATCH = _lib.CZ_FLAG_MATCH
 
 
 def blake3_16(data: bytes) -> bytes:
@@ -39,14 +40,22 @@ def _hdr(fields: dict, repr_len: int):
     return h
 
 
-def write_container(fields: dict, model_file_repr: bytes, payloads, seg_tokens=None, gates=None, engine=0, dictionary=None) -> bytes:
+def write_container(fields: dict, model_file_repr: bytes, payloads, seg_tokens=None, gates=None, engine=0, dictionary=None,
+                    match_order=0) -> bytes:
     """One payload and no seg_tokens -> byte-identical layout to the reference (header | [AGT2] | payload).
-    dictionary: dictionary_id() of the dictionary the payloads were coded with (CZ_FLAG_DICTIONARY + a DIC1 section), or None."""
+    dictionary: dictionary_id() of the dictionary the payloads were coded with (CZ_FLAG_DICTIONARY + a DIC1 section), or None.
+    match_order: the match model's order the payloads were coded with (CZ_FLAG_MATCH + a MAT1 section), or 0."""
     flags = fields.get("reserved_flags", 0)
     if dictionary is not None:
         if flags & _lib.CZ_FLAG_STORED:
             raise ValueError("a STORED payload is not coded: it has no dictionary")
         flags |= CZ_FLAG_DICTIONARY
+    if match_order:
+        if flags & _lib.CZ_FLAG_STORED:
+            raise ValueError("a STORED payload is not coded: it has no match model")
+        if not 1 <= int(match_order) <= 16:
+            raise ValueError(f"match order {match_order} is outside [1, 16]")
+        flags |= CZ_FLAG_MATCH
     segmented = seg_tokens is not None and len(payloads) >= 1 and not (len(payloads) == 1 and seg_tokens is None)
     if seg_tokens is not None:
         flags |= CZ_FLAG_SEGMENTS
@@ -78,6 +87,11 @@ def write_container(fields: dict, model_file_repr: bytes, payloads, seg_tokens=N
         k = lib.cz_container_write_dictionary(db, len(db), int(n_sym), (C.c_uint8 * 16)(*h16))
         assert k, "dictionary section write failed"
         out += bytes(db[:k])
+    if match_order:
+        mb = (C.c_uint8 * 16)()
+        k = lib.cz_container_write_match(mb, len(mb), int(match_order))
+        assert k, "match section write failed"
+        out += bytes(mb[:k])
     for p in payloads:
         out += p
     return bytes(out)
@@ -85,7 +99,8 @@ def write_container(fields: dict, model_file_repr: bytes, payloads, seg_tokens=N
 
 def read_container(blob: bytes):
     """Returns (fields dict, repr bytes, gates list or None, engine, seg_tokens, payload list).  A container with CZ_FLAG_DICTIONARY
-    has fields["dictionary"] = (n_symbols, BLAKE3-128 of the symbols), as dictionary_id() gives them."""
+    has fields["dictionary"] = (n_symbols, BLAKE3-128 of the symbols), as dictionary_id() gives them; one with CZ_FLAG_MATCH has
+    fields["match_order"], the order of its MAT1 section."""
     buf = (C.c_uint8 * len(blob)).from_buffer_copy(blob)
     h = _lib.HeaderV2()
     ro = C.c_size_t()
@@ -120,7 +135,7 @@ def read_container(blob: bytes):
                                        C.byref(cnt))
         n += k
         engine, seg_tokens = eng.value, st
-        n = _read_dictionary(blob, n, h, fields)
+        n = _read_match(blob, _read_dictionary(blob, n, h, fields), h, fields)
         if int(sb.sum()) != len(blob) - n:
             raise ValueError(f"segment table declares {int(sb.sum())} payload bytes but {len(blob) - n} follow it")
         if int(st.sum()) != int(h.token_count):
@@ -130,7 +145,7 @@ def read_container(blob: bytes):
             payloads.append(blob[n : n + int(b)])
             n += int(b)
     else:
-        n = _read_dictionary(blob, n, h, fields)
+        n = _read_match(blob, _read_dictionary(blob, n, h, fields), h, fields)
         payloads = [blob[n:]]
     return fields, rep, gates, engine, seg_tokens, payloads
 
@@ -148,4 +163,20 @@ def _read_dictionary(blob, n, h, fields):
     if not k:
         raise ValueError("bad dictionary section")
     fields["dictionary"] = (int(cnt.value), bytes(h16))
+    return n + k
+
+
+def _read_match(blob, n, h, fields):
+    """the MAT1 section at blob[n:] when the header has CZ_FLAG_MATCH: fills fields["match_order"], returns the offset after it.  A flag
+    without its section, a truncated section or an order outside [1, 16] raises ValueError."""
+    if not h.reserved_flags & CZ_FLAG_MATCH:
+        return n
+    if h.reserved_flags & _lib.CZ_FLAG_STORED:
+        raise ValueError("MATCH marks a coded payload: invalid with STORED")
+    sub = (C.c_uint8 * max(1, len(blob) - n)).from_buffer_copy(blob[n:] or b"\0")
+    order = C.c_uint32()
+    k = lib.cz_container_read_match(sub, len(blob) - n, C.byref(order))
+    if not k:
+        raise ValueError("bad match section")
+    fields["match_order"] = int(order.value)
     return n + k

@@ -330,4 +330,19 @@ size_t cz_container_read_dictionary(const uint8_t *buf, size_t len, uint64_t *n_
   return k + 16;
 }
 
+size_t cz_container_write_match(uint8_t *buf, size_t cap, uint32_t order) {
+  if (!buf || order < 1 || order > 16 || cap < 4 + var_len(order)) return 0;
+  memcpy(buf, "MAT1", 4);
+  return 4 + put_var(buf + 4, order);
+}
+
+size_t cz_container_read_match(const uint8_t *buf, size_t len, uint32_t *order) {
+  if (!buf || len < 5 || memcmp(buf, "MAT1", 4)) return 0;
+  uint64_t k;
+  const size_t r = get_var(buf + 4, len - 4, &k);
+  if (!r || k < 1 || k > 16) return 0;
+  if (order) *order = (uint32_t)k;
+  return 4 + r;
+}
+
 }  // extern "C"

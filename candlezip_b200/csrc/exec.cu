@@ -11,6 +11,7 @@
 
 #include "cdf_fast.cuh"
 #include "coder.cuh"
+#include "match.h"
 #include "model.h"
 #include "schedule.h"
 
@@ -68,13 +69,61 @@ __global__ void ac_decoder_init_kernel(const uint8_t *__restrict__ payload, cons
 // DS_NC = 1: two columns per warp (their add chains could fill each other's latency) measured SLOWER on B200 -- 3.18 against 2.87 ms
 // per step for the RWKV alphabet at 1,024 streams, 1.70 against 1.44 ms for SmolLM at 1,536 (253 registers, half as many warps).
 constexpr int DS_NC = 1, DS_WARPS = 8;
-template <int MODE>
+
+// Match model, decode side (match.h): after stream l (segment start s0, length len) decoded symbol `sym` at position i, count the
+// prediction it was decoded with (pred / bucket b, hit), insert position p = i + 1 under its context key and leave the prediction for p
+// in mv.next[l].  The whole warp runs it (warp-uniform: one stream per warp): lane k loads the k-th symbol of the context and compares
+// the k-th symbols before the two positions; lane 0 owns the table and counters.  t[i] is `sym` (lane 0 stores it in this same step).
+__device__ __forceinline__ void match_advance(const cz::MatchDecView &mv, int l, const uint32_t *__restrict__ t, uint64_t len, uint64_t i,
+                                              uint32_t sym, uint32_t pred, uint32_t b, bool hit) {
+  const int lane = threadIdx.x & 31;
+  const int K = (int)mv.order;
+  uint32_t *cnt = mv.cnt + (size_t)l * 32;
+  if (lane == 0 && pred != cz::kMatchNone) {
+    cnt[b] += 1;
+    cnt[16 + b] += hit ? 1u : 0u;
+  }
+  const uint64_t p = i + 1;
+  uint32_t npred = cz::kMatchNone, nw = 0, nb = 0;
+  if (p >= (uint64_t)K && p < len) {
+    const uint32_t x = lane < K ? (lane == K - 1 ? sym : t[p - K + lane]) : 0u;
+    uint32_t h = 0x811C9DC5u;
+    for (int k = 0; k < K; k++) h = (h ^ __shfl_sync(0xffffffffu, x, k)) * 0x01000193u;
+    const uint32_t key = (h * 0x9E3779B1u) >> (32 - cz::kMatchHashBits);
+    uint32_t j = 0;
+    if (lane == 0) {
+      uint32_t *slot = mv.table + ((size_t)l << cz::kMatchHashBits) + key;
+      j = *slot;
+      *slot = (uint32_t)p;
+    }
+    j = __shfl_sync(0xffffffffu, j, 0);
+    if (j != 0) {  // verify: how many symbols before j agree with those before p, up to K + NB - 1 (<= 31 lanes)
+      bool eq = false;
+      if (lane < K + cz::kMatchBuckets - 1 && (uint32_t)lane < j) eq = t[j - 1 - lane] == (lane == 0 ? sym : t[p - 1 - lane]);
+      const uint32_t run = (uint32_t)(__ffs(~__ballot_sync(0xffffffffu, eq)) - 1);
+      if (run >= (uint32_t)K) {
+        npred = j == i ? sym : t[j];
+        nb = run - (uint32_t)K;
+        if (lane == 0) {
+          uint64_t q = ((2ull * cnt[16 + nb] + 1) << 16) / (2ull * cnt[nb] + 2);
+          q = q < 1 ? 1 : (q > 65535 ? 65535 : q);
+          nw = (uint32_t)q << 14;
+        }
+      }
+    }
+  }
+  if (lane == 0) reinterpret_cast<uint4 *>(mv.next)[l] = make_uint4(npred, nw, nb, 0u);
+}
+
+template <int MODE, bool MATCH = false>
 __global__ void __launch_bounds__(DS_WARPS * 32) decode_step_kernel(const float *__restrict__ logits, int V, size_t ld, int n_lanes,
                                                                    const uint8_t *__restrict__ payload, const uint64_t *__restrict__ seg_off,
                                                                    const uint64_t *__restrict__ seg_start, uint64_t coded_index,
                                                                    AcDecoderState *__restrict__ st, uint32_t *__restrict__ ids_out,
                                                                    uint32_t *__restrict__ next_tok, int *__restrict__ err,
-                                                                   const int *__restrict__ colmax, const unsigned long long *__restrict__ ctr) {
+                                                                   const int *__restrict__ colmax, const unsigned long long *__restrict__ ctr,
+                                                                   const cz::MatchDecView mv) {
+  static_assert(!MATCH || DS_NC == 1, "the match model's branch must be warp-uniform: one stream per warp");
   if (ctr) coded_index = ctr[0];  // device-resident step counter: lets one captured CUDA graph serve every step
   __shared__ uint64_t s_tab[32 * 32];
   __shared__ __align__(16) double s_xch[DS_WARPS * DS_NC * 128];  // per warp and column: exchange lines + row ring (cdf_search_warp_n)
@@ -98,11 +147,23 @@ __global__ void __launch_bounds__(DS_WARPS * 32) decode_step_kernel(const float 
   uint32_t value[DS_NC];
   float mx[DS_NC];
   const float *col[DS_NC];
+  // match model: the flag of a stream with a prediction comes first; a hit is the predicted symbol, and no CDF search is needed
+  uint4 mnext = make_uint4(cz::kMatchNone, 0u, 0u, 0u);
+  bool mhit = false;
 #pragma unroll
   for (int c = 0; c < DS_NC; c++) {
     if (!live[c]) stream[c] = any;
     const int l = stream[c];
     d[c].resume(st[l], payload + seg_off[l], seg_off[l + 1] - seg_off[l]);
+    if constexpr (MATCH) {
+      mnext = reinterpret_cast<const uint4 *>(mv.next)[l];
+      if (mnext.x != cz::kMatchNone) {
+        mhit = d[c].peek_value() < mnext.y;
+        if (mhit) d[c].consume(0u, mnext.y);
+        else d[c].consume(mnext.y, CZ_AC_CDF_TOTAL);
+      }
+      if (mhit) continue;
+    }
     value[c] = d[c].peek_value();
     col[c] = logits + l;
     if (colmax) {
@@ -120,18 +181,30 @@ __global__ void __launch_bounds__(DS_WARPS * 32) decode_step_kernel(const float 
   }
   uint32_t sym[DS_NC], lo[DS_NC], hi[DS_NC];
   int errbits = 0;
-  cdf_search_warp_n<MODE, DS_NC>(col, ld, V, value, mx, tab, sym, lo, hi, errbits, s_xch + warp * (DS_NC * 128));
+  if (mhit) sym[0] = mnext.x;  // (only ever true with MATCH)
+  else cdf_search_warp_n<MODE, DS_NC>(col, ld, V, value, mx, tab, sym, lo, hi, errbits, s_xch + warp * (DS_NC * 128));
   if ((threadIdx.x & 31) == 0) {
     if (errbits) atomicOr(err, errbits);
 #pragma unroll
     for (int c = 0; c < DS_NC; c++) {
       if (!live[c]) continue;
       const int l = stream[c];
-      d[c].consume(lo[c], hi[c]);
+      if (!mhit) d[c].consume(lo[c], hi[c]);
       st[l] = d[c].s;
       ids_out[seg_start[l] + coded_index] = sym[c];
       next_tok[l] = sym[c];
+      if constexpr (MATCH) {
+        if (mv.pred_out) {
+          mv.pred_out[seg_start[l] + coded_index] = mnext.x;
+          mv.w_out[seg_start[l] + coded_index] = mnext.x == cz::kMatchNone ? 0u : mnext.y;
+        }
+      }
     }
+  }
+  if constexpr (MATCH) {
+    if (live[0])
+      match_advance(mv, stream[0], ids_out + seg_start[stream[0]], seg_start[stream[0] + 1] - seg_start[stream[0]], coded_index, sym[0],
+                    mnext.x, mnext.z, mhit);
   }
 }
 
@@ -223,23 +296,33 @@ int launch_decoder_init(cz_ctx *ctx, const uint8_t *payload, const uint64_t *seg
   CZ_CHECK_LAUNCH();
   return CZ_OK;
 }
+template <int MODE>
+static void decode_step_launch(cz_ctx *ctx, unsigned grid, const float *logits, int V, size_t ld, int n_lanes, const uint8_t *payload,
+                               const uint64_t *seg_off, const uint64_t *seg_start, uint64_t coded_index, czk::AcDecoderState *ds,
+                               uint32_t *ids_out, uint32_t *next_tok, const int *colmax, cudaStream_t st, const unsigned long long *ctr,
+                               const MatchDecView *mv) {
+  if (mv)
+    czk::decode_step_kernel<MODE, true><<<grid, czk::DS_WARPS * 32, 0, st>>>(logits, V, ld, n_lanes, payload, seg_off, seg_start, coded_index, ds,
+                                                                            ids_out, next_tok, ctx->err_flag_dev, colmax, ctr, *mv);
+  else
+    czk::decode_step_kernel<MODE><<<grid, czk::DS_WARPS * 32, 0, st>>>(logits, V, ld, n_lanes, payload, seg_off, seg_start, coded_index, ds,
+                                                                      ids_out, next_tok, ctx->err_flag_dev, colmax, ctr, MatchDecView());
+}
+// mv: the match model's decoder state (match_decode_begin), or nullptr when the call has no match model
 int launch_decode_step(cz_ctx *ctx, int mode, const float *logits, int V, size_t ld, int n_lanes, const uint8_t *payload,
                        const uint64_t *seg_off, const uint64_t *seg_start, uint64_t coded_index, void *decoder_state, uint32_t *ids_out,
-                       uint32_t *next_tok, const int *colmax, cudaStream_t st, const unsigned long long *ctr) {
+                       uint32_t *next_tok, const int *colmax, cudaStream_t st, const unsigned long long *ctr, const MatchDecView *mv) {
   const unsigned grid = (unsigned)ceil_div(n_lanes, czk::DS_NC * czk::DS_WARPS);
   czk::AcDecoderState *ds = (czk::AcDecoderState *)decoder_state;
   if (mode == CZ_CDF_SMOLLM)
-    CZ_LAUNCH(ctx, CZ_K_CDF,
-              (czk::decode_step_kernel<CZ_CDF_SMOLLM><<<grid, czk::DS_WARPS * 32, 0, st>>>(logits, V, ld, n_lanes, payload, seg_off, seg_start, coded_index, ds,
-                                                                            ids_out, next_tok, ctx->err_flag_dev, colmax, ctr)));
+    CZ_LAUNCH(ctx, CZ_K_CDF, (decode_step_launch<CZ_CDF_SMOLLM>(ctx, grid, logits, V, ld, n_lanes, payload, seg_off, seg_start, coded_index, ds,
+                                                                ids_out, next_tok, colmax, st, ctr, mv)));
   else if (mode == CZ_CDF_RWKV_LITERALS)
-    CZ_LAUNCH(ctx, CZ_K_CDF,
-              (czk::decode_step_kernel<CZ_CDF_RWKV_LITERALS><<<grid, czk::DS_WARPS * 32, 0, st>>>(logits, V, ld, n_lanes, payload, seg_off, seg_start, coded_index,
-                                                                                   ds, ids_out, next_tok, ctx->err_flag_dev, colmax, ctr)));
+    CZ_LAUNCH(ctx, CZ_K_CDF, (decode_step_launch<CZ_CDF_RWKV_LITERALS>(ctx, grid, logits, V, ld, n_lanes, payload, seg_off, seg_start, coded_index,
+                                                                       ds, ids_out, next_tok, colmax, st, ctr, mv)));
   else
-    CZ_LAUNCH(ctx, CZ_K_CDF,
-              (czk::decode_step_kernel<CZ_CDF_SMOLLM_FLOOR><<<grid, czk::DS_WARPS * 32, 0, st>>>(logits, V, ld, n_lanes, payload, seg_off, seg_start, coded_index,
-                                                                                  ds, ids_out, next_tok, ctx->err_flag_dev, colmax, ctr)));
+    CZ_LAUNCH(ctx, CZ_K_CDF, (decode_step_launch<CZ_CDF_SMOLLM_FLOOR>(ctx, grid, logits, V, ld, n_lanes, payload, seg_off, seg_start, coded_index,
+                                                                      ds, ids_out, next_tok, colmax, st, ctr, mv)));
   CZ_CHECK_LAUNCH();
   return CZ_OK;
 }
@@ -463,6 +546,10 @@ static int check_schedule_ids(const cz_model *m, const cz_schedule *s) {
     set_error("schedule: hint prime events are not available with a dictionary");
     return CZ_ERR_UNSUPPORTED;
   }
+  if (m->match_order && s->n_events) {
+    set_error("schedule: hint prime events are not available with the match model");
+    return CZ_ERR_UNSUPPORTED;
+  }
   for (uint32_t e = 0; e < s->n_events; e++) {
     if (s->events[e].prime_len && !s->events[e].prime) {
       set_error("schedule: prime event without tokens");
@@ -506,6 +593,10 @@ static int encode_core(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
   }
   if ((m->cl_lo_host || m->cl_hi_host || m->cl_ent_host) && m->cl_cap < n_tokens) {
     set_error("code-length sink too small: " + std::to_string(m->cl_cap) + " < " + std::to_string(n_tokens) + " tokens");
+    return CZ_ERR_INVALID;
+  }
+  if (m->match_order && (m->mo_pred_host || m->mo_w_host) && m->mo_cap < n_tokens) {
+    set_error("match-out sink too small: " + std::to_string(m->mo_cap) + " < " + std::to_string(n_tokens) + " tokens");
     return CZ_ERR_INVALID;
   }
   static const size_t env_rows = getenv("CZ_WAVE_ROWS") ? (size_t)atoll(getenv("CZ_WAVE_ROWS")) : 0;  // tuning aid
@@ -595,8 +686,10 @@ static int encode_core(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
   }
   CZ_TRY(join_cdf(m, st));
   // ---- arithmetic-coder lanes: one per segment ----
+  // (with the match model a token codes up to two intervals, the flag and the model's: at most 8 bytes)
+  const bool match = m->match_order && n_tokens;
   std::vector<uint64_t> lane_off(sched->seg_start, sched->seg_start + S + 1), raw_off(S + 1);
-  for (uint32_t g = 0; g <= S; g++) raw_off[g] = 4 * lane_off[g] + 8 * (uint64_t)g;
+  for (uint32_t g = 0; g <= S; g++) raw_off[g] = (match ? 8 : 4) * lane_off[g] + 8 * (uint64_t)g;
   CZ_TRY(d_lane.reserve((S + 1) * 8 * 5 + 64, st));
   uint64_t *d_lane_off = d_lane.as<uint64_t>(), *d_raw_off = d_lane_off + (S + 1), *d_len = d_raw_off + (S + 1),
            *d_dst_off = d_len + (S + 1);
@@ -606,8 +699,12 @@ static int encode_core(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
   CZ_CUDA_TRY(cudaMemcpyAsync(d_raw_off, raw_off.data(), (S + 1) * 8, cudaMemcpyHostToDevice, st));
   CZ_CUDA_TRY(cudaMemcpyAsync(d_eidx, &none, 8, cudaMemcpyHostToDevice, st));
   CZ_TRY(d_raw.reserve(raw_off[S] + 16, st));
-  CZ_TRY(launch_ac_encode_lanes(ctx, d_lo.as<uint32_t>(), d_hi.as<uint32_t>(), d_lane_off, S, d_raw.as<uint8_t>(), d_raw_off, d_len,
-                                d_eidx, st, d_zw));
+  const uint32_t *code_lo = d_lo.as<uint32_t>(), *code_hi = d_hi.as<uint32_t>();
+  const uint64_t *code_off = d_lane_off;
+  if (match)  // the list of flag and model intervals, and the lanes' offsets in it
+    CZ_TRY(match_encode_intervals(m, ids_dev, n_tokens, d_lane_off, S, d_lo.as<uint32_t>(), d_hi.as<uint32_t>(), st, &code_lo, &code_hi, &code_off));
+  CZ_TRY(launch_ac_encode_lanes(ctx, code_lo, code_hi, code_off, S, d_raw.as<uint8_t>(), d_raw_off, d_len, d_eidx, st, d_zw));
+  if (match) CZ_TRY(match_encode_finish(m, n_tokens, d_lane_off, S, d_zw, d_eidx, st));  // zero-width reports: list -> token indices
   std::vector<uint64_t> len(S);
   CZ_CUDA_TRY(cudaMemcpyAsync(len.data(), d_len, S * 8, cudaMemcpyDeviceToHost, st));
   // with a zero-width sink each lane reports its own first zero-width index there (its payload is left empty) instead of the call failing
@@ -632,6 +729,7 @@ static int encode_core(cz_model *m, const uint32_t *ids_dev, const uint32_t *ids
   if (n_tokens && m->cl_lo_host) CZ_CUDA_TRY(cudaMemcpyAsync(m->cl_lo_host, d_lo.p, n_tokens * 4, cudaMemcpyDeviceToHost, st));
   if (n_tokens && m->cl_hi_host) CZ_CUDA_TRY(cudaMemcpyAsync(m->cl_hi_host, d_hi.p, n_tokens * 4, cudaMemcpyDeviceToHost, st));
   if (n_tokens && ent_dev) CZ_CUDA_TRY(cudaMemcpyAsync(m->cl_ent_host, ent_dev, n_tokens * 8, cudaMemcpyDeviceToHost, st));
+  if (match) CZ_TRY(match_encode_copy_out(m, n_tokens, S, st));
   const double t_pre_sync = host_ms();
   CZ_CUDA_TRY(cudaStreamSynchronize(st));
   if (dbg)
@@ -793,7 +891,7 @@ int cz_encode(cz_model *m, const uint32_t *ids, size_t n_tokens, const cz_schedu
   GrowBuf &d_ids = m->sb[SB_IDS], &d_out = m->sb[SB_OUT];
   CZ_TRY(d_ids.reserve(n_tokens * 4 + 16, ctx->stream));
   if (n_tokens) CZ_CUDA_TRY(cudaMemcpyAsync(d_ids.p, ids, n_tokens * 4, cudaMemcpyHostToDevice, ctx->stream));
-  const size_t cap = 4 * n_tokens + 8 * (size_t)sched->n_segments + 16;
+  const size_t cap = (m->match_order ? 8 : 4) * n_tokens + 8 * (size_t)sched->n_segments + 16;
   CZ_TRY(d_out.reserve(cap, ctx->stream));
   CZ_TRY(encode_core(m, d_ids.as<uint32_t>(), ids, n_tokens, sched, d_out.as<uint8_t>(), cap, out->seg_off, out->cap));
   const uint64_t total = out->seg_off[sched->n_segments];
@@ -811,6 +909,10 @@ int cz_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, size
   CZ_TRY(check_schedule_ids(m, sched));
   CZ_TRY(model_finalize(m));
   if (n_tokens == 0) return CZ_OK;
+  if (m->match_order && (m->mo_pred_host || m->mo_w_host) && m->mo_cap < n_tokens) {
+    set_error("match-out sink too small: " + std::to_string(m->mo_cap) + " < " + std::to_string(n_tokens) + " tokens");
+    return CZ_ERR_INVALID;
+  }
   cz_ctx *ctx = m->ctx;
   cudaStream_t st = ctx->stream;
   CZ_CUDA_TRY(cudaSetDevice(ctx->device));
@@ -863,6 +965,8 @@ int cz_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, size
             (czk::ac_decoder_init_kernel<<<(unsigned)ceil_div(S, 128), 128, 0, st>>>(d_pay.as<uint8_t>(), d_off.as<uint64_t>(), (int)S,
                                                                                     d_state.as<czk::AcDecoderState>())));
   CZ_CHECK_LAUNCH();
+  MatchDecView mview;
+  if (m->match_order) CZ_TRY(match_decode_begin(m, S, n_tokens, st, &mview));
   KvView kv;
   kv.k = d_k.as<__nv_bfloat16>();
   kv.v = d_v.as<__nv_bfloat16>();
@@ -975,7 +1079,8 @@ int cz_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, size
         CZ_TRY(launch_logits_digest(ctx, d_logits.as<float>(), (size_t)c.vocab, (size_t)n_live, S_pad, m->sb[SB_CV].p,
                                     m->sb[SB_DIGEST].as<uint8_t>(), 0, nullptr, d_start.as<uint64_t>(), d_ctr, st));
       return launch_decode_step(ctx, coded_mode(m), d_logits.as<float>(), c.vocab, S_pad, n_live, d_pay.as<uint8_t>(), d_off.as<uint64_t>(),
-                                d_start.as<uint64_t>(), 0, d_state.p, d_ids.as<uint32_t>(), ws.tok, have_max ? ws.colmax : nullptr, st, d_ctr);
+                                d_start.as<uint64_t>(), 0, d_state.p, d_ids.as<uint32_t>(), ws.tok, have_max ? ws.colmax : nullptr, st, d_ctr,
+                                m->match_order ? &mview : nullptr);
     };
     auto step = [&]() -> int {
       CZ_TRY(decode_syms());
@@ -1028,6 +1133,7 @@ int cz_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, size
   }
   CZ_CUDA_TRY(cudaMemcpyAsync(ids_out, d_ids.p, n_tokens * 4, cudaMemcpyDeviceToHost, st));
   CZ_TRY(digest_end(m, n_tokens, st));
+  CZ_TRY(match_decode_end(m, n_tokens, st));
   CZ_CUDA_TRY(cudaStreamSynchronize(st));
   return CZ_OK;
 }

@@ -16,6 +16,7 @@
 
 #include "cdf_fast.cuh"
 #include "coder.cuh"
+#include "match.h"
 #include "model.h"
 
 namespace cz {
@@ -26,7 +27,7 @@ int launch_cdf_entropy(cz_ctx *ctx, int mode, const float *logits_dev, size_t V,
 int fetch_device_status(cz_ctx *ctx, unsigned long long *err_index_dev, unsigned long long *err_index_out);
 int launch_decode_step(cz_ctx *ctx, int mode, const float *logits, int V, size_t ld, int n_lanes, const uint8_t *payload,
                        const uint64_t *seg_off, const uint64_t *seg_start, uint64_t coded_index, void *decoder_state, uint32_t *ids_out,
-                       uint32_t *next_tok, const int *colmax, cudaStream_t st, const unsigned long long *ctr = nullptr);
+                       uint32_t *next_tok, const int *colmax, cudaStream_t st, const unsigned long long *ctr, const MatchDecView *mv);
 int launch_decoder_init(cz_ctx *ctx, const uint8_t *payload, const uint64_t *seg_off, int n_lanes, void *decoder_state, cudaStream_t st);
 size_t decoder_state_bytes();
 int launch_set_ctr(cz_ctx *ctx, unsigned long long *ctr, unsigned long long a, unsigned long long b, cudaStream_t st);
@@ -520,6 +521,8 @@ int rwkv_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, si
   CZ_CUDA_TRY(cudaMemcpyAsync(d_off.p, seg_off, (S + 1) * 8, cudaMemcpyHostToDevice, st));
   CZ_CUDA_TRY(cudaMemcpyAsync(d_start.p, sched->seg_start, (S + 1) * 8, cudaMemcpyHostToDevice, st));
   CZ_TRY(launch_decoder_init(ctx, d_pay.as<uint8_t>(), d_off.as<uint64_t>(), (int)S, d_state.p, st));
+  MatchDecView mview;  // the match model's per-stream state: literal escapes are ordinary symbols to it (a hit on one steps nothing)
+  if (m->match_order) CZ_TRY(match_decode_begin(m, S, n_tokens, st, &mview));
   const bool use_cm = c.engine == CZ_ENGINE_TCGEN05 && getenv("CZ_DEBUG_NO_COLMAX") == nullptr;
   const bool use_graph = getenv("CZ_DECODE_NO_GRAPH") == nullptr;
   unsigned long long *d_ctr = (unsigned long long *)(((uintptr_t)(d_sym + S) + 15) & ~(uintptr_t)15);  // aligned tail of d_meta
@@ -600,7 +603,7 @@ int rwkv_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, si
                                   d_start.as<uint64_t>(), d_ctr, st));
     return launch_decode_step(ctx, CZ_CDF_RWKV_LITERALS, d_keep.as<float>(), (int)V, S_pad, (int)S, d_pay.as<uint8_t>(), d_off.as<uint64_t>(),
                               d_start.as<uint64_t>(), 0, d_state.p, d_ids.as<uint32_t>(), (uint32_t *)d_sym, use_cm ? d_cm_keep : nullptr, st,
-                              d_ctr);
+                              d_ctr, m->match_order ? &mview : nullptr);
   };
   // one step = decode a symbol per stream, decide which streams step (literals do not), single-token forward, commit the new
   // logits columns.  The step-varying scalar (coded index) lives in d_ctr, so the launch sequence is captured once into a CUDA
@@ -685,6 +688,7 @@ int rwkv_decode(cz_model *m, const uint8_t *payload, const uint64_t *seg_off, si
   CZ_TRY(fetch_device_status(ctx, nullptr, nullptr));
   CZ_CUDA_TRY(cudaMemcpyAsync(ids_out, d_ids.p, n_tokens * 4, cudaMemcpyDeviceToHost, st));
   CZ_TRY(digest_end(m, n_tokens, st));
+  CZ_TRY(match_decode_end(m, n_tokens, st));
   CZ_CUDA_TRY(cudaStreamSynchronize(st));
   return CZ_OK;
 }

@@ -61,7 +61,7 @@ struct GrowBuf {
 };
 enum { SB_LO = 0, SB_HI, SB_SRC, SB_EXTRA, SB_LANE, SB_RAW, SB_IDS, SB_OUT, SB_PAY, SB_OFF, SB_START, SB_STATE, SB_DIDS, SB_K, SB_V,
        SB_LOGITS, SB_KVB, SB_TGT, SB_BITS, SB_JOFF, SB_XOUT, SB_RW_OIDX, SB_RW_SYMS, SB_RW_LO, SB_RW_HI, SB_RW_XE, SB_RW_FRESH,
-       SB_DIGEST, SB_CV, SB_ENT,
+       SB_DIGEST, SB_CV, SB_ENT, SB_MATCH, SB_MTEMP, SB_MDEC, SB_MOUT,
        SB_COUNT };
 
 // ---- RWKV-7 (rwkv7.cu) ----
@@ -136,6 +136,10 @@ struct cz_model {
   size_t cl_cap = 0;
   // cz_model_set_dictionary: every segment of cz_encode / cz_encode_dev / cz_decode is coded as if it followed these symbols
   std::vector<uint32_t> dictionary;
+  // cz_model_set_match: order K of the match model (0: off); cz_model_set_match_out: per-token prediction and flag weight (match.h)
+  uint32_t match_order = 0;
+  uint32_t *mo_pred_host = nullptr, *mo_w_host = nullptr;
+  size_t mo_cap = 0;
 };
 
 namespace cz {

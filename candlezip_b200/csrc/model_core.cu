@@ -565,6 +565,27 @@ int cz_model_set_dictionary(cz_model *m, const uint32_t *symbols, size_t n) {
   m->dictionary.assign(symbols, symbols + n);
   return CZ_OK;
 }
+int cz_model_set_match(cz_model *m, uint32_t order) {
+  if (!m) return CZ_ERR_INVALID;
+  if (order > 16) {
+    set_error("match model: order " + std::to_string(order) + " is outside [1, 16] (0: off)");
+    return CZ_ERR_INVALID;
+  }
+  m->match_order = order;
+  return CZ_OK;
+}
+int cz_model_set_match_out(cz_model *m, uint32_t *pred_out, uint32_t *w_out, size_t cap_tokens) {
+  const bool any = pred_out || w_out;
+  if (!m) return CZ_ERR_INVALID;
+  if (any && cap_tokens == 0) {
+    set_error("match-out sink: cap_tokens == 0 with a sink set");
+    return CZ_ERR_INVALID;
+  }
+  m->mo_pred_host = pred_out;
+  m->mo_w_host = w_out;
+  m->mo_cap = any ? cap_tokens : 0;
+  return CZ_OK;
+}
 int cz_model_tensor_count(const cz_model *m) { return m ? (int)m->tensors.size() : 0; }
 int cz_model_tensor_info(const cz_model *m, int idx, const char **name, size_t *n_elems) {
   if (!m || idx < 0 || idx >= (int)m->tensors.size()) return CZ_ERR_INVALID;

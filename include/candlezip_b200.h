@@ -269,6 +269,33 @@ int cz_model_set_code_length_out(cz_model *m, uint32_t *c_lo_out, uint32_t *c_hi
  * digest, code-length, zero-width sinks and the pdf floor work unchanged, indexed by global coded index. */
 int cz_model_set_dictionary(cz_model *m, const uint32_t *symbols, size_t n);
 
+/* Match model of order K (1..16; 0 is off, the default when the model is created).  It applies to the following cz_encode,
+ * cz_encode_dev and cz_decode calls on both architectures.  With t[0..n) the coded symbols of one segment (RWKV-7 literal escapes
+ * included; BOS and a dictionary are not: the history is the segment's own symbols), HB = 18 hash bits and NB = 16 length buckets:
+ *   key(i), i >= K      h = 0x811C9DC5; for x in t[i-K .. i-1], oldest first: h = (h ^ x) * 0x01000193 mod 2^32;
+ *                       key = (h * 0x9E3779B1 mod 2^32) >> (32 - HB)
+ *   candidate           j(i) = max{ j : K <= j < i, key(j) == key(i) } in the same segment (a table of 2^HB positions per stream)
+ *   length              len = the number of k = 0, 1, ... for which t[j-1-k] == t[i-1-k] (stopping at the first difference or at the
+ *                       segment's start), at most K + NB - 1.  len < K (a hash collision) or no candidate: no prediction.  Otherwise
+ *                       the prediction is pred = t[j], in bucket b = len - K
+ *   weight              hits_b / tries_b = right / all predictions of bucket b at earlier positions of the segment;
+ *                       p16 = clamp(((2 hits_b + 1) << 16) / (2 tries_b + 2), 1, 65535) (integer division), W = p16 << 14
+ *   intervals of t[i]   with a prediction, first the flag: [0, W) if t[i] == pred (a hit), else [W, 2^30); then the model's interval
+ *                       of t[i] unless it was a hit.
+ * A hit's model interval is never coded, so the zero-width report (CZ_ERR_ZERO_WIDTH, cz_model_set_zero_width_out) names the first
+ * non-hit token with an empty interval, by coded-token index.  cz_encode needs an output capacity of 8 bytes per token (4 without).
+ * The code-length sink still reports the model's intervals.  A schedule with hint-prime events is CZ_ERR_UNSUPPORTED while the match
+ * model is on.  cz_xe_bits, the session shim and cz_chunk_logits are unaffected; the digest, zero-width, code-length sinks, the pdf
+ * floor and the dictionary work unchanged.  A stream must be decoded with the order it was encoded with (the container's MAT1 section).
+ * Decode memory: 2^HB u32 positions per stream (1 MiB; 2 GiB at 2,048 streams), cleared at the start of each call.
+ * order > 16 is CZ_ERR_INVALID. */
+int cz_model_set_match(cz_model *m, uint32_t order);
+/* Match-out sink: with the match model on, cz_encode / cz_encode_dev and cz_decode write, per global coded index i, the prediction
+ * token i was coded with (pred_out[i], UINT32_MAX if none) and its flag weight W (w_out[i], 0 if none).  Encode and decode write the
+ * same values.  Either pointer may be NULL; both NULL (the default) is off.  The sinks are written only when the call returns CZ_OK.
+ * cap_tokens < the call's n_tokens makes the call return CZ_ERR_INVALID; a non-NULL pointer with cap_tokens == 0 is CZ_ERR_INVALID. */
+int cz_model_set_match_out(cz_model *m, uint32_t *pred_out, uint32_t *w_out, size_t cap_tokens);
+
 typedef struct {
   const uint32_t *prime;     /* tail(history, 511-|hint|) ++ hint, built by the caller or cz_xe_make_prime */
   uint32_t prime_len;
@@ -310,6 +337,9 @@ typedef struct {
 #define CZ_FLAG_DICTIONARY (1u << 11) /* extension: the payload was coded with a preset dictionary (cz_model_set_dictionary); a "DIC1"
                                          section names it, after the SEG1 table (or where it would be) and before the payloads.
                                          Never together with CZ_FLAG_STORED */
+#define CZ_FLAG_MATCH (1u << 12) /* extension: the payload was coded with the match model (cz_model_set_match); a "MAT1" section gives
+                                    its order, after the DIC1 section (or where it would be) and before the payloads.  Never together
+                                    with CZ_FLAG_STORED */
 
 size_t cz_container_header_size(const cz_header_v2 *h);
 /* writes header (+repr); returns bytes written or 0 if cap is too small */
@@ -328,6 +358,9 @@ size_t cz_container_read_segments(const uint8_t *buf, size_t len, int *engine, u
 /* dictionary section: "DIC1" varint n_symbols, then the BLAKE3-128 of the symbols as little-endian u32 (16 bytes) */
 size_t cz_container_write_dictionary(uint8_t *buf, size_t cap, uint64_t n_symbols, const uint8_t hash16[16]);
 size_t cz_container_read_dictionary(const uint8_t *buf, size_t len, uint64_t *n_symbols, uint8_t hash16[16]);
+/* match-model section: "MAT1" varint order.  The reader returns 0 for a truncated section or an order outside [1, 16] */
+size_t cz_container_write_match(uint8_t *buf, size_t cap, uint32_t order);
+size_t cz_container_read_match(const uint8_t *buf, size_t len, uint32_t *order);
 uint32_t cz_flags_pack(int agent_used, int agent_mock, int gates_present, uint32_t agent_chunk);
 /* BLAKE3-128 of a buffer (src/main.rs:901-920 use blake3 truncated to 16 bytes) */
 void cz_blake3_16(const uint8_t *data, size_t len, uint8_t out16[16]);

@@ -16,5 +16,6 @@ run tiny_simt 900 -k "tiny and simt"
 run tiny_tc 900 -k "tiny and not simt"
 run full 900 -k "full_size"
 run dictionary 900 -k "dictionary"
+run match 1200 -k "match"
 run rwkv 900 -k "(rwkv7 and not full_size) or hint_prime or gate_scan or file_level or cli_twin"
 for f in gpurun_out/*.log; do echo "---- $f"; tail -n 25 "$f"; done
