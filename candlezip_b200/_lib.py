@@ -10,6 +10,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libcandlezip_b200.so")
 
 u8p = C.POINTER(C.c_uint8)
+i32p = C.POINTER(C.c_int)
 u32p = C.POINTER(C.c_uint32)
 u64p = C.POINTER(C.c_uint64)
 f32p = C.POINTER(C.c_float)
@@ -159,6 +160,10 @@ SIGNATURES = {
                                    C.POINTER(C.c_uint16)]),
     "cz_test_attention": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_uint16), C.POINTER(C.c_uint16), C.POINTER(C.c_uint16), C.c_int,
                                    C.POINTER(C.c_uint16)]),
+    "cz_test_wkv7_scan": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.c_int, i32p, i32p, i32p, i32p, C.c_int, f32p, f32p, f32p, f32p,
+                                   C.POINTER(C.c_uint16)]),
+    "cz_test_rwkv_ln_mix": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, f32p, f32p, f32p, f32p, i32p, i32p, i32p,
+                                     f32p, f32p, C.c_float, C.POINTER(C.c_uint16), i32p]),
     "cz_test_expf_exhaustive": (C.c_int, [_vp, u64p, u64p, u64p]),
     "cz_test_div_random": (C.c_int, [_vp, C.c_uint64, C.c_uint64, u64p]),
     "cz_test_cdf_ecache_state": (C.c_int, [_vp, C.POINTER(C.c_int), u64p]),

@@ -526,13 +526,21 @@ void rwkv_free(cz_model *m) {
 // device.  in_place: T = 1 decode steps read and write the same token-shift buffers; slabs ping-pong them.
 // stream_active (device, nullable): per-stream flag for the stepwise decoder.
 
-// rwkv_ln_mix: the 8-elements-per-lane kernel when the width is a multiple of 256 (<= 1024) and every operand is 16-byte aligned
+// rwkv_ln_mix takes the 8-elements-per-lane kernel when the width is a multiple of 256 (<= 1024) and every operand is 16-byte aligned
+template <int NMIX>
+static bool ln_mix_takes_v8(int C, const float *x, const float *lnw, const float *lnb, const czk::MixMu &mu, const float *state_in,
+                            const float *state_out, const czk::MixOut &out) {
+  bool vec = C % 256 == 0 && C <= 1024 && (((uintptr_t)x | (uintptr_t)lnw | (uintptr_t)lnb | (uintptr_t)state_in | (uintptr_t)state_out) & 15) == 0;
+  for (int q = 0; q < NMIX; q++) vec = vec && (((uintptr_t)mu.p[q] | (uintptr_t)out.p[q]) & 15) == 0;
+  return vec;
+}
+
+// lane_form: run the element-per-lane kernel even where the v8 form applies (cz_test_rwkv_ln_mix compares the two)
 template <int NMIX>
 static int launch_ln_mix(cz_ctx *ctx, cudaStream_t st, unsigned grid, const float *x, const float *lnw, const float *lnb, const czk::MixMu &mu,
                          const int *prev_row, const int *slot, const int *flags, const float *state_in, float *state_out, const czk::MixOut &out,
-                         int n_rows, int C, float eps) {
-  bool vec = C % 256 == 0 && C <= 1024 && (((uintptr_t)x | (uintptr_t)lnw | (uintptr_t)lnb | (uintptr_t)state_in | (uintptr_t)state_out) & 15) == 0;
-  for (int q = 0; q < NMIX; q++) vec = vec && (((uintptr_t)mu.p[q] | (uintptr_t)out.p[q]) & 15) == 0;
+                         int n_rows, int C, float eps, bool lane_form = false) {
+  const bool vec = !lane_form && ln_mix_takes_v8<NMIX>(C, x, lnw, lnb, mu, state_in, state_out, out);
 #define CZ_LNMIX_V8(NCH)                                                                                                                       \
   CZ_LAUNCH(ctx, CZ_K_ELEMWISE,                                                                                                                \
             (czk::rwkv_ln_mix_v8_kernel<NMIX, NCH><<<grid, 128, 0, st>>>(x, lnw, lnb, mu, prev_row, slot, flags, state_in, state_out, out, n_rows, \
@@ -545,6 +553,20 @@ static int launch_ln_mix(cz_ctx *ctx, cudaStream_t st, unsigned grid, const floa
     CZ_LAUNCH(ctx, CZ_K_ELEMWISE,
               (czk::rwkv_ln_mix_kernel<NMIX><<<grid, 128, 0, st>>>(x, lnw, lnb, mu, prev_row, slot, flags, state_in, state_out, out, n_rows, C, eps)));
 #undef CZ_LNMIX_V8
+  CZ_CHECK_LAUNCH();
+  return CZ_OK;
+}
+
+// one WKV-7 scan: a warp per (stream, head); S is one layer's state [n_slots][H][4096]
+static int launch_wkv7_scan(cz_ctx *ctx, cudaStream_t st, bool layer0, const czk::WkvIo &io, const czk::WkvVecs &vc, const int *row_begin,
+                            const int *row_end, const int *stream_slot, const int *stream_active, float *S, __nv_bfloat16 *out, int n_streams,
+                            int C) {
+  const int H = C / 64;
+  const dim3 grid((unsigned)n_streams, (unsigned)H);
+  if (layer0)
+    CZ_LAUNCH(ctx, CZ_K_ATTN, (czk::wkv7_scan_kernel<true><<<grid, 32, 0, st>>>(io, vc, row_begin, row_end, stream_slot, stream_active, S, out, C, H)));
+  else
+    CZ_LAUNCH(ctx, CZ_K_ATTN, (czk::wkv7_scan_kernel<false><<<grid, 32, 0, st>>>(io, vc, row_begin, row_end, stream_slot, stream_active, S, out, C, H)));
   CZ_CHECK_LAUNCH();
   return CZ_OK;
 }
@@ -596,15 +618,8 @@ int rwkv_forward(cz_model *m, int n_rows, int n_streams, RwkvState &stt, bool in
     CZ_TRY(mm(w.lo, 128, W.g2, c.lora_g, C, w.f[6], C, EPI_STORE_F32, 192, CZ_K_GEMM));
     czk::WkvIo io{w.f[0], w.f[1], w.f[2], w.f[3], w.f[4], w.f[5], w.f[6], w.v_first};
     czk::WkvVecs vc{v + RV_W0 * C, v + RV_A0 * C, v + RV_V0 * C, v + RV_KK * C, v + RV_KA * C, v + RV_RK * C, v + RV_GNW * C, v + RV_GNB * C};
-    float *S = stt.S + (size_t)l * cap * H * 4096;
-    dim3 grid((unsigned)n_streams, (unsigned)H);
-    if (l == 0)
-      CZ_LAUNCH(ctx, CZ_K_ATTN,
-                (czk::wkv7_scan_kernel<true><<<grid, 32, 0, st>>>(io, vc, w.row_begin, w.row_end, w.stream_slot, stream_active, S, w.att, C, H)));
-    else
-      CZ_LAUNCH(ctx, CZ_K_ATTN,
-                (czk::wkv7_scan_kernel<false><<<grid, 32, 0, st>>>(io, vc, w.row_begin, w.row_end, w.stream_slot, stream_active, S, w.att, C, H)));
-    CZ_CHECK_LAUNCH();
+    CZ_TRY(launch_wkv7_scan(ctx, st, l == 0, io, vc, w.row_begin, w.row_end, w.stream_slot, stream_active, stt.S + (size_t)l * cap * H * 4096,
+                            w.att, n_streams, C));
     CZ_TRY(mm(w.att, C, W.wo, C, C, ws.x, C, EPI_ADD_F32, 192, CZ_K_GEMM_O));
     // feed-forward
     czk::MixMu mu1{};
@@ -634,3 +649,146 @@ int rwkv_final_norm_gather(cz_model *m, int n_logit, cudaStream_t st) {
 }
 
 }  // namespace cz
+
+// ---- test hooks (declared in include/candlezip_b200.h): the two RWKV-7 kernel families on host buffers, through the launchers
+// rwkv_forward uses, so tests can compare them with an f64 restatement at shapes and edges the model never produces on its own
+namespace cz {
+int require_device(cz_ctx *ctx);
+
+namespace {
+struct HookBufs {  // the device buffers of one hook call, freed on every return path
+  std::vector<void *> p;
+  ~HookBufs() {
+    for (void *q : p) cudaFree(q);
+  }
+  template <typename T>
+  int alloc(T *&out, size_t n) {
+    void *q = nullptr;
+    CZ_CUDA_TRY(cudaMalloc(&q, std::max<size_t>(n * sizeof(T), 16)));
+    p.push_back(q);
+    out = (T *)q;
+    return CZ_OK;
+  }
+};
+
+int hook_sync(cz_ctx *ctx, int rc, const char *what) {
+  if (rc != CZ_OK) return rc;
+  const cudaError_t e = cudaStreamSynchronize(ctx->stream);
+  if (e != cudaSuccess) {
+    set_error(std::string(what) + " execution failed: " + cudaGetErrorString(e));
+    return CZ_ERR_CUDA;
+  }
+  return CZ_OK;
+}
+
+template <int NMIX>
+int hook_ln_mix(cz_ctx *ctx, bool lane_form, int R, int C, const float *x, const float *lnw, const float *lnb, const float *mu,
+                const int *meta, const float *state_in, float *state_out, __nv_bfloat16 *out, float eps, int *form_used) {
+  czk::MixMu m{};
+  czk::MixOut o{};
+  for (int q = 0; q < NMIX; q++) {
+    m.p[q] = mu + (size_t)q * C;
+    o.p[q] = out + (size_t)q * R * C;
+  }
+  *form_used = !lane_form && ln_mix_takes_v8<NMIX>(C, x, lnw, lnb, m, state_in, state_out, o) ? 8 : 1;
+  return launch_ln_mix<NMIX>(ctx, ctx->stream, (unsigned)ceil_div(R, 4), x, lnw, lnb, m, meta, meta + R, meta + 2 * R, state_in, state_out, o, R,
+                             C, eps, lane_form);
+}
+}  // namespace
+}  // namespace cz
+
+extern "C" int cz_test_wkv7_scan(cz_ctx *ctx, int layer0, int R, int H, int n_streams, const int *row_begin, const int *row_end,
+                                 const int *stream_slot, const int *stream_active, int n_slots, const float *rows, float *v_first,
+                                 const float *vecs, float *state, uint16_t *out_bf16) {
+  using namespace cz;
+  CZ_TRY(require_device(ctx));
+  CZ_CUDA_TRY(cudaSetDevice(ctx->device));
+  bool ok = R > 0 && H >= 1 && H <= czk::RW_MAXC / 64 && n_streams > 0 && n_slots > 0 && row_begin && row_end && stream_slot && rows &&
+            v_first && vecs && state && out_bf16;
+  for (int s = 0; ok && s < n_streams; s++)
+    ok = row_begin[s] >= 0 && row_end[s] <= R && stream_slot[s] >= 0 && stream_slot[s] < n_slots;
+  if (!ok) {
+    set_error("cz_test_wkv7_scan: bad arguments");
+    return CZ_ERR_INVALID;
+  }
+  const int C = 64 * H;
+  const size_t RC = (size_t)R * C, SN = (size_t)n_slots * H * 4096, NS = (size_t)n_streams;
+  HookBufs d;
+  float *drows, *dvf, *dvecs, *dS;
+  __nv_bfloat16 *dout;
+  int *dmeta;
+  CZ_TRY(d.alloc(drows, 7 * RC));
+  CZ_TRY(d.alloc(dvf, RC));
+  CZ_TRY(d.alloc(dvecs, 8 * (size_t)C));
+  CZ_TRY(d.alloc(dS, SN));
+  CZ_TRY(d.alloc(dout, RC));
+  CZ_TRY(d.alloc(dmeta, 4 * NS));
+  CZ_CUDA_TRY(cudaMemcpy(drows, rows, 7 * RC * 4, cudaMemcpyHostToDevice));
+  CZ_CUDA_TRY(cudaMemcpy(dvf, v_first, RC * 4, cudaMemcpyHostToDevice));
+  CZ_CUDA_TRY(cudaMemcpy(dvecs, vecs, 8 * (size_t)C * 4, cudaMemcpyHostToDevice));
+  CZ_CUDA_TRY(cudaMemcpy(dS, state, SN * 4, cudaMemcpyHostToDevice));
+  CZ_CUDA_TRY(cudaMemcpy(dout, out_bf16, RC * 2, cudaMemcpyHostToDevice));
+  CZ_CUDA_TRY(cudaMemcpy(dmeta, row_begin, NS * 4, cudaMemcpyHostToDevice));
+  CZ_CUDA_TRY(cudaMemcpy(dmeta + NS, row_end, NS * 4, cudaMemcpyHostToDevice));
+  CZ_CUDA_TRY(cudaMemcpy(dmeta + 2 * NS, stream_slot, NS * 4, cudaMemcpyHostToDevice));
+  if (stream_active) CZ_CUDA_TRY(cudaMemcpy(dmeta + 3 * NS, stream_active, NS * 4, cudaMemcpyHostToDevice));
+  const czk::WkvIo io{drows, drows + RC, drows + 2 * RC, drows + 3 * RC, drows + 4 * RC, drows + 5 * RC, drows + 6 * RC, dvf};
+  const czk::WkvVecs vc{dvecs, dvecs + C, dvecs + 2 * C, dvecs + 3 * C, dvecs + 4 * C, dvecs + 5 * C, dvecs + 6 * C, dvecs + 7 * C};
+  CZ_TRY(hook_sync(ctx,
+                   launch_wkv7_scan(ctx, ctx->stream, layer0 != 0, io, vc, dmeta, dmeta + NS, dmeta + 2 * NS, stream_active ? dmeta + 3 * NS : nullptr,
+                                    dS, dout, n_streams, C),
+                   "wkv7 scan"));
+  CZ_CUDA_TRY(cudaMemcpy(v_first, dvf, RC * 4, cudaMemcpyDeviceToHost));
+  CZ_CUDA_TRY(cudaMemcpy(state, dS, SN * 4, cudaMemcpyDeviceToHost));
+  CZ_CUDA_TRY(cudaMemcpy(out_bf16, dout, RC * 2, cudaMemcpyDeviceToHost));
+  return CZ_OK;
+}
+
+extern "C" int cz_test_rwkv_ln_mix(cz_ctx *ctx, int nmix, int form, int in_place, int R, int C, int n_slots, const float *x, const float *lnw,
+                                   const float *lnb, const float *mu, const int *prev_row, const int *slot, const int *flags,
+                                   const float *state_in, float *state_out, float eps, uint16_t *out_bf16, int *form_used) {
+  using namespace cz;
+  CZ_TRY(require_device(ctx));
+  CZ_CUDA_TRY(cudaSetDevice(ctx->device));
+  bool ok = (nmix == 1 || nmix == 6) && (form == 0 || form == 1) && R > 0 && C > 0 && C <= czk::RW_MAXC && n_slots > 0 && x && lnw && lnb &&
+            mu && prev_row && slot && flags && state_in && state_out && out_bf16 && form_used;
+  for (int r = 0; ok && r < R; r++) ok = prev_row[r] >= -1 && prev_row[r] < R && slot[r] >= 0 && slot[r] < n_slots;
+  if (!ok) {
+    set_error("cz_test_rwkv_ln_mix: bad arguments");
+    return CZ_ERR_INVALID;
+  }
+  const size_t RC = (size_t)R * C, SN = (size_t)n_slots * C;
+  HookBufs d;
+  float *dx, *dw, *db, *dmu, *dsin, *dsout;
+  __nv_bfloat16 *dout;
+  int *dmeta;
+  CZ_TRY(d.alloc(dx, RC));
+  CZ_TRY(d.alloc(dw, (size_t)C));
+  CZ_TRY(d.alloc(db, (size_t)C));
+  CZ_TRY(d.alloc(dmu, (size_t)nmix * C));
+  CZ_TRY(d.alloc(dsin, SN));
+  CZ_TRY(d.alloc(dout, (size_t)nmix * RC));
+  CZ_TRY(d.alloc(dmeta, 3 * (size_t)R));
+  if (in_place) {
+    dsout = dsin;  // the stepwise decoder's T = 1 steps read and write the same token-shift rows
+  } else {
+    CZ_TRY(d.alloc(dsout, SN));
+    CZ_CUDA_TRY(cudaMemcpy(dsout, state_out, SN * 4, cudaMemcpyHostToDevice));
+  }
+  CZ_CUDA_TRY(cudaMemcpy(dx, x, RC * 4, cudaMemcpyHostToDevice));
+  CZ_CUDA_TRY(cudaMemcpy(dw, lnw, (size_t)C * 4, cudaMemcpyHostToDevice));
+  CZ_CUDA_TRY(cudaMemcpy(db, lnb, (size_t)C * 4, cudaMemcpyHostToDevice));
+  CZ_CUDA_TRY(cudaMemcpy(dmu, mu, (size_t)nmix * C * 4, cudaMemcpyHostToDevice));
+  CZ_CUDA_TRY(cudaMemcpy(dsin, state_in, SN * 4, cudaMemcpyHostToDevice));
+  CZ_CUDA_TRY(cudaMemset(dout, 0xff, (size_t)nmix * RC * 2));  // NaN: a row the kernel skips cannot pass for a result
+  CZ_CUDA_TRY(cudaMemcpy(dmeta, prev_row, (size_t)R * 4, cudaMemcpyHostToDevice));
+  CZ_CUDA_TRY(cudaMemcpy(dmeta + R, slot, (size_t)R * 4, cudaMemcpyHostToDevice));
+  CZ_CUDA_TRY(cudaMemcpy(dmeta + 2 * R, flags, (size_t)R * 4, cudaMemcpyHostToDevice));
+  const bool lane = form == 1;
+  const int rc = nmix == 6 ? hook_ln_mix<6>(ctx, lane, R, C, dx, dw, db, dmu, dmeta, dsin, dsout, dout, eps, form_used)
+                           : hook_ln_mix<1>(ctx, lane, R, C, dx, dw, db, dmu, dmeta, dsin, dsout, dout, eps, form_used);
+  CZ_TRY(hook_sync(ctx, rc, "rwkv ln-mix"));
+  CZ_CUDA_TRY(cudaMemcpy(state_out, dsout, SN * 4, cudaMemcpyDeviceToHost));
+  CZ_CUDA_TRY(cudaMemcpy(out_bf16, dout, (size_t)nmix * RC * 2, cudaMemcpyDeviceToHost));
+  return CZ_OK;
+}

@@ -396,6 +396,23 @@ int cz_test_gemm_norm(cz_ctx *ctx, int M, int N, int K, int N2, const uint16_t *
 int cz_test_attention(cz_ctx *ctx, int n_pos, int nh, int nkv, const uint16_t *q_bf16, const uint16_t *k_bf16,
                       const uint16_t *v_bf16, int mode, uint16_t *out_bf16);
 
+/* one WKV-7 scan (csrc/rwkv7.cu wkv7_scan_kernel<layer0>) over R rows of width C = 64 H (H <= 16): stream s walks rows
+ * row_begin[s] .. row_end[s]-1 in order from state slot stream_slot[s]; stream_active (nullable) skips streams whose flag is 0.
+ * rows [7][R][C] = r, k, v, w-LoRA, a-LoRA, v-LoRA, g (f32); vecs [8][C] = w0, a0, v0, k_k, k_a, r_k, gn_w, gn_b; v_first [R][C] in/out
+ * (written with layer0, read without); state [n_slots][H][4096] in/out in the kernel's layout (row i, column j of a head's 64x64
+ * matrix at (j/4)*256 + i*4 + j%4); out_bf16 [R][C] in/out (rows no active stream covers keep their contents) */
+int cz_test_wkv7_scan(cz_ctx *ctx, int layer0, int R, int H, int n_streams, const int *row_begin, const int *row_end, const int *stream_slot,
+                      const int *stream_active, int n_slots, const float *rows, float *v_first, const float *vecs, float *state,
+                      uint16_t *out_bf16);
+/* one LayerNorm + token-shift mix (rwkv_ln_mix, nmix 1 or 6) over R rows of width C <= 1024: x [R][C], lnw / lnb [C], mu [nmix][C],
+ * per row prev_row (-1: the previous token is state_in[slot]), slot and flags (bit 0 writes state_out[slot], bit 1 suppresses it);
+ * state_in [n_slots][C]; state_out [n_slots][C] in/out, or with in_place the kernel reads and writes one buffer that starts as
+ * state_in.  form 0 runs what the model would run, 1 forces the element-per-lane kernel; *form_used = elements per lane of the kernel
+ * that ran (1 or 8).  out_bf16 [nmix][R][C]. */
+int cz_test_rwkv_ln_mix(cz_ctx *ctx, int nmix, int form, int in_place, int R, int C, int n_slots, const float *x, const float *lnw,
+                        const float *lnb, const float *mu, const int *prev_row, const int *slot, const int *flags, const float *state_in,
+                        float *state_out, float eps, uint16_t *out_bf16, int *form_used);
+
 /* the CDF kernels' fast paths against the originals (csrc/cdf_fast.cuh): (1) every non-negative f32 argument pattern of
  * expf(-(max - logit)): the integer-conversion path must give the bits of the conversion path wherever it is taken; `checksum` =
  * sum over the patterns b of bits(expf(-float(b))) * (2 b + 1) mod 2^64 (NaN results as 0x7fc00000), which the CPU oracle reproduces

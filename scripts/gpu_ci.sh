@@ -12,10 +12,11 @@ rm -f gpurun_out/summary.txt
 run coder_cdf 600 -k "k1 or k2 or k3 or k9"
 run gemm_simt 300 -k "gemm and simt"
 run gemm_tc 300 -k "gemm and not simt"
-run tiny_simt 900 -k "tiny and simt"
-run tiny_tc 900 -k "tiny and not simt"
-run full 900 -k "full_size"
+run tiny_simt 900 -k "tiny and simt and not rwkv7_deep"
+run tiny_tc 900 -k "tiny and not simt and not rwkv7_deep"
+run full 900 -k "full_size and not rwkv7_deep"
 run dictionary 900 -k "dictionary"
 run match 1200 -k "match"
-run rwkv 900 -k "(rwkv7 and not full_size) or hint_prime or gate_scan or file_level or cli_twin"
+run rwkv 900 -k "((rwkv7 and not full_size) or hint_prime or gate_scan or file_level or cli_twin) and not rwkv7_deep"
+run rwkv_deep 1200 -k "rwkv7_deep"
 for f in gpurun_out/*.log; do echo "---- $f"; tail -n 25 "$f"; done

@@ -64,3 +64,12 @@ def make_weights(cfg, seed=0):
     vec("model.norm.bias", 0.0, 0.1)
     lin("lm_head.weight", V, C, 2.0)
     return {k: bf16_exact(v) for k, v in W.items()}
+
+
+def long_memory(W, cfg, seed=1):
+    """w_lora bias ~ N(-7, 0.5): decay ~ 0.999, the state keeps hundreds of tokens"""
+    rng = np.random.default_rng(seed)
+    W = dict(W)
+    for l in range(cfg["n_layers"]):
+        W[f"model.layers.{l}.attn.w_lora.lora.2.bias"] = bf16_exact(rng.normal(-7.0, 0.5, cfg["d_model"]))
+    return W

@@ -461,12 +461,14 @@ def test_rwkv7_tiny_logits_vs_oracle_and_golden(gpu_ctx, engine):
         assert np.abs(got[j] - z["logits"][j]).max() < 0.05 * sd, j
 
 
-@pytest.mark.parametrize("engine", [_lib.CZ_ENGINE_SIMT, _lib.CZ_ENGINE_TCGEN05], ids=["simt", "tc"])
-def test_rwkv7_stepwise_equals_slab_bitwise(gpu_ctx, engine):
-    """decode safety: T=1 steps, one long slab and several short slabs give bit-identical logits"""
+@pytest.mark.parametrize("engine,n", [(_lib.CZ_ENGINE_SIMT, 90), (_lib.CZ_ENGINE_TCGEN05, 90), (_lib.CZ_ENGINE_TCGEN05, 2048)],
+                         ids=["simt", "tc", "tc-long"])
+def test_rwkv7_stepwise_equals_slab_bitwise(gpu_ctx, engine, n):
+    """decode safety: T=1 steps, one long slab and several short slabs give bit-identical logits (the long case carries the
+    recurrent state over 2,047 steps)"""
     model, cfg, _ = _rwkv_tiny(gpu_ctx, engine)
     rng = np.random.default_rng(21)
-    toks = rng.integers(0, cfg["vocab"], 90).astype(np.uint32)
+    toks = rng.integers(0, cfg["vocab"], n).astype(np.uint32)
     slab = model.chunk_logits(toks[:1], toks[1:])
     s = model.session()
     step = np.stack([s.step_logits_tensor(t) for t in toks[:-1]])
@@ -478,7 +480,7 @@ def test_rwkv7_stepwise_equals_slab_bitwise(gpu_ctx, engine):
     assert s.index_pos() == 40
 
 
-@pytest.mark.parametrize("n,n_seg,lit", [(1, 1, 0.0), (400, 1, 0.0), (900, 3, 0.08), (257, 5, 0.3)])
+@pytest.mark.parametrize("n,n_seg,lit", [(1, 1, 0.0), (400, 1, 0.0), (900, 3, 0.08), (257, 5, 0.3), (4096, 4, 0.05)])
 def test_rwkv7_roundtrip_and_oracle_bitstream(gpu_ctx, n, n_seg, lit):
     model, cfg, W = _rwkv_tiny(gpu_ctx)
     V = cfg["vocab"]
